@@ -10,6 +10,7 @@ one physics step.  Metric: env-steps/s, whole job (all GPUs).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 200 --warmup 5
     python bench.py --impl reference --steps 5 --warmup 1     # CPU arm: oracle on host cores
+    python bench.py --dump-outputs out/   # also write the last timed step's outputs (seeded inputs: comparable across builds)
 """
 from __future__ import annotations
 
@@ -57,7 +58,33 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="headline workload only (no drone / humanoid lines in `secondary`)")
     ap.add_argument("--e2e-host-controller", action="store_true", help="e2e leg: evaluate the LQR law in NumPy on the host instead of on the device")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU-baseline sample duration")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each workload returned (state, controls, (A, B); rank 0's envs) "
+                         "to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
+
+
+# --dump-outputs writes at most this much per workload (a run times at most four workloads: 64 MiB in all); a workload
+# whose outputs are larger is written for a fixed, seeded sample of its envs
+DUMP_BYTES_PER_WORKLOAD = 16 << 20
+
+
+def dump_outputs(directory: str, prefix: str, env, result) -> None:
+    """What a caller of env.step() receives from one step -- the state and controls in env.data, (A, B) in result.info --
+    as float64 arrays with the env axis first, one DIR/<prefix><name>.npy each."""
+    import torch
+
+    arrays = {k: getattr(env.data, k).T for k in ("qpos", "qvel", "ctrl")}
+    arrays.update({k: result.info[k] for k in ("A", "B") if k in result.info})
+    nenv = arrays["qpos"].shape[0]
+    keep = min(nenv, DUMP_BYTES_PER_WORKLOAD // sum(8 * (t.numel() // nenv) for t in arrays.values()))
+    envs = np.sort(np.random.default_rng(0).choice(nenv, keep, replace=False)) if keep < nenv else slice(None)
+    os.makedirs(directory, exist_ok=True)
+    for k, t in arrays.items():
+        np.save(os.path.join(directory, prefix + k + ".npy"), np.ascontiguousarray(t.to("cpu", dtype=torch.float64).numpy()[envs]))
 
 
 DEFAULT_NENV = {"pendulum": 65536, "cartpole": 65536, "drone": 262144, "humanoid": 16384}
@@ -211,7 +238,7 @@ class ClockSampler(threading.Thread):
 
 
 CPU_KIND_NOTE = ("oracle = C restatement of mj_step / mjd_transitionFD, built -O3 -march=native with FP contraction for this arm "
-                 "(oracle/_fast, compiled on this host); mujoco itself is not installable offline")
+                 "(compiled on this host into a temporary directory); mujoco itself is not installable offline")
 
 
 def _cpu_model(model):
@@ -351,7 +378,7 @@ def make_controller(name: str, lin: bool, seed: int = 0, tv_lqr: bool = False):
 
 
 def run_workload(ctx, name: str, lin: bool, nenv: int, steps: int, warmup: int, *, use_graph: bool, want_e2e: bool,
-                 e2e_host_controller: bool, cpu_seconds: float, tv_lqr: bool = False) -> dict:
+                 e2e_host_controller: bool, cpu_seconds: float, tv_lqr: bool = False, dump: tuple | None = None) -> dict:
     """Times one workload on this rank's GPU and returns the fields of its JSON line (rank 0's copy is printed)."""
     import torch
     import torch.distributed as dist
@@ -429,13 +456,15 @@ def run_workload(ctx, name: str, lin: bool, nenv: int, steps: int, warmup: int, 
             torch.cuda._sleep(spin_cycles)
         flush.zero_()  # evict state / outputs from L2 between timed iterations (outside the event pair)
         starts[i].record()
-        env.step(return_obs=False)
+        result = env.step(return_obs=False)
         stops[i].record()
     sampler.sample_now()  # the queued steps are executing now
     barrier()
     wall = time.perf_counter() - wall0
     sampler.in_region = False
     clocks = sampler.stop()
+    if dump is not None and rank == 0:  # (directory, file-name prefix); before anything else touches the batch
+        dump_outputs(*dump, env, result)
     step_ms = [a.elapsed_time(b) for a, b in zip(starts, stops)]
     total_ms = float(sum(step_ms))
     # graph replays re-launch the captured kernels without passing through the C-ABI counter
@@ -734,8 +763,9 @@ def main():
     name = args.model
     lin = not args.no_linearize
     common = dict(use_graph=not args.no_graph, want_e2e=not args.no_e2e, e2e_host_controller=args.e2e_host_controller)
+    dump = lambda prefix: (args.dump_outputs, prefix) if args.dump_outputs else None  # noqa: E731
     out = run_workload(ctx, name, lin, args.nenv or DEFAULT_NENV[name], args.steps, args.warmup,
-                       cpu_seconds=0.0 if args.no_cpu_baseline else args.cpu_seconds, **common)
+                       cpu_seconds=0.0 if args.no_cpu_baseline else args.cpu_seconds, dump=dump(""), **common)
     out["host_binding"] = numa
     # BASELINE.json configs[2] / configs[3] ride along with the headline workload (same run, same clocks, same rank
     # count): drone free flight under random thrust and the humanoid with contacts, step only
@@ -743,14 +773,14 @@ def main():
         out["secondary"] = {}
         for sname in ("drone", "humanoid"):
             sec = run_workload(ctx, sname, False, DEFAULT_NENV[sname], args.steps, args.warmup,
-                               cpu_seconds=0.0 if args.no_cpu_baseline else min(args.cpu_seconds, 5.0), **common)
+                               cpu_seconds=0.0 if args.no_cpu_baseline else min(args.cpu_seconds, 5.0), dump=dump(sname + "_"), **common)
             out["secondary"][sname] = {k: sec[k] for k in ("value", "unit", "ms_per_step", "ms_per_step_per_rank", "steps", "config", "roofline",
                                                            "roofline_fp64", "cpu_baseline", "e2e", "gpu_launches", "contact_stats",
                                                            "bad_env_flags", "kernel_variant", "clocks")}
         # config #2 read literally ("per-step FD (A, B) linearisation for LQR"): the same workload with every env's gain
         # re-synthesised every tick from its own latest (A, B) -- DARE + gain (b2_dlqr), per-env control law, FD, step
         tv = run_workload(ctx, "cartpole", True, DEFAULT_NENV["cartpole"], args.steps, args.warmup, use_graph=not args.no_graph,
-                          want_e2e=False, e2e_host_controller=False, cpu_seconds=0.0, tv_lqr=True)
+                          want_e2e=False, e2e_host_controller=False, cpu_seconds=0.0, tv_lqr=True, dump=dump("cartpole_tv_lqr_"))
         out["secondary"]["cartpole_tv_lqr"] = {k: tv[k] for k in ("value", "unit", "ms_per_step", "ms_per_step_per_rank", "steps", "config",
                                                                   "gpu_launches", "bad_env_flags", "kernel_variant", "clocks")}
     if rank == 0:

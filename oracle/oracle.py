@@ -12,6 +12,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -20,33 +21,26 @@ _LIB = None
 _dp = C.POINTER(C.c_double)
 
 
-def _cpu_stamp() -> str:
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("model name"):
-                return line.split(":", 1)[1].strip()
-    except OSError:
-        pass
-    return "unknown-cpu"
-
-
 def build(force: bool = False, variant: str = "strict") -> str:
-    """strict: -O2 -ffp-contract=off, the parity oracle.  count: the op-counting build (orc_count.h).  fast: -O3
-    -march=native with contraction, ONLY for bench.py's CPU arm -- rebuilt whenever the host CPU differs from the one it
-    was compiled on (the file travels from the build box to the GPU box)."""
-    target = {"strict": "liborc.so", "count": "liborc_count.so", "fast": os.path.join("_fast", "liborc_fast.so")}[variant]
+    """strict: -O2 -ffp-contract=off, the parity oracle.  count: the op-counting build (orc_count.h).  Both are built
+    in the tree by ``__graft_entry__.build()``; this rebuilds them when a source is newer."""
+    target = {"strict": "liborc.so", "count": "liborc_count.so"}[variant]
     so = os.path.join(_HERE, target)
     src = [os.path.join(_HERE, f) for f in ("mjstep_oracle.c", "orc_math.h", "orc_count.h")]
     src.append(os.path.join(_HERE, "..", "include", "b2_model_layout.h"))
     stale = not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src)
-    stamp = os.path.join(_HERE, "_fast", "cpu.txt")
-    if variant == "fast" and not stale:
-        stale = not os.path.exists(stamp) or open(stamp).read() != _cpu_stamp()
     if force or stale:
         subprocess.run(["make", "-C", _HERE, "-B", target], check=True, capture_output=True)
-        if variant == "fast":
-            open(stamp, "w").write(_cpu_stamp())
     return so
+
+
+def _load_fast() -> C.CDLL:
+    """fast: -O3 -march=native with contraction, ONLY for bench.py's CPU arm.  Compiled for the CPU of the host that
+    runs it, in a temporary directory (the source tree may be read-only) that is removed once the library is loaded."""
+    with tempfile.TemporaryDirectory(prefix="orc_fast_") as tmp:
+        so = os.path.join(tmp, "liborc_fast.so")
+        subprocess.run(["make", "-C", _HERE, "-B", f"FAST_DIR={tmp}", so], check=True, capture_output=True)
+        return C.CDLL(so)
 
 
 _LIBS: dict[str, C.CDLL] = {}
@@ -56,7 +50,7 @@ def lib(variant: str = "strict") -> C.CDLL:
     global _LIB
     if variant != "strict":
         if variant not in _LIBS:
-            _LIBS[variant] = _declare(C.CDLL(build(variant=variant)))
+            _LIBS[variant] = _declare(_load_fast() if variant == "fast" else C.CDLL(build(variant=variant)))
             if variant == "count":
                 _LIBS[variant].orc_count_read.argtypes = [C.POINTER(C.c_ulonglong)]
         return _LIBS[variant]

@@ -1,9 +1,9 @@
 """Generate tests/golden/models/*.b2m from the reference's example MJCF files.
 
-Run in the build container (needs /root/reference):
-    python tests/golden/make_models.py
-The GPU box has no /root/reference, so GPU tests, smoke() and bench.py load these
-compiled-model files instead of the XML.  They are derived artefacts of OUR compiler.
+Needs a checkout of the original mujoco-template project:
+    B2_REFERENCE=<checkout> python tests/golden/make_models.py
+Tests, smoke() and bench.py load these compiled-model files instead of the XML, so they run
+without that checkout.  They are derived artefacts of OUR compiler.
 """
 import os
 import sys
@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, os.path.join(ROOT, "mujoco-template_b200"))
 from mujoco_template import _mj as mj  # noqa: E402
 
-REF = os.environ.get("B2_REFERENCE", "/root/reference")
+REF = os.environ.get("B2_REFERENCE", "")
 MODELS = {
     "pendulum": "examples/pendulum/pendulum.xml",
     "cartpole": "examples/cartpole/cartpole.xml",

@@ -1,11 +1,14 @@
 """Generates tests/golden/scenario_*.npz: the reference's example scenarios (its own controllers, imported unmodified from
-/root/reference/examples) run on the oracle-backed Env, recorded step by step.  The fixtures let the GPU box -- which has
-no /root/reference -- replay the same trajectories through the CUDA path (tests/test_gpu_parity.py::test_reference_scenario_*).
+the original mujoco-template checkout's examples/) run on the oracle-backed Env, recorded step by step.  The fixtures
+let the test suite replay the same trajectories without that checkout: on the oracle (tests/test_reference_scenarios.py)
+and through the CUDA path (tests/test_gpu_parity.py::test_reference_scenario_*).
 
-    python tests/golden/make_scenario_golden.py          # needs /root/reference; writes next to this file
+    B2_REFERENCE=<checkout> python tests/golden/make_scenario_golden.py          # writes next to this file
 
 Each file holds: qpos0 / qvel0 / ctrl0 / warm0 (state before the first step), ctrl[t] (what the controller wrote before step
-t), qpos[t] / qvel[t] / warm[t] (state and qacc_warmstart after step t), time[t], header + rows of the StateControlRecorder CSV, duration / max_steps.
+t), qpos[t] / qvel[t] / warm[t] (state and qacc_warmstart after step t), time[t], header + rows of the StateControlRecorder
+CSV (the humanoid's first ROWS_KEPT rows only: its CSV repeats qpos / qvel / ctrl and no test reads further), duration /
+max_steps.
 """
 import importlib
 import os
@@ -31,6 +34,7 @@ import test_reference_scenarios as T  # noqa: E402
 
 MODEL_OF = {"pendulum_pd": "pendulum", "pendulum_passive": "pendulum", "cartpole_pid": "cartpole", "drone_lqr": "drone",
             "humanoid_lqr": "humanoid"}
+ROWS_KEPT = {"humanoid_lqr": 100}  # keeps the file under 1 MB
 
 
 def main():
@@ -62,7 +66,7 @@ def main():
             rows = np.loadtxt(os.path.join(tmp, "log.csv"), delimiter=",", skiprows=1)
         assert steps == expected_steps, (name, steps)
         out = os.path.join(HERE, f"scenario_{name}.npz")
-        np.savez_compressed(out, model=MODEL_OF[name], steps=steps, header=np.array(header), rows=rows,
+        np.savez_compressed(out, model=MODEL_OF[name], steps=steps, header=np.array(header), rows=rows[:ROWS_KEPT.get(name)],
                             ctrl=np.array(ctrl).reshape(steps, -1), qpos=np.array(qpos), qvel=np.array(qvel), time=np.array(time),
                             warm=np.array(warm),
                             duration=np.array(np.nan if cfg.run.simulation.duration_seconds is None else cfg.run.simulation.duration_seconds),

@@ -1,10 +1,10 @@
 """Live parity against a real MuJoCo, wherever one is installed (SURVEY.md 8c pin 4).
 
-The build container and the GPU boxes have no ``mujoco`` wheel, so this module is skipped there and the oracle stays
-"parity unpinned".  On any machine with ``pip install mujoco`` (>= 3.1) it pins the oracle -- and therefore the CUDA
-path, which the GPU tests hold to the oracle -- to upstream: model constants from our MJCF compiler, per-step
-trajectories, mjd_transitionFD, Jacobians, sensors and inverse dynamics, on inline models and (when the reference tree
-is present, ``B2_REFERENCE`` or /root/reference) on the four example models.
+Without the ``mujoco`` package this module is skipped and the oracle stays "parity unpinned".  On any machine with
+``pip install mujoco`` (>= 3.1) it pins the oracle -- and therefore the CUDA path, which the GPU tests hold to the
+oracle -- to upstream: model constants from our MJCF compiler, per-step trajectories, mjd_transitionFD, Jacobians,
+sensors and inverse dynamics, on inline models and (when ``B2_REFERENCE`` names a checkout of the original
+mujoco-template project) on the four example models.
 """
 import os
 import warnings
@@ -19,7 +19,7 @@ from test_host_logic import BASE_XML  # noqa: E402
 from test_mjcf_compiler import ARM_XML  # noqa: E402
 from test_oracle_analytic import SENSOR_XML  # noqa: E402
 
-REF = os.environ.get("B2_REFERENCE", "/root/reference")
+REF = os.environ.get("B2_REFERENCE", "")
 EXAMPLES = {
     "pendulum": "examples/pendulum/pendulum.xml", "cartpole": "examples/cartpole/cartpole.xml",
     "drone": "examples/drone/scene.xml", "humanoid": "examples/humanoid/humanoid.xml",

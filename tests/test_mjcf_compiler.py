@@ -7,7 +7,7 @@ import pytest
 
 from conftest import GOLDEN, MODEL_NAMES, load_model
 
-REF = os.environ.get("B2_REFERENCE", "/root/reference")
+REF = os.environ.get("B2_REFERENCE", "")  # checkout of the original mujoco-template project
 REF_XML = {"pendulum": "examples/pendulum/pendulum.xml", "cartpole": "examples/cartpole/cartpole.xml",
            "drone": "examples/drone/scene.xml", "humanoid": "examples/humanoid/humanoid.xml"}
 
@@ -84,7 +84,8 @@ def test_example_model_dimensions():
     assert d.opt.density == 1.225 and d._c["has_fluid"] == 1 and d.ngeom == 11 and d.nsite == 5
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples")),
+                    reason="needs a checkout of the original mujoco-template project (B2_REFERENCE)")
 @pytest.mark.parametrize("name", MODEL_NAMES)
 def test_committed_model_files_match_a_fresh_compile(name):
     from mujoco_template import _mj as mj

@@ -1,6 +1,6 @@
 """Known answers published with the real engine's output.
 
-The reference ships DeepMind's LQR tutorial as source text only (``/root/reference/LQR.txt``; ``LQR.txt:158-163``
+The reference ships DeepMind's LQR tutorial as source text only (``LQR.txt`` of the original mujoco-template project; ``LQR.txt:158-163``
 ``mujoco.mj_inverse(model, data); print(data.qfrc_inverse)``, ``:165-205`` the height sweep and ``print('desired forces:',
 qfrc0)``).  The tutorial notebook as published upstream (mujoco/python/LQR.ipynb) carries the output cells of exactly
 these statements, produced by MuJoCo itself on the humanoid model the reference uses (``examples/humanoid/humanoid.xml``,

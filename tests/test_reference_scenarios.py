@@ -1,7 +1,8 @@
 """The reference's own example scenarios replayed through the drop-in.
 
-The reference's scenario modules and controllers (``/root/reference/examples/{pendulum,cartpole,drone,humanoid}``) are
-imported UNMODIFIED against this package: they only use ``mt.*`` and ``mt.mj.*`` (e.g.
+The reference's scenario modules and controllers (``examples/{pendulum,cartpole,drone,humanoid}`` of the original
+mujoco-template checkout named by ``B2_REFERENCE``) are imported UNMODIFIED against this package: they only use ``mt.*``
+and ``mt.mj.*`` (e.g.
 ``examples/drone/controllers/lqr.py:5,87-88,227``, ``examples/pendulum/controllers/pd.py:3``,
 ``examples/humanoid/controllers/lqr.py:47-95``).  The run harness itself (``PassiveRunSettings`` /
 ``PassiveRunHarness``: viewer, video, CLI plumbing -- out of scope, SURVEY.md section 2) is replaced by three recording
@@ -14,7 +15,8 @@ run_passive_headless(duration, max_steps, hooks).
   CSV schema, and the controllers doing their job (pendulum settles, drone reaches its goal, humanoid stays up);
 * gpu: the same scenarios on the CUDA path, CSV rows compared with the oracle-backed run.
 
-Nothing here runs on the GPU box unless the reference tree is present (it is not: these tests skip there).
+Those tests skip without the checkout.  The runs they make are recorded in tests/golden/scenario_*.npz
+(make_scenario_golden.py), and test_recorded_scenario_replays_on_oracle_backed_env replays the recordings without it.
 """
 import csv
 import importlib
@@ -25,10 +27,11 @@ from types import SimpleNamespace
 import numpy as np
 import pytest
 
-from conftest import ROOT  # noqa: F401  (sys.path set-up)
+from conftest import GOLDEN, load_model
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples")), reason="reference tree not present")
+REF = os.environ.get("B2_REFERENCE", "")
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples")),
+                                     reason="needs a checkout of the original mujoco-template project (B2_REFERENCE)")
 
 SCENARIOS = {
     # name: (scenario module, expected step count, CSV tolerance GPU-vs-oracle)
@@ -106,6 +109,58 @@ def _run(module_name: str, log_path):
 
 
 @pytest.mark.parametrize("name", list(SCENARIOS))
+def test_recorded_scenario_replays_on_oracle_backed_env(name, tmp_path):
+    """The recorded run of each scenario (its controls replayed open loop) on an oracle-backed ``Env`` driven as the
+    reference's harness drives it: the loop-exit rule gives the recorded step count, the CSV has the reference schema and
+    time column, and every step lands on the recorded state -- the oracle reproduces the reference controllers' runs."""
+    import mujoco_template as mt
+    from oracle_backend import make_env
+
+    f = np.load(os.path.join(GOLDEN, f"scenario_{name}.npz"))
+    model = load_model(str(f["model"]))
+    ctrl, expected_steps = f["ctrl"], SCENARIOS[name][1]
+    states = []
+
+    class Replay:
+        capabilities = mt.ControllerCapabilities()
+        k = 0
+        def prepare(self, m, d): pass
+        def __call__(self, m, d, t):
+            if m.nu:
+                d.ctrl[:] = ctrl[min(self.k, len(ctrl) - 1)]
+            self.k += 1
+
+    env = make_env(model, controller=Replay() if model.nu else None)
+    env.reset()
+    env.data.qpos[:] = f["qpos0"]; env.data.qvel[:] = f["qvel0"]
+    if model.nu:
+        env.data.ctrl[:] = f["ctrl0"]
+    env.handle.forward()
+    log = tmp_path / "log.csv"
+    rec = mt.StateControlRecorder(env, log_path=log, store_rows=True)
+    duration = None if np.isnan(f["duration"]) else float(f["duration"])
+    max_steps = None if int(f["max_steps"]) < 0 else int(f["max_steps"])
+    tap = lambda _r: states.append(np.concatenate([env.data.qpos, env.data.qvel, env.data.qacc_warmstart]))  # noqa: E731
+    with rec:
+        steps = mt.run_passive_headless(env, duration=duration, max_steps=max_steps, hooks=[tap, rec])
+    assert steps == int(f["steps"]) == expected_steps
+    with open(log) as fh:
+        rows = list(csv.reader(fh))
+    header = [str(h) for h in f["header"]]
+    assert rows[0] == header[:len(rows[0])] and len(rows[0]) == 1 + model.nq + model.nv + max(model.nu, 1)
+    got = np.array(rows[1:], dtype=float)
+    assert got.shape == (expected_steps, len(rows[0])) and np.isfinite(got).all()
+    np.testing.assert_allclose(got[:, 0], float(model.opt.timestep) * np.arange(1, expected_steps + 1), rtol=0, atol=1e-9)
+    ref = f["rows"][:, :got.shape[1]]
+    err = np.abs(got[:len(ref)] - ref) / np.maximum(1.0, np.abs(ref))
+    assert err.max() <= 1e-9, (name, float(err.max()))
+    want = np.concatenate([f["qpos"], f["qvel"], f["warm"]], axis=1)
+    err = np.abs(np.array(states) - want) / np.maximum(1.0, np.abs(want))
+    assert err.max() <= 1e-9, (name, float(err.max()), int(err.max(axis=1).argmax()))
+
+
+@needs_reference
+@pytest.mark.parametrize("name", list(SCENARIOS))
 def test_reference_scenario_on_oracle_backed_env(name, reference_examples, monkeypatch, tmp_path):
     module_name, expected_steps, _ = SCENARIOS[name]
     _use_oracle_backend(monkeypatch)
@@ -140,6 +195,7 @@ def test_reference_scenario_on_oracle_backed_env(name, reference_examples, monke
         # amplitude (measured, DESIGN.md section 5).  Whether upstream MuJoCo holds seed 1 cannot be checked here.
 
 
+@needs_reference
 def test_reference_humanoid_lqr_balances_without_control_noise(reference_examples, monkeypatch, tmp_path):
     """The same scenario with `perturbations_enabled=False`: the LQR law built from THIS engine's mj_inverse, (A, B),
     subtree-CoM and body-CoM Jacobians keeps the humanoid on one leg for the whole 6 s and comes to rest."""
@@ -157,6 +213,7 @@ def test_reference_humanoid_lqr_balances_without_control_noise(reference_example
     assert env.data.ncon >= 2
 
 
+@needs_reference
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(SCENARIOS))
 def test_reference_scenario_cuda_rows_match_oracle_rows(name, reference_examples, monkeypatch, tmp_path):

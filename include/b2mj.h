@@ -16,7 +16,7 @@
  *    default stream) unless stated otherwise.  Device memory is allocated in b2_model_create /
  *    b2_batch_create (model images, warp-engine scratch) and on the FIRST call of the entry points
  *    that need extra buffers (b2_control_tick / b2_step_lazy: shadow state; b2_step_host: staging;
- *    b2_lqr_set_gain); b2_step, b2_forward, b2_linearize and b2_jacobian never allocate.
+ *    b2_lqr_set_gain); b2_step, b2_forward, b2_linearize, b2_linearize_sensors and b2_jacobian never allocate.
  *  - No process-wide model state: a model's constants live in per-model device images handed to
  *    every launch, so batches of different models can be driven from different threads and streams,
  *    and a captured CUDA graph replays with the model it was captured with.  One b2_batch must not be
@@ -109,6 +109,15 @@ int b2_forward(b2_batch* batch, const b2_state* state, const b2_derived* derived
  * (reference mujoco_template/linearization.py:16-35).  A: (2nv, 2nv, nenv), B: (2nv, nu, nenv),
  * element (r, c, e) at base[(r * ncols + c) * nenv + e].  State is not modified. */
 int b2_linearize(b2_batch* batch, const b2_state* state, double eps, int centered, void* A, void* B, void* stream);
+
+/* Replaces mj.mjd_transitionFD(model, data, eps, centered, A, B, C, D) with the sensor Jacobians: b2_linearize's (A, B)
+ * plus C = d sensordata / dx (nsensordata, 2nv, nenv) and D = d sensordata / du (nsensordata, nu, nenv), same layout, from
+ * the same rollouts in the same launch.  A rollout's reading is the sensordata of its forward pass at the perturbed input
+ * state (RK4: the first stage); readings are differenced by plain subtraction (framequat components too), control columns
+ * follow B's ctrlrange rules.  Any of A, B, C, D may be NULL, but not all four.  Without sensors this is b2_linearize.
+ * State is not modified; never allocates. */
+int b2_linearize_sensors(b2_batch* batch, const b2_state* state, double eps, int centered, void* A, void* B, void* C, void* D,
+                         void* stream);
 
 /* Replaces mj.mj_jacSite / mj_jacBody / mj_jacBodyCom / mj_jacSubtreeCom
  * (reference mujoco_template/jacobians.py:44,55,67,79).  jacp/jacr: (3, nv, nenv); jacr may be NULL. */

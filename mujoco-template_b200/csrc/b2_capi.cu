@@ -366,6 +366,30 @@ int b2_linearize(b2_batch* b, const b2_state* st, double eps, int centered, void
   return do_linearize(b, st, b->nenv, eps, centered, A, B, stream);
 }
 
+int b2_linearize_sensors(b2_batch* b, const b2_state* st, double eps, int centered, void* A, void* B, void* C, void* D, void* stream) {
+  B2_CHECK_STATE("b2_linearize_sensors");
+  if (!(eps > 0)) return fail(B2_ERR_LINEARIZE, "b2_linearize_sensors: eps must be > 0");
+  if (!A && !B && !C && !D) return fail(B2_ERR_ARG, "b2_linearize_sensors: A, B, C and D are all NULL");
+  const b2m_view& v = b->model->v;
+  // without sensors (or without C / D to fill) this is b2_linearize; the warp engine only runs models without sensors
+  if (v.nsensordata == 0 || (!C && !D)) return (A || B) ? do_linearize(b, st, b->nenv, eps, centered, A, B, stream) : B2_OK;
+  int rc;
+  if (const b2::SpecKernels* k = active_spec(b)) {
+    cudaError_t e = cudaSetDevice(b->device);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+    if (!k->linearize_sensors[prec_index(b)]) return fail(B2_ERR_ARG, "b2_linearize_sensors: specialised kernel set has no sensor variant");
+    rc = k->linearize_sensors[prec_index(b)](st, b->nenv, b->nenv, eps, centered, A, B, C, D, stream);
+  } else {
+    const void* lane = nullptr;
+    if ((rc = lane_image(b, &lane))) return rc;
+    const int ncol = b2::fd_task_count(v.integrator, v.nv, v.nu);
+    rc = b->precision == B2_F64 ? b2::b2k_linearize_sensors_f64(lane, b->model->cls, st, b->nenv, b->nenv, ncol, eps, centered, A, B, C, D, stream)
+                                : b2::b2k_linearize_sensors_f32(lane, b->model->cls, st, b->nenv, b->nenv, ncol, eps, centered, A, B, C, D, stream);
+  }
+  g_launches++;
+  return rc ? cuda_fail((cudaError_t)rc, "linearize_sensors launch") : B2_OK;
+}
+
 int b2_jacobian(b2_batch* b, const b2_state* st, int kind, int objid, void* jacp, void* jacr, void* stream) {
   if (!b || !st || !st->qpos) return fail(B2_ERR_ARG, "b2_jacobian: null batch/state pointer");
   const b2m_view& v = b->model->v;

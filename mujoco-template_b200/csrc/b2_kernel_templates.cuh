@@ -7,6 +7,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "../../include/b2mj.h"
 #include "b2_engine.cuh"
 
@@ -180,6 +182,7 @@ template <class M> B2_DEV int fd_tasks() { return fd_task_count(M::integrator(),
 // resident blocks is short of.  The controls are the exception (they may come from the control law, not from st.ctrl).
 template <typename T>
 struct NominalInMemory {
+  static constexpr bool kSens = false;
   StateDev<T> st;
   int N, e;
   const T* u0;
@@ -188,10 +191,24 @@ struct NominalInMemory {
   B2_DEV T u(int k) const { return u0[k]; }
   B2_DEV T w(int k) const { return st.warm ? __ldg(st.warm + (size_t)k * N + e) : T(0); }
 };
+// ... plus the outputs of the sensor Jacobians (k_linearize<..., SENS = true>) and fd_column's place in them.  (Kept in the
+// accessor rather than as arguments and locals of fd_column: the instantiations without sensors then compile to exactly
+// the code they had before the sensor variant existed.)
+template <typename T>
+struct NominalWithSensors : NominalInMemory<T> {
+  static constexpr bool kSens = true;
+  T *dsdx, *dsdu;
+  mutable T* col;      // entry (0, c, e) of the current column in dsdx / dsdu, or null
+  mutable int ncol;    // columns of that array
+  mutable bool first;  // no rollout of the column has stored its reading yet
+};
 
 // One column of the FD linearisation for env e -- c < nv: tangent-space position column, c < 2nv: velocity column, else
 // control column c - 2nv -- or, with nominal = true, the unperturbed step itself, which leaves the advanced state in
 // env.qpos / env.qvel / env.warm.  nom: accessor of the env's nominal state.
+// With S::kSens (NominalWithSensors) the same rollouts also give the column of the sensor Jacobians, nom.dsdx =
+// d sensordata / dx (nsensordata, 2nv, N) for state columns and nom.dsdu = d sensordata / du (nsensordata, nu, N) for
+// control columns (either may be null).
 template <int PART, typename T, class D, class M, class S>
 B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
                       T eps, T inv_eps, int centered, int N, int e, T* A, T* B, bool& pos_valid, bool& vel_valid) {
@@ -221,6 +238,19 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
     back = (centered || !fwd) && (!lim || (u - eps >= lo && u - eps <= hi && u >= lo && u <= hi));
   }
   const int need = nominal ? 4 : ((fwd ? 1 : 0) | (back ? 2 : 0) | ((fwd != back) ? 4 : 0));  // plus, minus, nominal rollouts
+  // SENS: the column's sensor entries live in the output array itself, not in registers (the group thread of the drone is
+  // at the 255-register limit already).  Each (r, c, e) entry has one owning thread: its first rollout stores the reading
+  // with its sign, its second adds its own and scales, so the entry is (s2 - s1) * ih -- the plain difference quotient,
+  // with no tangent-space handling (framequat components included), as upstream mjd_stepFD differences sensordata.
+  if constexpr (S::kSens) {
+    nom.col = nullptr;
+    if (!nominal) {
+      nom.col = c < ndx ? nom.dsdx : nom.dsdu;
+      nom.ncol = c < ndx ? ndx : nu;
+      if (nom.col) nom.col += (size_t)(c < ndx ? c : c - ndx) * N + e;
+      nom.first = true;
+    }
+  }
   // rolled phase loop: the physics is instantiated once; all array indices stay static.  pos_valid (owned by the
   // caller) says that env already holds the position stage of the nominal qpos from an earlier rollout of this thread
   B2_NOUNROLL
@@ -247,6 +277,23 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
     env.forward_acc();
     B2_UNROLL
     for (int k = 0; k < nv; k++) if (!(fabs(env.qacc[k]) <= T(1e10))) env.flags |= 4;
+    if constexpr (S::kSens) {
+      // this rollout's sensordata: its forward pass at the perturbed input state, before integration (RK4: the first stage,
+      // as mj_step leaves it).  sensors() uses spat as scratch; nothing kept across rollouts (pos_valid / vel_valid) lives
+      // there -- the velocity stage's only use of it is as bias_forces' scratch.
+      if (nom.col) {
+        T sd[D::NSD];
+        env.sensors(sd);
+        const bool to2 = phase == 0 || (phase == 2 && !fwd);
+        const T sg = to2 ? T(1) : T(-1), ih = (fwd && back) ? T(0.5) * inv_eps : inv_eps;
+        B2_UNROLL
+        for (int r = 0; r < M::nsensordata(); r++) {
+          T* p = nom.col + (size_t)r * nom.ncol * N;
+          *p = nom.first ? sg * sd[r] : fma(sg, sd[r], *p) * ih;
+        }
+        nom.first = false;
+      }
+    }
     if (M::integrator() == 1) env.rk4(); else env.euler();
     vel_valid = PART != 2 && kind != 1 && kind != 2 && M::integrator() == 0;  // this rollout's velocity stage was the nominal one
     pos_valid = PART != 2 && kind != 1 && M::integrator() == 0;
@@ -279,6 +326,9 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
   } else {
     B2_UNROLL
     for (int k = 0; k < ndx; k++) col[k] = 0;
+    if constexpr (S::kSens) {
+      if (nom.col) { B2_UNROLL for (int r = 0; r < M::nsensordata(); r++) nom.col[(size_t)r * nom.ncol * N] = 0; }
+    }
   }
   if (c < ndx) { if (A) { B2_UNROLL for (int r = 0; r < ndx; r++) A[((size_t)r * ndx + c) * N + e] = col[r]; } }
   else if (B) { B2_UNROLL for (int r = 0; r < ndx; r++) B[((size_t)r * nu + (c - ndx)) * N + e] = col[r]; }
@@ -310,9 +360,11 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
 #else
 #define B2_LIN_BOUNDS(PART) __launch_bounds__((PART) == 2 ? B2_LINP_THREADS : B2_LIN_THREADS, (PART) == 2 ? B2_LINP_MIN_BLOCKS : B2_LIN_MIN_BLOCKS)
 #endif
-template <typename T, class D, class M, int PART = 0>
+// SENS (b2_linearize_sensors): the rollouts also produce the sensor Jacobians dsdx (nsensordata, 2nv, N) and dsdu
+// (nsensordata, nu, N), layout as A / B; launched with gain == nullptr and no shadow (no control law, no env advance).
+template <typename T, class D, class M, int PART = 0, bool SENS = false>
 __global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N, T eps, int centered, T* A, T* B, const T* __restrict__ gain, StateDev<T> shadow,
-                                                                                 const void* image = nullptr) {
+                                                                                 const void* image = nullptr, T* dsdx = nullptr, T* dsdu = nullptr) {
   model_load<M>(image, 0);
   const int nq = M::nq(), nv = M::nv(), nu = M::nu(), ndx = 2 * nv;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -337,7 +389,10 @@ __global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N
     B2_UNROLL
     for (int k = 0; k < nu; k++) u0[k] = st.ctrl[(size_t)k * N + e];
   }
-  const NominalInMemory<T> nom{st, N, e, u0};
+  typedef typename std::conditional<SENS, NominalWithSensors<T>, NominalInMemory<T>>::type Nominal;
+  Nominal nom;
+  nom.st = st; nom.N = N; nom.e = e; nom.u0 = u0;
+  if constexpr (SENS) { nom.dsdx = dsdx; nom.dsdu = dsdu; }
   const bool grouped = M::integrator() == 0;  // not a constant expression for the runtime provider
   const int groups = fd_group_count(nv, nu);
   int c0 = task, c1 = task + 1;

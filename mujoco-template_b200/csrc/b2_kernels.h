@@ -20,6 +20,8 @@ namespace b2 {
   int b2k_step##SUF(const void* image, int cls, const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain, const b2_state* park, void* stream);                  \
   int b2k_linearize##SUF(const void* image, int cls, const b2_state* st, int count, int N, int ncol, double eps, int centered, void* A, void* B,         \
                          const void* gain, const b2_state* shadow, void* stream);                                                                                    \
+  int b2k_linearize_sensors##SUF(const void* image, int cls, const b2_state* st, int count, int N, int ncol, double eps, int centered, void* A,  \
+                                 void* B, void* dsdx, void* dsdu, void* stream);                                                                         \
   int b2k_commit_state##SUF(const b2_state* st, const b2_state* shadow, int count, int N, int nq, int nv, int nu, void* stream); \
   int b2k_jacobian##SUF(const void* image, int cls, const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream);    \
   int b2k_inverse##SUF(const void* image, int cls, const b2_state* st, int N, const void* qacc, void* qfrc, void* moment, void* stream);     \

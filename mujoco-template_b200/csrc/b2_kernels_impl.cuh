@@ -243,6 +243,18 @@ int B2_FN(b2k_linearize)(const void* image, int cls, const b2_state* st, int cou
                        to_dev<real>(st), count, N, (real)eps, centered, (real*)A, (real*)B, (const real*)gain, to_dev<real>(shadow), image)));
   return (int)cudaGetLastError();
 }
+// (A, B) and the sensor Jacobians from the same rollouts (k_linearize<..., SENS = true>); no control law, no env advance
+int B2_FN(b2k_linearize_sensors)(const void* image, int cls, const b2_state* st, int count, int N, int ncol, double eps, int centered, void* A,
+                                 void* B, void* dsdx, void* dsdu, void* stream) {
+  const int threads = 128;
+  const long long total = (long long)count * ncol;
+  const int blocks = (int)((total + threads - 1) / threads);
+  const b2_state* no_shadow = nullptr;
+  B2_DISPATCH(cls, (k_linearize<real, DD, RuntimeModel<DD>, 0, true><<<blocks, threads, 0, (cudaStream_t)stream>>>(
+                       to_dev<real>(st), count, N, (real)eps, centered, (real*)A, (real*)B, nullptr, to_dev<real>(no_shadow), image,
+                       (real*)dsdx, (real*)dsdu)));
+  return (int)cudaGetLastError();
+}
 int B2_FN(b2k_commit_state)(const b2_state* st, const b2_state* shadow, int count, int N, int nq, int nv, int nu, void* stream) {
   int bx = (count + 255) / 256;
   if (bx > 148 * 8) bx = 148 * 8;

@@ -21,6 +21,10 @@ struct SpecKernels {
   int (*linearize[2])(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, const void* gain,
                       const b2_state* shadow, void* stream);
   int (*jacobian[2])(const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream);
+  // b2_linearize_sensors: (A, B) and the sensor Jacobians dsdx / dsdu from the same rollouts.  Emitted only for models with
+  // sensors; null otherwise (the call is then b2_linearize)
+  int (*linearize_sensors[2])(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, void* dsdx,
+                              void* dsdu, void* stream);
 };
 
 void register_spec(const SpecKernels* k);

@@ -23,7 +23,7 @@ _lib: C.CDLL | None = None
 # every symbol include/b2mj.h declares (tests check the shared object exports all of them)
 EXPORTED_SYMBOLS = (
     "b2_model_create", "b2_model_destroy", "b2_model_set_actuator_disabled", "b2_batch_create",
-    "b2_batch_destroy", "b2_step", "b2_forward", "b2_linearize", "b2_jacobian", "b2_integrate_pos",
+    "b2_batch_destroy", "b2_step", "b2_forward", "b2_linearize", "b2_linearize_sensors", "b2_jacobian", "b2_integrate_pos",
     "b2_differentiate_pos", "b2_inverse", "b2_lqr_set_gain", "b2_lqr_control", "b2_control_tick", "b2_refresh_derived", "b2_step_lazy", "b2_step_host", "b2_step_host_wait", "b2_stream_synchronize", "b2_launch_count",
     "b2_batch_size_class", "b2_last_error", "b2_version", "b2_fp_peak", "b2_batch_kernel_variant",
     "b2_recorder_create", "b2_recorder_record", "b2_recorder_destroy", "b2_dlqr", "b2_random_controls", "b2_warp_queue_histogram", "b2_lqr_control_env",
@@ -78,6 +78,7 @@ def lib() -> C.CDLL:
     L.b2_step.argtypes = [vp, C.POINTER(State), i, C.POINTER(Derived), vp]
     L.b2_forward.argtypes = [vp, C.POINTER(State), C.POINTER(Derived), vp]
     L.b2_linearize.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp]
+    L.b2_linearize_sensors.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp, vp, vp]
     L.b2_jacobian.argtypes = [vp, C.POINTER(State), i, i, vp, vp, vp]
     L.b2_inverse.argtypes = [vp, C.POINTER(State), vp, vp, vp, vp]
     L.b2_lqr_set_gain.argtypes = [vp, C.POINTER(d), C.POINTER(d), C.POINTER(d)]
@@ -169,6 +170,11 @@ class NativeBatch:
 
     def linearize(self, state: State, eps: float, centered: bool, A: int, B: int, stream: int = 0) -> None:
         check(self._L.b2_linearize(self.handle, C.byref(state), float(eps), int(bool(centered)), A, B, stream))
+
+    def linearize_sensors(self, state: State, eps: float, centered: bool, A: int | None, B: int | None, C_: int | None,
+                          D_: int | None, stream: int = 0) -> None:
+        """``b2_linearize_sensors``: (A, B) and the sensor Jacobians C = d sensordata / dx, D = d sensordata / du."""
+        check(self._L.b2_linearize_sensors(self.handle, C.byref(state), float(eps), int(bool(centered)), A, B, C_, D_, stream))
 
     def jacobian(self, state: State, kind: int, objid: int, jacp: int, jacr: int | None, stream: int = 0) -> None:
         check(self._L.b2_jacobian(self.handle, C.byref(state), int(kind), int(objid), jacp, jacr, stream))

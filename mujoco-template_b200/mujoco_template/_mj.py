@@ -343,6 +343,22 @@ class NativeBackend:
                      B.data_ptr() if m.nu else None)
         return A, B
 
+    def linearize_sensors(self, eps: float, centered: bool, out=None):
+        """(A, B, C, D) from one FD launch (``b2_linearize_sensors``): ``linearize``'s (A, B) plus the sensor Jacobians
+        C = d sensordata / dx of shape (nsensordata, 2nv, nenv) and D = d sensordata / du of shape (nsensordata, nu, nenv).
+        ``out=(A, B, C, D)`` overwrites existing buffers; an entry that is None gets a fresh one."""
+        torch, m = self.torch, self.model
+        nx, ns = 2 * m.nv, m.nsensordata
+        shapes = ((nx, nx, self.nenv), (nx, m.nu, self.nenv), (ns, nx, self.nenv), (ns, m.nu, self.nenv))
+        bufs = list(out) if out is not None else [None] * 4
+        for k, shape in enumerate(shapes):
+            if bufs[k] is None:
+                bufs[k] = (torch.zeros(shape, dtype=self.dtype).pin_memory() if self.host_mapped
+                           else torch.empty(shape, device=f"cuda:{self.device}", dtype=self.dtype))  # every entry is written
+        self._launch("linearize_sensors", self.batch.linearize_sensors, self.state_struct(), eps, centered,
+                     *[t.data_ptr() if t.numel() else None for t in bufs])
+        return tuple(bufs)
+
     def jacobian(self, kind: int, objid: int, want_rot: bool):
         torch, m = self.torch, self.model
         mk = (lambda: torch.zeros((3, m.nv, self.nenv), dtype=self.dtype).pin_memory()) if self.host_mapped else (
@@ -550,8 +566,16 @@ def _to_host_matrix(t, nenv: int) -> np.ndarray:
 
 
 def mjd_transitionFD(model: MjModel, data: MjData, eps: float, flg_centered: bool, A, B, C_=None, D_=None) -> None:
-    """Single-env signature of upstream: fills row-major ``A (2nv,2nv)`` and ``B (2nv,nu)`` in place."""
-    At, Bt = data.backend.linearize(float(eps), bool(flg_centered))
+    """Single-env signature of upstream: fills row-major ``A (2nv,2nv)`` and ``B (2nv,nu)`` in place, and with ``C_`` /
+    ``D_`` the sensor Jacobians ``C (nsensordata,2nv)`` and ``D (nsensordata,nu)`` from the same rollouts."""
+    if C_ is not None or D_ is not None:
+        At, Bt, Ct, Dt = data.backend.linearize_sensors(float(eps), bool(flg_centered))
+        if C_ is not None and model.nsensordata:
+            C_[...] = _to_host_matrix(Ct, 1)[:, :, 0]
+        if D_ is not None and model.nsensordata and model.nu:
+            D_[...] = _to_host_matrix(Dt, 1)[:, :, 0]
+    else:
+        At, Bt = data.backend.linearize(float(eps), bool(flg_centered))
     if A is not None:
         A[...] = _to_host_matrix(At, 1)[:, :, 0]
     if B is not None and model.nu:

@@ -135,6 +135,9 @@ def emit_spec(compiled: dict, name: str) -> str:
     ncol = 2 * nv + nu
     # k_linearize: Euler deals the velocity / control columns out in groups of B2_FD_GROUP = 4 (b2_kernel_templates.cuh)
     fd_tasks = (nv + nu + 3) // 4 + nv if int(c["integrator"]) == 0 else ncol
+    # the sensor-Jacobian FD launcher exists only for models with sensors (the others' C-ABI call is b2_linearize), so the
+    # generated sources of sensorless models do not change with it
+    has_sensors = int(c["nsensordata"]) > 0
     A('#include "../b2_kernel_templates.cuh"')
     A('#include "../b2_spec_registry.h"')
     A("")
@@ -184,13 +187,23 @@ def emit_spec(compiled: dict, name: str) -> str:
             A(f"  k_linearize<{T}, SDims, SModel<{T}>><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, (const {T}*)gain, to_dev<{T}>(shadow));")
         A("  return (int)cudaGetLastError();")
         A("}")
+        if has_sensors:
+            # (A, B) plus the sensor Jacobians from the same rollouts: one kernel for all FD tasks, no control law, no advance
+            A(f"int spec_linearize_sensors{suf}(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, void* dsdx, void* dsdu, void* stream) {{")
+            A(f"  const int threads = {lin_threads}; const long long total = (long long)count * {fd_tasks};")
+            A("  const int blocks = (int)((total + threads - 1) / threads);")
+            A("  const b2_state* no_shadow = nullptr;")
+            A(f"  k_linearize<{T}, SDims, SModel<{T}>, 0, true><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, nullptr, to_dev<{T}>(no_shadow), nullptr, ({T}*)dsdx, ({T}*)dsdu);")
+            A("  return (int)cudaGetLastError();")
+            A("}")
         A(f"int spec_jacobian{suf}(const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {{")
         A("  const int threads = 128, blocks = (N + threads - 1) / threads;")
         A(f"  k_jacobian<{T}, SDims, SModel<{T}>><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), N, kind, objid, ({T}*)jacp, ({T}*)jacr);")
         A("  return (int)cudaGetLastError();")
         A("}")
+    sens_init = ", {spec_linearize_sensors, spec_linearize_sensors32}" if has_sensors else ""
     A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{spec_step, spec_step32}}, '
-      f'{{spec_linearize, spec_linearize32}}, {{spec_jacobian, spec_jacobian32}}}};')
+      f'{{spec_linearize, spec_linearize32}}, {{spec_jacobian, spec_jacobian32}}{sens_init}}};')
     A("struct Registrar { Registrar() { register_spec(&kSpec); } } registrar;")
     A("}  // namespace")
     A("}  // namespace b2")

@@ -190,12 +190,19 @@ class BatchedEnv:
         mj.mj_forward(self.model, self.data)
 
     # ---- hot path
-    def linearize(self, eps: float | None = None, centered: bool = True):
+    def linearize(self, eps: float | None = None, centered: bool = True, *, sensors: bool = False):
         """(A, B) of every env: ``(nenv, 2nv, 2nv)`` and ``(nenv, 2nv, nu)`` views of fresh SoA buffers -- or of the
         controller's own ``lin_out`` buffers when it provides them (a controller that consumes the linearisation on the
-        device, e.g. ``BatchedTVLQRController``, needs them at a fixed address from tick to tick)."""
+        device, e.g. ``BatchedTVLQRController``, needs them at a fixed address from tick to tick).
+
+        ``sensors=True`` returns (A, B, C, D): also the sensor Jacobians C = d sensordata / dx ``(nenv, nsensordata, 2nv)``
+        and D = d sensordata / du ``(nenv, nsensordata, nu)`` (fresh buffers), from the same FD launch."""
         out = getattr(self.controller, "lin_out", None)
-        A, B = self.data.backend.linearize(self.lin_eps if eps is None else float(eps), centered, out=out)
+        eps = self.lin_eps if eps is None else float(eps)
+        if sensors:
+            mats = self.data.backend.linearize_sensors(eps, centered, out=None if out is None else (*out, None, None))
+            return tuple(t.permute(2, 0, 1) for t in mats)
+        A, B = self.data.backend.linearize(eps, centered, out=out)
         return A.permute(2, 0, 1), B.permute(2, 0, 1)
 
     def jacobians(self, tokens: Iterable[str] | None = None):

@@ -214,17 +214,13 @@ static int prepare_warp(b2_batch* b) {
                         : b2::b2k_warp_plan_f32(&b->model->v, b->nenv, &wpb, &blocks);
   if (slots <= 0) return B2_OK;  // not enough shared memory: stay on the lane engine
   const size_t bytes = f64 ? b2::b2k_warp_scratch_bytes_f64(&b->model->v, slots) : b2::b2k_warp_scratch_bytes_f32(&b->model->v, slots);
-  // + the work-queue counter of the persistent kernel + the buffers of the cost-ordered queue (B2_WARP_SORT=0: plain order)
-  const char* srt = getenv("B2_WARP_SORT");
-  const bool sorted = !(srt && srt[0] == '0');
-  const size_t sort_bytes = sorted ? (f64 ? b2::b2k_warp_sort_bytes_f64(b->nenv) : b2::b2k_warp_sort_bytes_f32(b->nenv)) : 0;
+  // + the work-queue counter of the persistent kernel + the buffers of the cost-ordered queue
+  const size_t sort_bytes = f64 ? b2::b2k_warp_sort_bytes_f64(b->nenv) : b2::b2k_warp_sort_bytes_f32(b->nenv);
   cudaError_t e = cudaMalloc(&b->d_jscratch, bytes + 256 + sort_bytes);
   if (e != cudaSuccess) return cuda_fail(e, "warp-engine scratch cudaMalloc");
   b->d_warp_counter = (char*)b->d_jscratch + bytes;
-  if (sorted) {
-    b->d_warp_sort = (char*)b->d_warp_counter + 256;
-    if ((e = cudaMemset(b->d_warp_sort, 0, sort_bytes)) != cudaSuccess) return cuda_fail(e, "warp-engine queue cudaMemset");
-  }
+  b->d_warp_sort = (char*)b->d_warp_counter + 256;
+  if ((e = cudaMemset(b->d_warp_sort, 0, sort_bytes)) != cudaSuccess) return cuda_fail(e, "warp-engine queue cudaMemset");
   b->warp_mode = 1; b->warp_wpb = wpb; b->warp_blocks = blocks; b->warp_slots = slots;
   return B2_OK;
 }
@@ -275,7 +271,7 @@ static int launch_generic_step(b2_batch* b, const b2_state* st, const b2_derived
   if (b->warp_mode == 1 && count == b->nenv) {
     const void* image = nullptr;
     if ((rc = warp_image_of(b, &image))) return rc;
-    if (b->d_warp_sort && b->warp_wpb > 1 && nsteps > 0) g_launches += 2;  // the queue's histogram and scatter kernels
+    if (b->warp_wpb > 1 && nsteps > 0) g_launches += 2;  // the queue's histogram and scatter kernels
     return f64 ? b2::b2k_warp_step_f64(image, &b->model->v, st, derived, b->nenv, nsteps, b->d_jscratch, b->d_warp_counter, b->d_warp_sort, b->warp_wpb, b->warp_blocks, park, stream)
                : b2::b2k_warp_step_f32(image, &b->model->v, st, derived, b->nenv, nsteps, b->d_jscratch, b->d_warp_counter, b->d_warp_sort, b->warp_wpb, b->warp_blocks, park, stream);
   }
@@ -316,23 +312,24 @@ static int do_step(b2_batch* b, const b2_state* st, int count, int nsteps, const
   g_launches++;
   return rc ? cuda_fail((cudaError_t)rc, "step launch") : B2_OK;
 }
+// C / D (b2_linearize_sensors): the sensor Jacobians from the same rollouts; either one non-null selects the sensor variant
+// of the FD kernel, which has no control law and no env advance
 static int do_linearize(b2_batch* b, const b2_state* st, int count, double eps, int centered, void* A, void* B, void* stream,
-                        const void* gain = nullptr, const b2_state* shadow = nullptr) {
+                        const void* gain = nullptr, const b2_state* shadow = nullptr, void* C = nullptr, void* D = nullptr) {
+  const bool sensors = C || D;
   int rc;
-  // FD tasks per env: see k_linearize (Euler: one thread for all velocity / control columns + one per position column)
-  const int ncol = b2::fd_task_count(b->model->v.integrator, b->model->v.nv, b->model->v.nu);
   if (const b2::SpecKernels* k = active_spec(b)) {
     cudaError_t e = cudaSetDevice(b->device);
     if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    rc = k->linearize[prec_index(b)](st, count, b->nenv, eps, centered, A, B, gain, shadow, stream);
+    const int p = prec_index(b);
+    rc = sensors ? k->linearize_sensors[p](st, count, b->nenv, eps, centered, A, B, C, D, stream)
+                 : k->linearize[p](st, count, b->nenv, eps, centered, A, B, gain, shadow, stream);
   } else {
     const void* lane = nullptr;
     if ((rc = lane_image(b, &lane))) return rc;
-    // large models on the warp engine: one warp per (column, env) rollout pair (B2_WARP_FD=0: lane engine)
-    const char* wfd = getenv("B2_WARP_FD");
-    const bool warp_fd = !(wfd && wfd[0] == '0');
     if ((rc = prepare_warp(b))) return rc;
-    if (warp_fd && b->warp_mode == 1 && count == b->nenv && !gain && !shadow) {
+    // large models on the warp engine: one warp per (column, env) rollout pair (the warp engine runs no model with sensors)
+    if (b->warp_mode == 1 && count == b->nenv && !gain && !shadow && !sensors) {
       const void* image = nullptr;
       if ((rc = warp_image_of(b, &image))) return rc;
       rc = b->precision == B2_F64
@@ -341,8 +338,16 @@ static int do_linearize(b2_batch* b, const b2_state* st, int count, double eps, 
       g_launches++;
       return rc ? cuda_fail((cudaError_t)rc, "warp linearize launch") : B2_OK;
     }
-    rc = b->precision == B2_F64 ? b2::b2k_linearize_f64(lane, b->model->cls, st, count, b->nenv, ncol, eps, centered, A, B, gain, shadow, stream)
-                                : b2::b2k_linearize_f32(lane, b->model->cls, st, count, b->nenv, ncol, eps, centered, A, B, gain, shadow, stream);
+    // FD tasks per env: see k_linearize (Euler: one thread per group of velocity / control columns + one per position column)
+    const b2m_view& v = b->model->v;
+    const int ntask = b2::fd_task_count(v.integrator, v.nv, v.nu);
+    const bool f64 = b->precision == B2_F64;
+    if (sensors)
+      rc = f64 ? b2::b2k_linearize_sensors_f64(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, C, D, stream)
+               : b2::b2k_linearize_sensors_f32(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, C, D, stream);
+    else
+      rc = f64 ? b2::b2k_linearize_f64(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream)
+               : b2::b2k_linearize_f32(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream);
   }
   g_launches++;
   return rc ? cuda_fail((cudaError_t)rc, "linearize launch") : B2_OK;
@@ -373,21 +378,9 @@ int b2_linearize_sensors(b2_batch* b, const b2_state* st, double eps, int center
   const b2m_view& v = b->model->v;
   // without sensors (or without C / D to fill) this is b2_linearize; the warp engine only runs models without sensors
   if (v.nsensordata == 0 || (!C && !D)) return (A || B) ? do_linearize(b, st, b->nenv, eps, centered, A, B, stream) : B2_OK;
-  int rc;
-  if (const b2::SpecKernels* k = active_spec(b)) {
-    cudaError_t e = cudaSetDevice(b->device);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+  if (const b2::SpecKernels* k = active_spec(b))
     if (!k->linearize_sensors[prec_index(b)]) return fail(B2_ERR_ARG, "b2_linearize_sensors: specialised kernel set has no sensor variant");
-    rc = k->linearize_sensors[prec_index(b)](st, b->nenv, b->nenv, eps, centered, A, B, C, D, stream);
-  } else {
-    const void* lane = nullptr;
-    if ((rc = lane_image(b, &lane))) return rc;
-    const int ncol = b2::fd_task_count(v.integrator, v.nv, v.nu);
-    rc = b->precision == B2_F64 ? b2::b2k_linearize_sensors_f64(lane, b->model->cls, st, b->nenv, b->nenv, ncol, eps, centered, A, B, C, D, stream)
-                                : b2::b2k_linearize_sensors_f32(lane, b->model->cls, st, b->nenv, b->nenv, ncol, eps, centered, A, B, C, D, stream);
-  }
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "linearize_sensors launch") : B2_OK;
+  return do_linearize(b, st, b->nenv, eps, centered, A, B, stream, nullptr, nullptr, C, D);
 }
 
 int b2_jacobian(b2_batch* b, const b2_state* st, int kind, int objid, void* jacp, void* jacr, void* stream) {
@@ -610,8 +603,7 @@ int b2_step_host(b2_batch* b, const b2_state* hs, int nsteps, int linearize, dou
   // chunking: warp-engine batches and small batches go through in one piece
   // two chunks measured best at N = 65536 (1.72e8 vs 1.55e8 with 4, 0.94e8 with 16): every extra chunk adds ~11 copy nodes
   // (an async call overlaps with the other batch's call instead: one chunk measured best there, 1.93e8 vs 1.89e8)
-  int nchunk = (b->warp_mode == 1 || N < 4096 || async) ? 1 : 2;
-  if (const char* env_chunks = getenv("B2_HOST_CHUNKS")) { const int c = atoi(env_chunks); if (c >= 1 && c <= 64 && nchunk > 1) nchunk = c; }
+  const int nchunk = (b->warp_mode == 1 || N < 4096 || async) ? 1 : 2;
   if (!b->pipe_ready) {
     for (int i = 0; i < 3; i++) if ((e = cudaStreamCreateWithFlags(&b->pipe[i], cudaStreamNonBlocking))) return cuda_fail(e, "cudaStreamCreate");
     for (int i = 0; i < 3; i++) if ((e = cudaEventCreateWithFlags(&b->pipe_ev[i], cudaEventDisableTiming))) return cuda_fail(e, "cudaEventCreate");
@@ -834,7 +826,7 @@ void b2_recorder_destroy(b2_recorder* r) {
 
 int b2_warp_queue_histogram(b2_batch* b, int* hist16, void* stream) {
   if (!b || !hist16) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: null pointer");
-  if (b->warp_mode != 1 || !b->d_warp_sort) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: batch does not run on the warp engine's ordered queue");
+  if (b->warp_mode != 1) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: batch does not run on the warp engine's ordered queue");
   cudaError_t e = cudaSetDevice(b->device);
   if (!e) e = cudaStreamSynchronize((cudaStream_t)stream);
   int bins[64] = {0};

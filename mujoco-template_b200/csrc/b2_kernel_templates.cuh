@@ -12,15 +12,13 @@
 #include "../../include/b2mj.h"
 #include "b2_engine.cuh"
 
-// minimum resident blocks per SM requested for the FD kernel (caps registers per thread)
+// block size of the FD kernel and the minimum resident blocks per SM requested for it (caps registers per thread); the
+// generated translation units of small models set their own
 #ifndef B2_LIN_THREADS
 #define B2_LIN_THREADS 128
 #endif
 #ifndef B2_LIN_MIN_BLOCKS
 #define B2_LIN_MIN_BLOCKS 1
-#endif
-#ifndef B2_STEP_MIN_BLOCKS
-#define B2_STEP_MIN_BLOCKS 1
 #endif
 
 namespace b2 {
@@ -114,8 +112,8 @@ B2_DEV void lqr_law(const LaneEnv<T, D, M>& env, const T* q, const T* v, const T
 // nsteps x mj_step with ctrl held; nsteps == 0 means mj_forward (no integration).
 // The step loop is rolled: one inlined copy of the physics per kernel.
 template <typename T, class D, class M>
-__global__ void __launch_bounds__(128, B2_STEP_MIN_BLOCKS) k_step(StateDev<T> st, DerivedDev<T> out, int want_derived, int count, int N, int nsteps, const T* __restrict__ gain,
-                                                                  StateDev<T> park, const void* image = nullptr) {
+__global__ void __launch_bounds__(128, 1) k_step(StateDev<T> st, DerivedDev<T> out, int want_derived, int count, int N, int nsteps, const T* __restrict__ gain,
+                                                 StateDev<T> park, const void* image = nullptr) {
   model_load<M>(image, 0);
   // count envs are processed; N is the env stride of the SoA arrays (count < N for a chunk of a larger batch)
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -170,13 +168,20 @@ __global__ void __launch_bounds__(128, B2_STEP_MIN_BLOCKS) k_step(StateDev<T> st
   if (st.warm) { B2_UNROLL for (int k = 0; k < M::nv(); k++) st.warm[(size_t)k * N + e] = env.warm[k]; }
   if (st.flags && env.flags) st.flags[e] |= env.flags;
 }
+// Host launchers of k_step, k_linearize and k_jacobian, shared by the generic and the generated translation units: they
+// own the block size and the grid.  image: the runtime provider's model image (null for a static provider).
+// (Deduced return types: a launcher, and with it its kernel, is instantiated where it is called rather than at the end of
+// the translation unit, so the kernels keep their place in the module; cicc's inlining, and so the SASS of the other
+// kernels of the module, depends on that order.)
+template <typename T, class D, class M>
+auto launch_step(const void* image, const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain,
+                 const b2_state* park, void* stream) {
+  const int threads = 128, blocks = (count + threads - 1) / threads;
+  k_step<T, D, M><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<T>(st), to_dev<T>(out), out != nullptr, count, N, nsteps, (const T*)gain,
+                                                                to_dev<T>(park), image);
+  return (int)cudaGetLastError();
+}
 
-// number of FD threads per env (see k_linearize)
-// Euler: the nv + nu velocity / control columns are dealt out in groups of B2_FD_GROUP (one group if there are at most
-// that many: cartpole) -- each group is one thread that runs the shared position stage once -- followed by one thread
-// per position column.  Larger groups save more position stages but serialise more rollouts in one thread.
-// (B2_FD_GROUP, fd_group_count, fd_task_count: b2_model_dev.cuh, shared with the host launchers)
-template <class M> B2_DEV int fd_tasks() { return fd_task_count(M::integrator(), M::nv(), M::nu()); }
 // The nominal state of a thread's env is re-read from the SoA arrays at the start of every rollout (L1/L2 hits) rather
 // than held in registers: ~14 fewer live registers across the physics, which is what the 168-register budget of three
 // resident blocks is short of.  The controls are the exception (they may come from the control law, not from st.ctrl).
@@ -209,7 +214,7 @@ struct NominalWithSensors : NominalInMemory<T> {
 // With S::kSens (NominalWithSensors) the same rollouts also give the column of the sensor Jacobians, nom.dsdx =
 // d sensordata / dx (nsensordata, 2nv, N) for state columns and nom.dsdu = d sensordata / du (nsensordata, nu, N) for
 // control columns (either may be null).
-template <int PART, typename T, class D, class M, class S>
+template <typename T, class D, class M, class S>
 B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
                       T eps, T inv_eps, int centered, int N, int e, T* A, T* B, bool& pos_valid, bool& vel_valid) {
   constexpr int NQ = D::NQ, NV = D::NV;
@@ -223,8 +228,7 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
   for (int k = 0; k < 2 * nv; k++) dacc[k] = 0;
   int kind, i;
   bool fwd = true, back = centered != 0;
-  if (PART == 2) { kind = 1; i = c; }  // position-column kernel: the column kind is a compile-time fact
-  else if (nominal) { kind = 0; i = 0; fwd = back = false; }
+  if (nominal) { kind = 0; i = 0; fwd = back = false; }
   else if (c < nv) { kind = 1; i = c; }
   else if (c < ndx) { kind = 2; i = c - nv; }
   else {
@@ -295,8 +299,8 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
       }
     }
     if (M::integrator() == 1) env.rk4(); else env.euler();
-    vel_valid = PART != 2 && kind != 1 && kind != 2 && M::integrator() == 0;  // this rollout's velocity stage was the nominal one
-    pos_valid = PART != 2 && kind != 1 && M::integrator() == 0;
+    vel_valid = kind != 1 && kind != 2 && M::integrator() == 0;  // this rollout's velocity stage was the nominal one
+    pos_valid = kind != 1 && M::integrator() == 0;
     // plus -> s2, minus -> s1, nominal -> whichever end the one-sided quotient is missing
     const bool to2 = phase == 0 || (phase == 2 && !fwd);
     if (scalar_only) {
@@ -340,35 +344,20 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
 // differences at the ctrlrange bounds.
 // Work split: under Euler the velocity and control columns all share the position stage of the nominal qpos, so a
 // thread takes a group of up to B2_FD_GROUP of them, runs that stage once and then their rollouts (tasks 0..groups-1,
-// launched first: they are the longest); each position column is a thread of its own (two full rollouts).  RK4 models
-// have nothing to share between columns: one thread per (env, column).
-// register budget of the FD kernel: either through the resident-blocks hint or, with B2_LIN_MAXNREG, as an explicit cap
-// (ptxas settles on 168 registers for any hint between 3 x 128 and 5 x 64 threads per SM)
-// PART: 0 = one kernel for all FD tasks of an env; 1 = the velocity / control groups (+ the env advance) only; 2 = the
-// position columns only.  The split exists for the register budget: a position-column thread runs two full rollouts and
-// keeps nothing across them -- 168 registers without a spill, 12 warps per SM -- while the group thread keeps the position
-// stage and both factorisations alive across up to seven rollouts and needs 253 (8 warps per SM); one kernel for both has
-// to take the larger budget for all its threads.
-#ifndef B2_LINP_THREADS
-#define B2_LINP_THREADS 128
-#endif
-#ifndef B2_LINP_MIN_BLOCKS
-#define B2_LINP_MIN_BLOCKS 3
-#endif
-#ifdef B2_LIN_MAXNREG
-#define B2_LIN_BOUNDS(PART) __maxnreg__(B2_LIN_MAXNREG)
-#else
-#define B2_LIN_BOUNDS(PART) __launch_bounds__((PART) == 2 ? B2_LINP_THREADS : B2_LIN_THREADS, (PART) == 2 ? B2_LINP_MIN_BLOCKS : B2_LIN_MIN_BLOCKS)
-#endif
+// launched first: they are the longest); each position column is a thread of its own (two full rollouts).  Larger
+// groups save more position stages but serialise more rollouts in one thread.  RK4 models have nothing to share between
+// columns: one thread per (env, column).  fd_task_count (b2_model_dev.cuh) gives the threads per env.
+// (Splitting the launch into a kernel for the groups and one for the position columns, each with its own register budget,
+// was measured on the cartpole tick and rejected: profiles/ab_cartpole_lin_split_r03c.txt.)
 // SENS (b2_linearize_sensors): the rollouts also produce the sensor Jacobians dsdx (nsensordata, 2nv, N) and dsdu
 // (nsensordata, nu, N), layout as A / B; launched with gain == nullptr and no shadow (no control law, no env advance).
-template <typename T, class D, class M, int PART = 0, bool SENS = false>
-__global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N, T eps, int centered, T* A, T* B, const T* __restrict__ gain, StateDev<T> shadow,
-                                                                                 const void* image = nullptr, T* dsdx = nullptr, T* dsdu = nullptr) {
+template <typename T, class D, class M, bool SENS = false>
+__global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize(StateDev<T> st, int count, int N, T eps, int centered, T* A, T* B, const T* __restrict__ gain,
+                                                                                 StateDev<T> shadow, const void* image = nullptr, T* dsdx = nullptr, T* dsdu = nullptr) {
   model_load<M>(image, 0);
   const int nq = M::nq(), nv = M::nv(), nu = M::nu(), ndx = 2 * nv;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const int ntask = PART == 0 ? fd_tasks<M>() : (PART == 1 ? fd_group_count(nv, nu) : nv);
+  const int ntask = fd_task_count(M::integrator(), nv, nu);
   const long long total = (long long)count * ntask;
   if (idx >= total) return;
   // count envs, env stride N; task-major.  32-bit division when the launch fits (a 64-bit one is ~100 instructions)
@@ -396,15 +385,14 @@ __global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N
   const bool grouped = M::integrator() == 0;  // not a constant expression for the runtime provider
   const int groups = fd_group_count(nv, nu);
   int c0 = task, c1 = task + 1;
-  if (PART == 2) { c0 = task; c1 = task + 1; }
-  else if (grouped) {
+  if (grouped) {
     if (task < groups) { c0 = nv + task * B2_FD_GROUP; c1 = c0 + B2_FD_GROUP < ndx + nu ? c0 + B2_FD_GROUP : ndx + nu; }
     else { c0 = task - groups; c1 = c0 + 1; }
   }
   // shadow.qpos != null (grouped form only): the thread of the velocity / control columns also advances the env -- its
   // position stage is the step's -- and leaves the new state in the shadow arrays (the other threads of the env still
   // read the nominal state); k_commit_state swaps the two afterwards
-  const bool advance = PART != 2 && grouped && task == 0 && shadow.qpos != nullptr;
+  const bool advance = grouped && task == 0 && shadow.qpos != nullptr;
   bool pos_valid = false, vel_valid = false;
   const T inv_eps = T(1) / eps;
   // mj_checkPos / mj_checkVel once on the nominal state (an eps perturbation of a finite state is finite)
@@ -418,7 +406,7 @@ __global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N
   B2_NOUNROLL
   for (int c = c0; c < c1 + (advance ? 1 : 0) && !frozen; c++) {
     const bool nominal = c == c1;  // the advance comes after the group's columns, on the same position stage
-    fd_column<PART>(env, nom, nominal ? ndx + nu : c, nominal, eps, inv_eps, centered, N, e, A, B, pos_valid, vel_valid);
+    fd_column(env, nom, nominal ? ndx + nu : c, nominal, eps, inv_eps, centered, N, e, A, B, pos_valid, vel_valid);
   }
   if (advance) {
     B2_UNROLL
@@ -429,6 +417,17 @@ __global__ void B2_LIN_BOUNDS(PART) k_linearize(StateDev<T> st, int count, int N
     for (int k = 0; k < nu; k++) shadow.ctrl[(size_t)k * N + e] = u0[k];
   }
   if (st.flags && env.flags) atomicOr(st.flags + e, env.flags);
+}
+// ntask: FD threads per env, fd_task_count of the model (an argument: a runtime provider's accessors read shared memory).
+// The block size is the one the kernel's __launch_bounds__ were compiled for.
+template <typename T, class D, class M, bool SENS = false>
+auto launch_linearize(const void* image, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A, void* B,
+                      const void* gain, const b2_state* shadow, void* dsdx, void* dsdu, void* stream) {
+  const long long total = (long long)count * ntask;
+  const int blocks = (int)((total + B2_LIN_THREADS - 1) / B2_LIN_THREADS);
+  k_linearize<T, D, M, SENS><<<blocks, B2_LIN_THREADS, 0, (cudaStream_t)stream>>>(to_dev<T>(st), count, N, (T)eps, centered, (T*)A, (T*)B, (const T*)gain,
+                                                                                  to_dev<T>(shadow), image, (T*)dsdx, (T*)dsdu);
+  return (int)cudaGetLastError();
 }
 
 // After a launch that advanced envs into the shadow arrays: swap state and shadow (rows of count elements, row stride N).
@@ -489,6 +488,12 @@ __global__ void __launch_bounds__(128) k_jacobian(StateDev<T> st, int N, int kin
   }
   if (jacp) { B2_UNROLL for (int k = 0; k < 3 * nv; k++) jacp[(size_t)k * N + e] = jp[k]; }
   if (jacr) { B2_UNROLL for (int k = 0; k < 3 * nv; k++) jacr[(size_t)k * N + e] = jr[k]; }
+}
+template <typename T, class D, class M>
+auto launch_jacobian(const void* image, const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {
+  const int threads = 128, blocks = (N + threads - 1) / threads;
+  k_jacobian<T, D, M><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<T>(st), N, kind, objid, (T*)jacp, (T*)jacr, image);
+  return (int)cudaGetLastError();
 }
 
 // mj_inverse for a prescribed acceleration (steady_ctrl0: reference mujoco_template/setpoints.py:23-30);

@@ -115,10 +115,9 @@ double B2_FN(b2k_fma_peak)(void* stream) {
 }
 int B2_FN(b2k_step)(const void* image, int cls, const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain,
                     const b2_state* park, void* stream) {
-  const int threads = 128, blocks = (count + threads - 1) / threads;
-  B2_DISPATCH(cls, (k_step<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
-                       to_dev<real>(st), to_dev<real>(out), out != nullptr, count, N, nsteps, (const real*)gain, to_dev<real>(park), image)));
-  return (int)cudaGetLastError();
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_step<real, DD, RuntimeModel<DD>>(image, st, out, count, N, nsteps, gain, park, stream)));
+  return rc;
 }
 // ---- warp engine (large models): launch geometry and per-warp scratch are sized by the host
 // Sizes with a compiled-in kernel variant (every workspace offset and loop bound a constant): the humanoid's.
@@ -133,7 +132,6 @@ static int view_maxdepth(const b2m_view* v) {
   return best;
 }
 static bool dims_are_humanoid(const b2m_view* v) {
-  if (const char* x = getenv("B2_WARP_STATIC_DIMS")) if (x[0] == '0') return false;
   typedef DimsHumanoid H;
   return v->nq == H::NQ && v->nv == H::NV && v->nu == H::NU && v->nbody == H::NB && v->njnt == H::NJ && v->ngeom == H::NG &&
          v->ntendon == H::NT && view_maxdepth(v) == H::DEPTH;
@@ -142,23 +140,9 @@ static bool dims_are_humanoid(const b2m_view* v) {
   if (dims_are_humanoid(v)) { typedef ImageModel<real, DimsHumanoid> WM; CALL; } \
   else { typedef ImageModel<real, DimsRuntime> WM; CALL; }
 
-// lock-step mode of the warp kernels (WarpEnv::forward<LS>): 1 = every stage and every Newton round behind the block
-// barrier, 2 = stages only (the Newton loop runs free), 0 = none.  Measured on the humanoid (200-step rollout, blocks of four
-// warps, cost-ordered queue): mode 2 7.44e6 env-steps/s, mode 1 7.30e6 -- the Newton loop's code is small enough to stay
-// in the instruction cache, and a warp no longer waits for its block mates in every round.
-#ifndef B2_WARP_LS_MODE
-#define B2_WARP_LS_MODE 2
-#endif
 static int warp_ws_reals_of(const b2m_view* v) { return warp_ws_reals(v->nq, v->nv, v->nu, v->nbody, v->njnt, v->ngeom, v->ntendon); }
 static size_t warp_block_smem(const b2m_view* v, int wpb, int extra_reals) {
-  size_t extra = 0;
-  if (const char* x = getenv("B2_WARP_EXTRA_SMEM")) extra = (size_t)atoi(x);  // tuning: lowers the resident blocks per SM
-  return extra + (size_t)wpb * ((size_t)warp_ws_reals_of(v) + extra_reals) * sizeof(real);
-}
-static int warp_wpb() {  // warps (envs) per lock-step block: 4 x 128 registers = 16 resident warps per SM, four to a fetch
-  int wpb = 4;
-  if (const char* x = getenv("B2_WARP_LS_WPB")) { const int w = atoi(x); if (w >= 1 && w <= 8) wpb = w; }
-  return wpb;
+  return (size_t)wpb * ((size_t)warp_ws_reals_of(v) + extra_reals) * sizeof(real);
 }
 template <class K>
 static int warp_occupancy(K kern, int wpb, size_t smem, int* per_sm) {
@@ -178,16 +162,15 @@ int B2_FN(b2k_warp_plan)(const b2m_view* v, int N, int* out_wpb, int* out_blocks
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  int wpb = warp_wpb();
+  int wpb = 4;  // warps (envs) per lock-step block: 4 x 128 registers = 16 resident warps per SM, four to a fetch
   while (wpb > 1 && warp_block_smem(v, wpb, 0) + 1024 > (size_t)smem_max) wpb--;
   const size_t smem = warp_block_smem(v, wpb, 0);
   int per_sm = 0, rc = 0;
-  B2_WARP_DIMS(v, (rc = warp_occupancy(k_warp_step_ls<real, WM, B2_WARP_LS_MODE>, wpb, smem, &per_sm)));
+  B2_WARP_DIMS(v, (rc = warp_occupancy(k_warp_step_ls<real, WM>, wpb, smem, &per_sm)));
   if (rc) return -1;
   int blocks = sms * per_sm;
   const int need = (N + wpb - 1) / wpb;
   if (blocks > need) blocks = need;
-  if (getenv("B2_WARP_DEBUG")) fprintf(stderr, "[b2mj] warp plan: %d warps/block, %d blocks/SM, %zu B shared memory/block, static dims %d\n", wpb, per_sm, smem, (int)dims_are_humanoid(v));
   *out_wpb = wpb; *out_blocks = blocks;
   return blocks * wpb;
 }
@@ -213,7 +196,7 @@ int B2_FN(b2k_warp_step)(const void* image, const b2m_view* v, const b2_state* s
     k_cost_hist<kCostBins><<<sb, 256, 0, s>>>(cost, N, hist);
     k_cost_scatter<kCostBins><<<sb, 256, 0, s>>>(cost, N, hist, hist + kCostBins, perm);
   }
-  B2_WARP_DIMS(v, (k_warp_step_ls<real, WM, B2_WARP_LS_MODE><<<blocks, wpb * 32, smem, s>>>(
+  B2_WARP_DIMS(v, (k_warp_step_ls<real, WM><<<blocks, wpb * 32, smem, s>>>(
                       (const WarpImage<real>*)image, to_dev<real>(st), to_dev<real>(out), out != nullptr, N, nsteps, (real*)jscratch, (int*)counter,
                       perm, cost, to_dev<real>(park))));
   return (int)cudaGetLastError();
@@ -225,35 +208,30 @@ int B2_FN(b2k_warp_linearize)(const void* image, const b2m_view* v, const b2_sta
   int per_sm = 0, dev = 0, sms = 0, rc = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  B2_WARP_DIMS(v, (rc = warp_occupancy(k_warp_linearize<real, WM, B2_WARP_LS_MODE>, wpb, smem, &per_sm)));
+  B2_WARP_DIMS(v, (rc = warp_occupancy(k_warp_linearize<real, WM>, wpb, smem, &per_sm)));
   if (rc) return (int)cudaErrorLaunchOutOfResources;
   if (blocks > sms * per_sm) blocks = sms * per_sm;  // persistent: never more blocks than fit at once (scratch slots are per block)
   cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(int), (cudaStream_t)stream);
   if (e != cudaSuccess) return (int)e;
-  B2_WARP_DIMS(v, (k_warp_linearize<real, WM, B2_WARP_LS_MODE><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(
+  B2_WARP_DIMS(v, (k_warp_linearize<real, WM><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(
                       (const WarpImage<real>*)image, to_dev<real>(st), N, (real)eps, centered, (real*)A, (real*)B, (real*)jscratch, (int*)counter)));
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_linearize)(const void* image, int cls, const b2_state* st, int count, int N, int ncol, double eps, int centered, void* A, void* B,
+// ntask: FD tasks per env (fd_task_count of the model)
+int B2_FN(b2k_linearize)(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A, void* B,
                          const void* gain, const b2_state* shadow, void* stream) {
-  const int threads = 128;
-  const long long total = (long long)count * ncol;  // ncol: FD tasks per env (b2_capi: nv + 1 under Euler, else 2nv + nu)
-  const int blocks = (int)((total + threads - 1) / threads);
-  B2_DISPATCH(cls, (k_linearize<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
-                       to_dev<real>(st), count, N, (real)eps, centered, (real*)A, (real*)B, (const real*)gain, to_dev<real>(shadow), image)));
-  return (int)cudaGetLastError();
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_linearize<real, DD, RuntimeModel<DD>>(image, st, count, N, ntask, eps, centered, A, B, gain, shadow, nullptr,
+                                                                      nullptr, stream)));
+  return rc;
 }
 // (A, B) and the sensor Jacobians from the same rollouts (k_linearize<..., SENS = true>); no control law, no env advance
-int B2_FN(b2k_linearize_sensors)(const void* image, int cls, const b2_state* st, int count, int N, int ncol, double eps, int centered, void* A,
+int B2_FN(b2k_linearize_sensors)(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A,
                                  void* B, void* dsdx, void* dsdu, void* stream) {
-  const int threads = 128;
-  const long long total = (long long)count * ncol;
-  const int blocks = (int)((total + threads - 1) / threads);
-  const b2_state* no_shadow = nullptr;
-  B2_DISPATCH(cls, (k_linearize<real, DD, RuntimeModel<DD>, 0, true><<<blocks, threads, 0, (cudaStream_t)stream>>>(
-                       to_dev<real>(st), count, N, (real)eps, centered, (real*)A, (real*)B, nullptr, to_dev<real>(no_shadow), image,
-                       (real*)dsdx, (real*)dsdu)));
-  return (int)cudaGetLastError();
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_linearize<real, DD, RuntimeModel<DD>, true>(image, st, count, N, ntask, eps, centered, A, B, nullptr, nullptr,
+                                                                            dsdx, dsdu, stream)));
+  return rc;
 }
 int B2_FN(b2k_commit_state)(const b2_state* st, const b2_state* shadow, int count, int N, int nq, int nv, int nu, void* stream) {
   int bx = (count + 255) / 256;
@@ -262,10 +240,9 @@ int B2_FN(b2k_commit_state)(const b2_state* st, const b2_state* shadow, int coun
   return (int)cudaGetLastError();
 }
 int B2_FN(b2k_jacobian)(const void* image, int cls, const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {
-  const int threads = 128, blocks = (N + threads - 1) / threads;
-  B2_DISPATCH(cls, (k_jacobian<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
-                       to_dev<real>(st), N, kind, objid, (real*)jacp, (real*)jacr, image)));
-  return (int)cudaGetLastError();
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_jacobian<real, DD, RuntimeModel<DD>>(image, st, N, kind, objid, jacp, jacr, stream)));
+  return rc;
 }
 int B2_FN(b2k_inverse)(const void* image, int cls, const b2_state* st, int N, const void* qacc, void* qfrc, void* moment, void* stream) {
   const int threads = 128, blocks = (N + threads - 1) / threads;
@@ -283,19 +260,16 @@ int B2_FN(b2k_lqr_control)(const void* image, int cls, const b2_state* st, int c
 int B2_FN(b2k_dare)(const void* A, const void* B, const void* qr /* device: Q, R, Rinv */, int nx, int nu, int N, int max_doublings,
                     double tol, void* K, void* P, int* status, void* stream) {
   const real* qd = (const real*)qr;
-  // small systems: one env per thread, compile-time sizes (B2_DARE_WARP=1 forces the warp kernel)
-  const char* force_warp = getenv("B2_DARE_WARP");
-  if (!(force_warp && force_warp[0] == '1')) {
-#define B2_DARE_SMALL(NX_, NU_)                                                                                                   \
-    if (nx == NX_ && nu == NU_) {                                                                                                 \
-      k_dare_small<real, NX_, NU_><<<(N + 63) / 64, 64, 0, (cudaStream_t)stream>>>((const real*)A, (const real*)B, qd, qd + nx * nx, \
-                                                                                  qd + nx * nx + nu * nu, N, max_doublings, (real)tol,   \
-                                                                                  (real*)K, (real*)P, status);                     \
-      return (int)cudaGetLastError();                                                                                             \
-    }
-    B2_DARE_SMALL(2, 1) B2_DARE_SMALL(4, 1) B2_DARE_SMALL(4, 2)
-#undef B2_DARE_SMALL
+  // small systems: one env per thread, compile-time sizes
+#define B2_DARE_SMALL(NX_, NU_)                                                                                                 \
+  if (nx == NX_ && nu == NU_) {                                                                                                 \
+    k_dare_small<real, NX_, NU_><<<(N + 63) / 64, 64, 0, (cudaStream_t)stream>>>((const real*)A, (const real*)B, qd, qd + nx * nx, \
+                                                                                qd + nx * nx + nu * nu, N, max_doublings, (real)tol,   \
+                                                                                (real*)K, (real*)P, status);                     \
+    return (int)cudaGetLastError();                                                                                             \
   }
+  B2_DARE_SMALL(2, 1) B2_DARE_SMALL(4, 1) B2_DARE_SMALL(4, 2)
+#undef B2_DARE_SMALL
   int dev = 0, smem_max = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);

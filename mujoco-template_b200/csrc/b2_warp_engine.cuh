@@ -306,7 +306,6 @@ struct WarpEnv {
   // dyn_list the merged ancestor lists in the scratch slot (merge_branches) -- instead of falling back to a dense
   // Cholesky (round 1 and the first half of round 2: 17 % of the executed instructions once humanoids lie on the floor).
   bool rows_cross;
-  int solve_cycles;  // clock cycles this env spent in its last constraint stage: the work queue's sort key
   unsigned tree_mask, amask;
   int* dyn_nanc;
   unsigned char* dyn_list;
@@ -1117,74 +1116,60 @@ struct WarpEnv {
     __syncwarp();
     solve_H(H, Mgrad);
   }
-  // LS ("lock step"): the warps of a block run the same stage at the same time, separated by block barriers, so that
-  // one instruction fetch from L2 serves all of them.  The kernel is bound by instruction-fetch bandwidth: its 276 KB of
+  // Lock step: the warps of a block run the same stage at the same time, separated by block barriers, so that one
+  // instruction fetch from L2 serves all of them.  The kernel is bound by instruction-fetch bandwidth: its 276 KB of
   // SASS cannot stay in the 32 KB L1.5 instruction cache, and two resident warps per SM already reach 69 % of the
-  // throughput of eight that run out of phase.
-  // LS: 0 none, 1 everywhere, 2 not inside the Newton loop.  The lock-step group is the whole block and the barrier is
-  // barrier 0: a register-valued barrier id makes ptxas reserve all 16 barriers per block, which caps an SM at four
-  // blocks whatever the registers and shared memory would allow (ncu "Block Limit Barriers", profiles/ncu_hum_step_r01j.txt).
-  template <int LS> B2_DEV void stage_sync() const {
-    if (LS) __syncthreads();
-  }
-  B2_DEV bool group_or(bool p) const { return __syncthreads_or((int)p) != 0; }
-  template <int LS>
+  // throughput of eight that run out of phase.  The Newton loop runs free (no barrier per round): measured on the
+  // humanoid (200-step rollout, blocks of four warps, cost-ordered queue) 7.44e6 env-steps/s against 7.30e6 with a barrier
+  // in every round -- the loop's code is small enough to stay in the instruction cache, and a warp no longer waits for its
+  // block mates.  The lock-step group is the whole block and the barrier is barrier 0: a register-valued barrier id makes
+  // ptxas reserve all 16 barriers per block, which caps an SM at four blocks whatever the registers and shared memory
+  // would allow (ncu "Block Limit Barriers", profiles/ncu_hum_step_r01j.txt).
+  B2_DEV void stage_sync() const { __syncthreads(); }
   B2_DEV void constrained_acceleration() {
     const int nv = mdl.nv();
-#ifdef B2_WARP_KEY_CYCLES
-    const long long t_begin = clock64();
-#endif
     niter = 0;
     bool done = false;
     if (!nefc) {
       WFOR(k, nv) { qacc[k] = a_smooth[k]; warm[k] = a_smooth[k]; f_con[k] = 0; }
       __syncwarp();
-      solve_cycles = 0;
-      if (LS != 1) return;
-      done = true;
-    } else {
-      row_params();
-      hess_valid = false;
-      WFOR(k, nv) qacc[k] = warm[k];
+      return;
+    }
+    row_params();
+    hess_valid = false;
+    WFOR(k, nv) qacc[k] = warm[k];
+    __syncwarp();
+    mul_J(Jaref, qacc, row_aref);
+    T cw = row_cost(Jaref);
+    mul_M(Ma, qacc);
+    T g = 0;
+    WFOR(k, nv) g += T(0.5) * (Ma[k] - f_smooth[k]) * (qacc[k] - a_smooth[k]);
+    cw += warp_sum(g);
+    mul_J(Jv, a_smooth, row_aref);
+    const T cs = row_cost(Jv);
+    if (cw > cs) {
+      WFOR(k, nv) qacc[k] = a_smooth[k];
+      WFOR(i, nefc) Jaref[i] = Jv[i];
       __syncwarp();
-      mul_J(Jaref, qacc, row_aref);
-      T cw = row_cost(Jaref);
       mul_M(Ma, qacc);
-      T g = 0;
-      WFOR(k, nv) g += T(0.5) * (Ma[k] - f_smooth[k]) * (qacc[k] - a_smooth[k]);
-      cw += warp_sum(g);
-      mul_J(Jv, a_smooth, row_aref);
-      const T cs = row_cost(Jv);
-      if (cw > cs) {
-        WFOR(k, nv) qacc[k] = a_smooth[k];
-        WFOR(i, nefc) Jaref[i] = Jv[i];
-        __syncwarp();
-        mul_M(Ma, qacc);
-      }
     }
     const T scale = T(1) / (mdl.meaninertia() * T(nv > 1 ? nv : 1));
     T old = 0;
     bool first = true;
-    while (true) {
-      // lock step: every warp of the block takes part in every round until the slowest env has converged
-      if (LS == 1) { if (!group_or(!done)) break; }
-      else if (done) break;
-      if (!done) {
-        newton_gradient();
-        if (!first) {
-          const T gn = dotv(grad, grad);
-          niter++;
-          if (scale * (old - cost) < mdl.tolerance() || scale * sqrt(gn) < mdl.tolerance()) done = true;
-        }
-        if (!done && niter >= mdl.iterations()) done = true;  // iteration cap: the iterate stands, no further search
-        if (!done) {
-          newton_direction();
-          first = false;
-          WFOR(k, nv) search[k] = -Mgrad[k];
-          __syncwarp();
-        }
+    while (!done) {
+      newton_gradient();
+      if (!first) {
+        const T gn = dotv(grad, grad);
+        niter++;
+        if (scale * (old - cost) < mdl.tolerance() || scale * sqrt(gn) < mdl.tolerance()) done = true;
       }
-      stage_sync<LS == 1>();
+      if (!done && niter >= mdl.iterations()) done = true;  // iteration cap: the iterate stands, no further search
+      if (!done) {
+        newton_direction();
+        first = false;
+        WFOR(k, nv) search[k] = -Mgrad[k];
+        __syncwarp();
+      }
       if (!done) {
         const T alpha = line_search();
         if (alpha == 0) done = true;
@@ -1196,44 +1181,39 @@ struct WarpEnv {
         }
       }
     }
-    if (nefc) {
-      WFOR(k, nv) warm[k] = qacc[k];
-      __syncwarp();
-    }
-#ifdef B2_WARP_KEY_CYCLES
-    solve_cycles = (int)(clock64() - t_begin);  // this env's own constraint-stage time (no block barrier inside when LS != 1)
-#endif
+    WFOR(k, nv) warm[k] = qacc[k];
+    __syncwarp();
   }
 
   // ------------------------------------------------------------------ forward + Euler
   // after_position(): called once the position-dependent arrays (xpos .. geom_xpos, com) are complete and before their
   // storage is reused -- the kernels export the derived outputs there.
-  template <int LS, class F>
+  template <class F>
   B2_DEV void forward(F&& after_position) {
     const int nv = mdl.nv(), np = nv * (nv + 1) / 2;
     kinematics();
-    stage_sync<LS>();
+    stage_sync();
     collide();
-    stage_sync<LS>();
+    stage_sync();
     com_frame();
     after_position();
-    stage_sync<LS>();
+    stage_sync();
     make_rows();
-    stage_sync<LS>();
+    stage_sync();
     mass_matrix();  // from here on region X holds the dynamics arrays
-    stage_sync<LS>();
+    stage_sync();
     velocities();
     passive_forces();
-    stage_sync<LS>();
+    stage_sync();
     bias_forces();
     WFOR(e, np) LDp[e] = Mp[e];  // ... and from here on the factor and the solver vectors
     __syncwarp();
-    stage_sync<LS>();
+    stage_sync();
     factor_LD();
-    stage_sync<LS>();
+    stage_sync();
     smooth_dynamics();
-    stage_sync<LS>();
-    constrained_acceleration<LS>();
+    stage_sync();
+    constrained_acceleration();
   }
   B2_DEV void check_state() {
     int bad = 0;

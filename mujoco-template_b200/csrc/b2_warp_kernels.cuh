@@ -89,10 +89,10 @@ __global__ void __launch_bounds__(256) k_cost_scatter(const int* __restrict__ co
 
 // nsteps x mj_step (nsteps == 0: mj_forward), one env per warp, persistent over envs: the first gridDim * wpb envs are
 // assigned statically, the rest through an atomic work queue (env costs differ with contacts and Newton iterations).
-// The warps of a block run their envs stage by stage behind the block barrier (WarpEnv::forward<LS>), so that one
+// The warps of a block run their envs stage by stage behind the block barrier (WarpEnv::forward), so that one
 // instruction fetch serves all of them; warps without an env of their own at the tail of the batch recompute the last env
 // and discard the result, so that every warp reaches every barrier.
-template <typename T, class M, int LS>
+template <typename T, class M>
 __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_step_ls(const WarpImage<T>* __restrict__ img, StateDev<T> st, DerivedDev<T> out,
                                                             int want_derived, int N, int nsteps, T* jscratch, int* queue,
                                                             const int* __restrict__ perm, int* cost, StateDev<T> park) {
@@ -132,10 +132,10 @@ __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_step_ls(const WarpImage<T>* 
         __syncwarp();
       }
       const bool store = want_derived && s == total - 1 && mine && !frozen;
-      env.template forward<LS>([&] { if (store) warp_store_position(env, out, N, e); });
+      env.forward([&] { if (store) warp_store_position(env, out, N, e); });
       env.check_acc();
       if (store) warp_store_solution(env, out, N, e);
-      env.template stage_sync<LS>();
+      env.stage_sync();
       if (nsteps > 0) env.euler();
     }
     if (mine && !frozen) {
@@ -148,17 +148,13 @@ __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_step_ls(const WarpImage<T>* 
     }
     // queue key of the next step: Newton rounds of this one, envs whose rows couple two branches of the tree (merged
     // ancestor lists: longer factorisation sweeps) in the upper half of the bins.  (The measured cycle count of the env's
-    // constraint stage as the key -- B2_WARP_KEY_CYCLES, 16 K / 32 K-cycle bins -- was 4 % slower: 7.7e6 against 8.0e6
-    // env-steps/s; the clock also counts the time the warp waits for its SM's other warps.)
-#ifdef B2_WARP_KEY_CYCLES
-    if (mine && cost && lane == 0) cost[e] = frozen ? 0 : (env.solve_cycles >> B2_WARP_KEY_CYCLES);
-#else
+    // constraint stage as the key, in 16 K / 32 K-cycle bins, was 4 % slower: 7.7e6 against 8.0e6 env-steps/s; the clock
+    // also counts the time the warp waits for its SM's other warps.)
     if (mine && cost && lane == 0) {
       int key = ((env.nefc && env.rows_cross) ? 8 : 0) + (env.niter < 7 ? env.niter : 7);
       if (kCostBins == 64) key = key * 4 + (env.nefc < 12 ? 0 : (env.nefc < 24 ? 1 : (env.nefc < 36 ? 2 : 3)));
       cost[e] = frozen ? 0 : key;
     }
-#endif
     if (threadIdx.x == 0) s_next = nw + atomicAdd(queue, wpb);
     __syncthreads();
     first = s_next;
@@ -171,7 +167,7 @@ __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_step_ls(const WarpImage<T>* 
 // nominal state: plus / minus for a centred column, plus (or minus) and the nominal step where a control sits at its
 // range bound (mjd_transitionFD's one-sidedness, as k_linearize).  Every rollout restores qacc_warmstart.  The columns go
 // to A (2nv x 2nv x N) and B (2nv x nu x N), env fastest.  extra = 2 (nq + nv) reals per warp hold the two end states.
-template <typename T, class M, int LS>
+template <typename T, class M>
 __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_linearize(const WarpImage<T>* __restrict__ img, StateDev<T> st, int N, T eps, int centered,
                                                               T* A, T* B, T* jscratch, int* queue) {
   extern __shared__ double b2_smem[];
@@ -223,9 +219,9 @@ __global__ void __maxnreg__(B2_WARP_REGS(M)) k_warp_linearize(const WarpImage<T>
       }
       __syncwarp();
       env.check_state();
-      env.template forward<LS>([] {});
+      env.forward([] {});
       env.check_acc();
-      env.template stage_sync<LS>();
+      env.stage_sync();
       env.euler();
       flags_all |= env.flags;
       T* dst = ends[side];

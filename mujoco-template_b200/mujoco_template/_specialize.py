@@ -39,19 +39,12 @@ REAL_ARRAYS = ("gravity", "wind", "body_pos", "body_quat", "body_ipos", "body_iq
                "actuator_forcerange", "actuator_gainprm", "actuator_biasprm", "pair_margin", "pair_gap", "pair_friction",
                "pair_solref", "pair_solimp", "sensor_cutoff")
 
-# FD kernel block shape for small models: (threads per block, min resident blocks per SM).  64 x 4 lets ptxas use 253
-# registers -- the cartpole FD kernel then has no spills at all -- at 8 warps per SM, in blocks small enough that the last
+# FD kernel block shape for small models (nv <= 2): (threads per block, min resident blocks per SM).  64 x 4 lets ptxas use
+# 253 registers -- the cartpole FD kernel then has no spills at all -- at 8 warps per SM, in blocks small enough that the last
 # wave of the launch is short: 36.4 us against 38.6 us for 128 x 3 (168 registers, 320 B of spills, 12 warps); explicit caps
 # in between (184 / 200 / 216 registers at 9-11 warps) are all slower (round 2, profiles/ab_cartpole_lin_shapes_r02k.txt).
-import os as _os
-LIN_SHAPE = tuple(int(x) for x in _os.environ.get("B2_LIN_SHAPE", "64,4").split(","))
-# B2_LIN_SPLIT=1 (build-time experiment, Euler models with nv <= 2): the FD launch as two kernels, the velocity / control
-# groups (LIN_SHAPE, 253 registers) and the position columns (LINP_SHAPE: 168 registers without a spill, 12 warps per SM).
-# Measured on the cartpole tick: +2 % device-timed when the two run back to back on one stream (1.65e9 against 1.62e9
-# env-steps/s), nothing when they overlap on two streams (the fork / join costs what the overlap gains), and -6 % end to end
-# (the PCIe write pipeline of the direct (A, B) stores drains between the launches).  Off by default.
-LINP_SHAPE = tuple(int(x) for x in _os.environ.get("B2_LINP_SHAPE", "128,3").split(","))
-LIN_SPLIT = _os.environ.get("B2_LIN_SPLIT", "0") == "1"
+# Larger models keep the kernel's default, 128 x 1.
+SMALL_LIN_SHAPE = (64, 4)
 
 _MAX_CONTACTS = {(0, 2): 1, (0, 3): 2, (0, 6): 4, (0, 4): 1, (2, 2): 1, (2, 3): 1, (3, 3): 2}
 
@@ -124,17 +117,9 @@ def emit_spec(compiled: dict, name: str) -> str:
     A(f"// GENERATED by mujoco_template/_specialize.py for model '{name}' -- do not edit.")
     A("// Static model provider: every accessor folds to a compile-time constant after unrolling.")
     A("#define B2_STATIC_MODEL 1")
-    # small models: ask for >= 3 resident blocks/SM in the FD kernel (<= 168 registers, measured best on B200)
-    lin_threads, lin_blocks = (LIN_SHAPE if nv <= 2 else (128, 1))
-    linp_threads, linp_blocks = LINP_SHAPE
-    lin_split = LIN_SPLIT and nv <= 2 and int(c["integrator"]) == 0
+    lin_threads, lin_blocks = SMALL_LIN_SHAPE if nv <= 2 else (128, 1)
     A(f"#define B2_LIN_THREADS {lin_threads}")
     A(f"#define B2_LIN_MIN_BLOCKS {lin_blocks}")
-    A(f"#define B2_LINP_THREADS {linp_threads}")
-    A(f"#define B2_LINP_MIN_BLOCKS {linp_blocks}")
-    ncol = 2 * nv + nu
-    # k_linearize: Euler deals the velocity / control columns out in groups of B2_FD_GROUP = 4 (b2_kernel_templates.cuh)
-    fd_tasks = (nv + nu + 3) // 4 + nv if int(c["integrator"]) == 0 else ncol
     # the sensor-Jacobian FD launcher exists only for models with sensors (the others' C-ABI call is b2_linearize), so the
     # generated sources of sensorless models do not change with it
     has_sensors = int(c["nsensordata"]) > 0
@@ -165,41 +150,24 @@ def emit_spec(compiled: dict, name: str) -> str:
         A(f"  static B2_DEV T {k}(int i) {{ static constexpr T t[{one(v.size)}] = {{{body}}}; return t[i]; }}")
     A("};")
     A("")
+    # launchers: b2_kernel_templates.cuh's launch_* own block size and grid; the FD task count is the kernel's own rule,
+    # evaluated on the host from the provider's constexpr accessors
     for T, suf in (("double", ""), ("float", "32")):
+        M = f"{T}, SDims, SModel<{T}>"
+        ntask = f"fd_task_count(SModel<{T}>::integrator(), SModel<{T}>::nv(), SModel<{T}>::nu())"
         A(f"int spec_step{suf}(const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain, const b2_state* park, void* stream) {{")
-        A("  const int threads = 128, blocks = (count + threads - 1) / threads;")
-        A(f"  k_step<{T}, SDims, SModel<{T}>><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), to_dev<{T}>(out), out != nullptr, count, N, nsteps, (const {T}*)gain, to_dev<{T}>(park));")
-        A("  return (int)cudaGetLastError();")
+        A(f"  return launch_step<{M}>(nullptr, st, out, count, N, nsteps, gain, park, stream);")
         A("}")
         A(f"int spec_linearize{suf}(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, const void* gain, const b2_state* shadow, void* stream) {{")
-        if lin_split:
-            # two launches on the same stream: the velocity / control groups (253 registers, they also advance the env), then
-            # the position columns (168 registers without a spill: 12 warps per SM) -- see k_linearize's PART
-            groups = (nv + nu + 3) // 4
-            A("  cudaStream_t s = (cudaStream_t)stream, side = s;")
-            A(f"  const int threads = {lin_threads}; const long long total = (long long)count * {groups};")
-            A(f"  k_linearize<{T}, SDims, SModel<{T}>, 1><<<(int)((total + threads - 1) / threads), threads, 0, s>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, (const {T}*)gain, to_dev<{T}>(shadow));")
-            A(f"  const int threads_p = {linp_threads}; const long long total_p = (long long)count * {nv};")
-            A(f"  k_linearize<{T}, SDims, SModel<{T}>, 2><<<(int)((total_p + threads_p - 1) / threads_p), threads_p, 0, side>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, (const {T}*)gain, to_dev<{T}>(shadow));")
-        else:
-            A(f"  const int threads = {lin_threads}; const long long total = (long long)count * {fd_tasks};")
-            A("  const int blocks = (int)((total + threads - 1) / threads);")
-            A(f"  k_linearize<{T}, SDims, SModel<{T}>><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, (const {T}*)gain, to_dev<{T}>(shadow));")
-        A("  return (int)cudaGetLastError();")
+        A(f"  return launch_linearize<{M}>(nullptr, st, count, N, {ntask}, eps, centered, A, B, gain, shadow, nullptr, nullptr, stream);")
         A("}")
         if has_sensors:
-            # (A, B) plus the sensor Jacobians from the same rollouts: one kernel for all FD tasks, no control law, no advance
+            # (A, B) plus the sensor Jacobians from the same rollouts: no control law, no advance
             A(f"int spec_linearize_sensors{suf}(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, void* dsdx, void* dsdu, void* stream) {{")
-            A(f"  const int threads = {lin_threads}; const long long total = (long long)count * {fd_tasks};")
-            A("  const int blocks = (int)((total + threads - 1) / threads);")
-            A("  const b2_state* no_shadow = nullptr;")
-            A(f"  k_linearize<{T}, SDims, SModel<{T}>, 0, true><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), count, N, ({T})eps, centered, ({T}*)A, ({T}*)B, nullptr, to_dev<{T}>(no_shadow), nullptr, ({T}*)dsdx, ({T}*)dsdu);")
-            A("  return (int)cudaGetLastError();")
+            A(f"  return launch_linearize<{M}, true>(nullptr, st, count, N, {ntask}, eps, centered, A, B, nullptr, nullptr, dsdx, dsdu, stream);")
             A("}")
         A(f"int spec_jacobian{suf}(const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {{")
-        A("  const int threads = 128, blocks = (N + threads - 1) / threads;")
-        A(f"  k_jacobian<{T}, SDims, SModel<{T}>><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<{T}>(st), N, kind, objid, ({T}*)jacp, ({T}*)jacr);")
-        A("  return (int)cudaGetLastError();")
+        A(f"  return launch_jacobian<{M}>(nullptr, st, N, kind, objid, jacp, jacr, stream);")
         A("}")
     sens_init = ", {spec_linearize_sensors, spec_linearize_sensors32}" if has_sensors else ""
     A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{spec_step, spec_step32}}, '

@@ -237,7 +237,7 @@ def test_warp_engine_fd_matches_lane_engine_fd(monkeypatch):
     ctrl[3, 0] = -1.0
     out = {}
     for warp in ("1", "0"):
-        monkeypatch.setenv("B2_WARP_FD", warp)
+        monkeypatch.setenv("B2_DISABLE_WARP", "0" if warp == "1" else "1")  # the batch picks its engine when it is created
         data = _batch(model, n)
         _upload(data, qpos, qvel, ctrl)
         A, B = data.backend.linearize(1e-6, True)

@@ -16,7 +16,7 @@
  *    default stream) unless stated otherwise.  Device memory is allocated in b2_model_create /
  *    b2_batch_create (model images, warp-engine scratch) and on the FIRST call of the entry points
  *    that need extra buffers (b2_control_tick / b2_step_lazy: shadow state; b2_step_host: staging;
- *    b2_lqr_set_gain); b2_step, b2_forward, b2_linearize, b2_linearize_sensors and b2_jacobian never allocate.
+ *    b2_lqr_set_gain); b2_step, b2_rollout, b2_forward, b2_linearize, b2_linearize_sensors and b2_jacobian never allocate.
  *  - No process-wide model state: a model's constants live in per-model device images handed to
  *    every launch, so batches of different models can be driven from different threads and streams,
  *    and a captured CUDA graph replays with the model it was captured with.  One b2_batch must not be
@@ -101,6 +101,23 @@ void b2_batch_destroy(b2_batch* batch);
 /* Replaces mj.mj_step (reference mujoco_template/model.py:56-57, driven by env.py:190):
  * advances every env `nsteps` steps with ctrl held constant.  `derived` may be NULL. */
 int b2_step(b2_batch* batch, const b2_state* state, int nsteps, const b2_derived* derived, void* stream);
+
+/* Open-loop rollout of every env (upstream mujoco.rollout's role; sampling planners, shooting, the forward pass of iLQR):
+ * for t = 0 .. nsteps-1, state.ctrl <- ctrl_seq[t]; one mj_step; record.  Exactly the loop
+ *     state.ctrl <- ctrl_seq[t]; b2_step(batch, state, 1, t == nsteps-1 ? derived : NULL)
+ * with the state recorded after each call.  On the lane engine it is one launch that keeps every env in registers.
+ * ctrl_seq    (nsteps, nu, nenv), element (t, a, e) at base[(t*nu + a)*nenv + e]; NULL = hold state.ctrl (b2_step's case)
+ * qpos_traj   (nsteps, nq, nenv): the state after step t (mj_step's qpos), may be NULL
+ * qvel_traj   (nsteps, nv, nenv): likewise, may be NULL
+ * sensor_traj (nsteps, nsensordata, nenv): the sensordata step t leaves (the forward pass of the pre-step state,
+ *             as mj_step leaves it); may be NULL; ignored when the model has no sensors
+ * derived     as in b2_step: the derived arrays of the LAST step; may be NULL.
+ * After the call state.qpos / qvel / qacc_warmstart hold the final state, state.ctrl holds ctrl_seq[nsteps-1] and
+ * flags are OR-ed as the loop ORs them.  Controls outside ctrlrange are clamped inside the physics; ctrl_seq is not
+ * modified.  A diverged env is flagged and frozen from the step that detects it: its remaining qpos / qvel rows repeat
+ * the state it is frozen in, its remaining sensor rows are NaN (no forward pass ran).  nsteps < 1: B2_ERR_ARG. */
+int b2_rollout(b2_batch* batch, const b2_state* state, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj,
+               void* sensor_traj, const b2_derived* derived, void* stream);
 
 /* Replaces mj.mj_forward (reference model.py:53-54, env.py:157): no integration. */
 int b2_forward(b2_batch* batch, const b2_state* state, const b2_derived* derived, void* stream);

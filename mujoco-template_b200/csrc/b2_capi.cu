@@ -312,6 +312,40 @@ static int do_step(b2_batch* b, const b2_state* st, int count, int nsteps, const
   g_launches++;
   return rc ? cuda_fail((cudaError_t)rc, "step launch") : B2_OK;
 }
+// b2_rollout.  Lane engine (specialised or generic kernels): one k_rollout launch.  Warp engine: the contract's loop itself,
+// one warp step per control row -- a humanoid step of a full batch takes milliseconds, so a launch per step costs nothing,
+// and every step re-orders the warp engine's cost-ordered queue as b2_step does.
+static int do_rollout(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj,
+                      const b2_derived* derived, void* stream) {
+  const b2m_view& v = b->model->v;
+  int rc;
+  if (const b2::SpecKernels* k = active_spec(b)) {
+    cudaError_t e = cudaSetDevice(b->device);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+    rc = k->rollout[prec_index(b)](st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);
+  } else {
+    const void* lane = nullptr;
+    if ((rc = lane_image(b, &lane)) || (rc = prepare_warp(b))) return rc;
+    if (b->warp_mode == 1) {  // the warp engine runs no model with sensors: sensor_traj is null here
+      const size_t N = (size_t)b->nenv, es = b->esz, ctrl_bytes = v.nu * N * es, qpos_bytes = v.nq * N * es, qvel_bytes = v.nv * N * es;
+      cudaStream_t s = (cudaStream_t)stream;
+      for (int t = 0; t < nsteps; t++) {
+        cudaError_t e = cudaSuccess;
+        if (ctrl_seq && ctrl_bytes) e = cudaMemcpyAsync(st->ctrl, (const char*)ctrl_seq + t * ctrl_bytes, ctrl_bytes, cudaMemcpyDefault, s);
+        if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: control row copy");
+        if ((rc = do_step(b, st, b->nenv, 1, t == nsteps - 1 ? derived : nullptr, stream))) return rc;
+        if (qpos_traj) e = cudaMemcpyAsync((char*)qpos_traj + t * qpos_bytes, st->qpos, qpos_bytes, cudaMemcpyDefault, s);
+        if (e == cudaSuccess && qvel_traj) e = cudaMemcpyAsync((char*)qvel_traj + t * qvel_bytes, st->qvel, qvel_bytes, cudaMemcpyDefault, s);
+        if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: trajectory row copy");
+      }
+      return B2_OK;
+    }
+    rc = b->precision == B2_F64 ? b2::b2k_rollout_f64(lane, b->model->cls, st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream)
+                                : b2::b2k_rollout_f32(lane, b->model->cls, st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);
+  }
+  g_launches++;
+  return rc ? cuda_fail((cudaError_t)rc, "rollout launch") : B2_OK;
+}
 // C / D (b2_linearize_sensors): the sensor Jacobians from the same rollouts; either one non-null selects the sensor variant
 // of the FD kernel, which has no control law and no env advance
 static int do_linearize(b2_batch* b, const b2_state* st, int count, double eps, int centered, void* A, void* B, void* stream,
@@ -357,6 +391,14 @@ int b2_step(b2_batch* b, const b2_state* st, int nsteps, const b2_derived* deriv
   B2_CHECK_STATE("b2_step");
   if (nsteps < 1) return fail(B2_ERR_ARG, "b2_step: nsteps must be >= 1");
   return do_step(b, st, b->nenv, nsteps, derived, stream);
+}
+
+int b2_rollout(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj,
+               const b2_derived* derived, void* stream) {
+  B2_CHECK_STATE("b2_rollout");
+  if (nsteps < 1) return fail(B2_ERR_ARG, "b2_rollout: nsteps must be >= 1");
+  const b2m_view& v = b->model->v;
+  return do_rollout(b, st, nsteps, v.nu ? ctrl_seq : nullptr, qpos_traj, qvel_traj, v.nsensordata ? sensor_traj : nullptr, derived, stream);
 }
 
 int b2_forward(b2_batch* b, const b2_state* st, const b2_derived* derived, void* stream) {

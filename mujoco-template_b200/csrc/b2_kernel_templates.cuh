@@ -628,4 +628,70 @@ __global__ void __launch_bounds__(128) k_differentiate_pos(T* out, T dt, const T
   for (int k = 0; k < M::nv(); k++) out[(size_t)k * N + e] = env.qvel[k];
 }
 
+// Open-loop rollout (b2_rollout): for s = 0 .. nsteps-1, ctrl <- ctrl_seq[s] (when given), one mj_step, record.  The same
+// result as a loop of k_step launches with nsteps = 1, with the state in registers across all steps: ctrl_seq
+// (nsteps, nu, N), qpos_traj (nsteps, nq, N), qvel_traj (nsteps, nv, N), sensor_traj (nsteps, nsensordata, N); any of them
+// may be null.  A row of sensor_traj is the reading of step s's forward pass (before integration, as mj_step leaves it).
+// A diverged env is frozen from the step that detects it, as in k_step; its remaining state rows repeat the state it is
+// frozen in (the one the loop would leave in the state arrays) and its remaining sensor rows are NaN (no forward pass ran).
+// Kept apart from k_step (its own arguments, per-step I/O and frozen-env handling) so k_step's instantiations stay as they are.
+template <typename T, class D, class M>
+__global__ void __launch_bounds__(128, 1) k_rollout(StateDev<T> st, DerivedDev<T> out, int want_derived, int N, int nsteps,
+                                                    const T* __restrict__ ctrl_seq, T* qpos_traj, T* qvel_traj, T* sensor_traj,
+                                                    const void* image = nullptr) {
+  model_load<M>(image, 0);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  RowStore<T, D> rows;
+  LaneEnv<T, D, M> env(rows);
+  constexpr bool kLate = LaneEnv<T, D, M>::kLateMass;
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu(), nsd = M::nsensor() > 0 ? M::nsensordata() : 0;
+  load_state(env, st, N, e);
+  int s = 0;
+  B2_NOUNROLL
+  for (; s < nsteps; s++) {
+    if (ctrl_seq) { B2_UNROLL for (int k = 0; k < nu; k++) env.ctrl[k] = ctrl_seq[((size_t)s * nu + k) * N + e]; }
+    env.check_state();
+    if (env.flags & 3) break;
+    env.template forward_position<kLate>();
+    env.forward_velocity();
+    env.template forward_acc<kLate>();
+    B2_UNROLL
+    for (int k = 0; k < nv; k++) if (!(fabs(env.qacc[k]) <= T(1e10))) env.flags |= 4;
+    if (sensor_traj && nsd > 0) {
+      T sd[D::NSD];
+      env.sensors(sd);
+      B2_UNROLL
+      for (int k = 0; k < nsd; k++) sensor_traj[((size_t)s * nsd + k) * N + e] = sd[k];
+    }
+    if (want_derived && s == nsteps - 1) store_derived(env, out, N, e);
+    if (M::integrator() == 1) env.rk4(); else env.euler();
+    if (qpos_traj) { B2_UNROLL for (int k = 0; k < nq; k++) qpos_traj[((size_t)s * nq + k) * N + e] = env.qpos[k]; }
+    if (qvel_traj) { B2_UNROLL for (int k = 0; k < nv; k++) qvel_traj[((size_t)s * nv + k) * N + e] = env.qvel[k]; }
+  }
+  // frozen at step s (s == nsteps when the env never diverged)
+  B2_NOUNROLL
+  for (int r = s; r < nsteps; r++) {
+    if (qpos_traj) { B2_UNROLL for (int k = 0; k < nq; k++) qpos_traj[((size_t)r * nq + k) * N + e] = env.qpos[k]; }
+    if (qvel_traj) { B2_UNROLL for (int k = 0; k < nv; k++) qvel_traj[((size_t)r * nv + k) * N + e] = env.qvel[k]; }
+    if (sensor_traj && nsd > 0) { B2_UNROLL for (int k = 0; k < nsd; k++) sensor_traj[((size_t)r * nsd + k) * N + e] = T(__int_as_float(0x7fc00000)); }
+  }
+  B2_UNROLL
+  for (int k = 0; k < nq; k++) st.qpos[(size_t)k * N + e] = env.qpos[k];
+  B2_UNROLL
+  for (int k = 0; k < nv; k++) st.qvel[(size_t)k * N + e] = env.qvel[k];
+  if (st.warm) { B2_UNROLL for (int k = 0; k < nv; k++) st.warm[(size_t)k * N + e] = env.warm[k]; }
+  // the loop leaves the last control row in state.ctrl, frozen envs included
+  if (ctrl_seq) { B2_UNROLL for (int k = 0; k < nu; k++) st.ctrl[(size_t)k * N + e] = ctrl_seq[((size_t)(nsteps - 1) * nu + k) * N + e]; }
+  if (st.flags && env.flags) st.flags[e] |= env.flags;
+}
+template <typename T, class D, class M>
+auto launch_rollout(const void* image, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj,
+                    void* qvel_traj, void* sensor_traj, void* stream) {
+  const int threads = 128, blocks = (N + threads - 1) / threads;
+  k_rollout<T, D, M><<<blocks, threads, 0, (cudaStream_t)stream>>>(to_dev<T>(st), to_dev<T>(out), out != nullptr, N, nsteps, (const T*)ctrl_seq,
+                                                                   (T*)qpos_traj, (T*)qvel_traj, (T*)sensor_traj, image);
+  return (int)cudaGetLastError();
+}
+
 }  // namespace b2

@@ -33,7 +33,9 @@ namespace b2 {
                                int watch_row, double watch_min, const void* reset_qpos, const void* reset_qvel, void* stream);             \
   int b2k_record_rows##SUF(const void* cols, int ncol, const int* env_index, int nsel, int N, double time, void* out, void* stream); \
   int b2k_integrate_pos##SUF(const void* image, int cls, void* qpos, const void* qvel, double dt, int N, void* stream);                       \
-  int b2k_differentiate_pos##SUF(const void* image, int cls, void* out, double dt, const void* q1, const void* q2, int N, void* stream);
+  int b2k_differentiate_pos##SUF(const void* image, int cls, void* out, double dt, const void* q1, const void* q2, int N, void* stream); \
+  int b2k_rollout##SUF(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, \
+                       void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream);
 B2_DECL(_f64)
 B2_DECL(_f32)
 #undef B2_DECL

@@ -315,5 +315,11 @@ int B2_FN(b2k_differentiate_pos)(const void* image, int cls, void* out, double d
                        (real*)out, (real)dt, (const real*)q1, (const real*)q2, N, image)));
   return (int)cudaGetLastError();
 }
+int B2_FN(b2k_rollout)(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq,
+                       void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_rollout<real, DD, RuntimeModel<DD>>(image, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream)));
+  return rc;
+}
 
 }  // namespace b2

@@ -25,6 +25,9 @@ struct SpecKernels {
   // sensors; null otherwise (the call is then b2_linearize)
   int (*linearize_sensors[2])(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, void* dsdx,
                               void* dsdu, void* stream);
+  // b2_rollout: per-step controls and the recorded trajectory of every env in one launch (k_rollout)
+  int (*rollout[2])(const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj,
+                    void* qvel_traj, void* sensor_traj, void* stream);
 };
 
 void register_spec(const SpecKernels* k);

@@ -23,7 +23,7 @@ _lib: C.CDLL | None = None
 # every symbol include/b2mj.h declares (tests check the shared object exports all of them)
 EXPORTED_SYMBOLS = (
     "b2_model_create", "b2_model_destroy", "b2_model_set_actuator_disabled", "b2_batch_create",
-    "b2_batch_destroy", "b2_step", "b2_forward", "b2_linearize", "b2_linearize_sensors", "b2_jacobian", "b2_integrate_pos",
+    "b2_batch_destroy", "b2_step", "b2_rollout", "b2_forward", "b2_linearize", "b2_linearize_sensors", "b2_jacobian", "b2_integrate_pos",
     "b2_differentiate_pos", "b2_inverse", "b2_lqr_set_gain", "b2_lqr_control", "b2_control_tick", "b2_refresh_derived", "b2_step_lazy", "b2_step_host", "b2_step_host_wait", "b2_stream_synchronize", "b2_launch_count",
     "b2_batch_size_class", "b2_last_error", "b2_version", "b2_fp_peak", "b2_batch_kernel_variant",
     "b2_recorder_create", "b2_recorder_record", "b2_recorder_destroy", "b2_dlqr", "b2_random_controls", "b2_warp_queue_histogram", "b2_lqr_control_env",
@@ -76,6 +76,7 @@ def lib() -> C.CDLL:
     L.b2_batch_kernel_variant.argtypes = [vp]
     L.b2_batch_kernel_variant.restype = C.c_char_p
     L.b2_step.argtypes = [vp, C.POINTER(State), i, C.POINTER(Derived), vp]
+    L.b2_rollout.argtypes = [vp, C.POINTER(State), i, vp, vp, vp, vp, C.POINTER(Derived), vp]
     L.b2_forward.argtypes = [vp, C.POINTER(State), C.POINTER(Derived), vp]
     L.b2_linearize.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp]
     L.b2_linearize_sensors.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp, vp, vp]
@@ -164,6 +165,13 @@ class NativeBatch:
 
     def step(self, state: State, nsteps: int, derived: Derived | None, stream: int = 0) -> None:
         check(self._L.b2_step(self.handle, C.byref(state), int(nsteps), C.byref(derived) if derived is not None else None, stream))
+
+    def rollout(self, state: State, nsteps: int, ctrl_seq: int | None, qpos_traj: int | None, qvel_traj: int | None,
+                sensor_traj: int | None, derived: Derived | None, stream: int = 0) -> None:
+        """``b2_rollout``: ``nsteps`` steps with control row t of ``ctrl_seq`` (nsteps, nu, nenv) applied at step t (None: held
+        controls), recording the state (and sensordata) after every step into the (nsteps, dim, nenv) trajectory arrays."""
+        check(self._L.b2_rollout(self.handle, C.byref(state), int(nsteps), ctrl_seq, qpos_traj, qvel_traj, sensor_traj,
+                                 C.byref(derived) if derived is not None else None, stream))
 
     def forward(self, state: State, derived: Derived | None, stream: int = 0) -> None:
         check(self._L.b2_forward(self.handle, C.byref(state), C.byref(derived) if derived is not None else None, stream))

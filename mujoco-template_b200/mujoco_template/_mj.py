@@ -297,6 +297,26 @@ class NativeBackend:
         self.derived_stale = False
         self._launch("step", self.batch.step, self.state_struct(), nsteps, self.derived_struct() if derived else None)
 
+    def rollout(self, ctrl_seq, nsteps: int, record: bool, out=None, derived: bool = True):
+        """Open-loop rollout (``b2_rollout``): ``nsteps`` steps, control row t of ``ctrl_seq`` applied at step t.
+        ``ctrl_seq``: a tensor laid out as (nsteps, nu, nenv) -- row-contiguous blocks, env fastest -- or None (the
+        controls held).  With ``record`` returns (qpos_traj, qvel_traj, sensor_traj), of shapes (nsteps, nq, nenv),
+        (nsteps, nv, nenv) and (nsteps, nsensordata, nenv) (None without sensors): the state, and the sensordata mj_step
+        leaves, after every step.  Fresh buffers unless ``out`` gives them; an entry of ``out`` may be None (not
+        recorded).  The derived arrays are those of the last step (``derived=False``: not written)."""
+        torch, m = self.torch, self.model
+        T = int(nsteps)
+        if out is None and record:
+            mk = ((lambda dim: torch.zeros((T, dim, self.nenv), dtype=self.dtype).pin_memory()) if self.host_mapped else
+                  (lambda dim: torch.empty((T, dim, self.nenv), device=f"cuda:{self.device}", dtype=self.dtype)))
+            out = (mk(m.nq), mk(m.nv), mk(m.nsensordata) if m.nsensordata else None)
+        bufs = tuple(out) if out is not None else (None, None, None)
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
+        self.derived_stale = False
+        self._launch("rollout", self.batch.rollout, self.state_struct(), T, ptr(ctrl_seq) if m.nu else None, *map(ptr, bufs),
+                     self.derived_struct() if derived else None)
+        return bufs if out is not None else None
+
     def forward(self) -> None:
         self.derived_stale = False
         self._launch("forward", self.batch.forward, self.state_struct(), self.derived_struct())

@@ -2,7 +2,7 @@
 
 For a compiled model this writes ``csrc/generated/spec_<name>.cu``: a provider class whose
 accessors return compile-time constants (function-local ``constexpr`` tables), exact-size
-capacity constants, launchers for the step / linearize / jacobian kernels instantiated with that
+capacity constants, launchers for the step / linearize / jacobian / rollout kernels instantiated with that
 provider, and a registrar keyed by the FNV-1a hash of the model blob.  ``libb2mj.so`` picks the
 specialised kernels automatically when ``b2_model_create`` sees a blob with a registered hash;
 any other model runs on the generic (constant-memory) kernels.
@@ -169,9 +169,14 @@ def emit_spec(compiled: dict, name: str) -> str:
         A(f"int spec_jacobian{suf}(const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {{")
         A(f"  return launch_jacobian<{M}>(nullptr, st, N, kind, objid, jacp, jacr, stream);")
         A("}")
-    sens_init = ", {spec_linearize_sensors, spec_linearize_sensors32}" if has_sensors else ""
+    # the rollout kernels come after all the others: cicc's inlining, and so the other kernels' code, depends on kernel order
+    for T, suf in (("double", ""), ("float", "32")):
+        A(f"int spec_rollout{suf}(const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {{")
+        A(f"  return launch_rollout<{T}, SDims, SModel<{T}>>(nullptr, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);")
+        A("}")
+    sens_init = "{spec_linearize_sensors, spec_linearize_sensors32}" if has_sensors else "{nullptr, nullptr}"
     A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{spec_step, spec_step32}}, '
-      f'{{spec_linearize, spec_linearize32}}, {{spec_jacobian, spec_jacobian32}}{sens_init}}};')
+      f'{{spec_linearize, spec_linearize32}}, {{spec_jacobian, spec_jacobian32}}, {sens_init}, {{spec_rollout, spec_rollout32}}}};')
     A("struct Registrar { Registrar() { register_spec(&kSpec); } } registrar;")
     A("}  // namespace")
     A("}  // namespace b2")

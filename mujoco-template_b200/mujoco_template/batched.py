@@ -324,13 +324,53 @@ class BatchedEnv:
                 info[key] = value
         return StepResult(obs=obs, reward=reward, done=done, info=info)
 
-    def rollout(self, nsteps: int) -> None:
-        """``nsteps`` steps with the current controls held, fused in one kernel launch."""
-        if nsteps < 1:
+    def rollout(self, nsteps: int | None = None, *, controls=None, record: bool = False):
+        """``nsteps`` steps of every env in one kernel launch (the warp engine of large models: one launch per step).
+
+        Open loop: the controller is not called.  Without ``controls`` the current controls are held.  ``controls`` is a
+        ``(nenv, T, nu)`` tensor (any strides; on the batch's device, in its dtype): row t is applied at step t, and
+        ``data.ctrl`` holds row T-1 afterwards.  ``nsteps`` may then be omitted; if given it must equal T.  It is handed to
+        the kernel as a ``(T, nu, nenv)`` layout, which costs no copy when ``controls`` is already a permuted view of such a
+        buffer.  Controls outside ``ctrlrange`` are clamped inside the physics, as in ``step``.
+
+        ``record=True`` returns ``{"qpos": (nenv, T, nq), "qvel": (nenv, T, nv)}`` -- the state after every step -- plus
+        ``"sensordata": (nenv, T, nsensordata)`` when the model has sensors (the reading each step leaves, as ``mj_step``
+        leaves it), as permuted views of fresh ``(T, dim, nenv)`` buffers.  An env that diverges is flagged and frozen: its
+        remaining rows repeat its frozen state, and its remaining sensor rows are NaN.  Otherwise returns None.
+        ``data.time`` advances by T timesteps and the derived arrays are those of the last step."""
+        backend, m = self.data.backend, self.model
+        seq = None
+        if controls is not None:
+            import torch
+
+            if m.nu == 0:
+                raise ConfigError("rollout(controls=...): the model has no actuators (nu=0)")
+            if not isinstance(controls, torch.Tensor) or controls.dim() != 3 or controls.shape[0] != self.nenv or controls.shape[2] != m.nu:
+                raise ConfigError(f"rollout(controls=...): expected a (nenv={self.nenv}, T, nu={m.nu}) tensor, got "
+                                  f"{tuple(controls.shape) if isinstance(controls, torch.Tensor) else type(controls).__name__}")
+            ref = self.data.qpos
+            if controls.device != ref.device or controls.dtype != ref.dtype:
+                raise ConfigError(f"rollout(controls=...): expected {ref.dtype} on {ref.device}, got {controls.dtype} on {controls.device}")
+            if nsteps is not None and int(nsteps) != controls.shape[1]:
+                raise ConfigError(f"rollout: nsteps={nsteps} disagrees with the {controls.shape[1]} rows of controls")
+            nsteps = controls.shape[1]
+            seq = controls.permute(1, 2, 0).contiguous()  # (T, nu, nenv); no copy for a permuted (T, nu, nenv) buffer
+        if nsteps is None or int(nsteps) < 1:
             raise ConfigError("nsteps must be >= 1")
-        self.data.backend.step(int(nsteps))
-        self._advance_time(int(nsteps))
-        self._substep += int(nsteps)
+        nsteps = int(nsteps)
+        out = None
+        if seq is None and not record:
+            backend.step(nsteps)
+        else:
+            out = backend.rollout(seq, nsteps, record)
+        self._advance_time(nsteps)
+        self._substep += nsteps
+        if not record:
+            return None
+        traj = {"qpos": out[0].permute(2, 0, 1), "qvel": out[1].permute(2, 0, 1)}
+        if out[2] is not None:
+            traj["sensordata"] = out[2].permute(2, 0, 1)
+        return traj
 
     def passive(self, *, duration: float | None = None, max_steps: int | None = None, hooks=None,
                 return_obs: bool = True) -> Iterator[StepResult]:

@@ -1,8 +1,9 @@
 // C-ABI of the B200-native batched physics path (see include/b2mj.h for the contract and the
 // reference call sites each entry point replaces).  Host-only logic: model bookkeeping,
-// constant-bank residency, launches, and the host-buffer (e2e) variant.
+// the models' device images, launches, and the host-buffer (e2e) variant.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <cstdio>
@@ -16,7 +17,6 @@
 #include "../../include/b2mj.h"
 #include "b2_kernels.h"
 #include "b2_model_dev.cuh"
-#include "b2_spec_registry.h"
 
 namespace {
 thread_local std::string g_err;
@@ -27,6 +27,12 @@ int fail(int code, const std::string& msg) { g_err = msg; return code; }
 int cuda_fail(cudaError_t e, const char* what) {
   return fail(B2_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
+// counts one launch; rc is the launcher's cudaError_t
+int launched(int rc, const char* what) {
+  g_launches++;
+  return rc ? cuda_fail((cudaError_t)rc, what) : B2_OK;
+}
+const b2::Kernels* kernels(int precision) { return precision == B2_F64 ? &b2::kernels_f64 : &b2::kernels_f32; }
 }  // namespace
 
 struct b2_model {
@@ -35,7 +41,8 @@ struct b2_model {
   std::vector<int> disabled;
   int cls;
   unsigned long long serial;
-  const b2::SpecKernels* spec;  // model-specialised FP64 kernels, or nullptr (generic path)
+  const b2::SpecKernels* spec;  // model-specialised kernels, or nullptr (generic kernels)
+  const b2::LaneKernels* lane[2];  // [0] FP64, [1] FP32: the lane-engine launchers of spec, or the generic ones
   // The model's images in device memory, per device and precision: [.][.][0] the lane engine's (DevModel of the model's
   // size class), [.][.][1] the warp engine's (constants + factorisation work lists).  Kernels get them by pointer, so
   // nothing about a model is process-wide device state: batches of different models are independent of each other on
@@ -61,7 +68,11 @@ const SpecKernels* find_spec(uint64_t hash, size_t size) {
 }
 }  // namespace b2
 
-static inline const b2::SpecKernels* active_spec(const b2_batch* b);
+static void set_spec(b2_model* m, const b2::SpecKernels* spec) {
+  m->spec = spec;
+  m->lane[0] = spec ? &spec->lane[0] : &b2::kernels_f64.generic;
+  m->lane[1] = spec ? &spec->lane[1] : &b2::kernels_f32.generic;
+}
 
 struct HostStepKey {
   void *qpos, *qvel, *ctrl, *warm, *A, *B;
@@ -73,11 +84,14 @@ struct HostStepKey {
 struct b2_batch {
   const b2_model* model;
   int nenv, device, precision;
+  int pi;  // 0 FP64, 1 FP32: index of the model's per-precision kernels and images
+  const b2::Kernels* k;  // the generic kernels of this precision
   size_t esz;
   // device staging for b2_step_host
   void *d_qpos = nullptr, *d_qvel = nullptr, *d_ctrl = nullptr, *d_warm = nullptr, *d_A = nullptr, *d_B = nullptr;
-  // warp engine (large models): -1 not yet decided, 0 lane engine, 1 warp engine
-  int warp_mode = -1, warp_wpb = 0, warp_blocks = 0, warp_slots = 0;
+  // warp engine (large models), decided in b2_batch_create
+  bool warp = false;
+  int warp_wpb = 0, warp_blocks = 0, warp_slots = 0;
   void* d_jscratch = nullptr;
   void* d_warp_counter = nullptr;  // inside d_jscratch
   void* d_warp_sort = nullptr;     // inside d_jscratch: cost-ordered queue (hist / cursor, cost[N], perm[N])
@@ -92,8 +106,6 @@ struct b2_batch {
   HostStepKey host_key;
   int host_graph_launches = 0;
 };
-
-static int b2_batch_setup(b2_batch* b, const void** image);
 
 // The warp engine covers the feature set of large articulated models (humanoid); everything else
 // in the large size class runs on the lane engine.
@@ -112,6 +124,62 @@ static bool warp_engine_supports(const b2m_view& v) {
   }
   return true;
 }
+
+// decide whether the batch runs on the large-model warp engine; plan its launch and scratch
+static int prepare_warp(b2_batch* b) {
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+  if (b->model->cls != 2 || !warp_engine_supports(b->model->v)) return B2_OK;
+  int wpb = 0, blocks = 0;
+  const int slots = b->k->warp_plan(&b->model->v, b->nenv, &wpb, &blocks);
+  if (slots <= 0) return B2_OK;  // not enough shared memory: stay on the lane engine
+  const size_t bytes = b->k->warp_scratch_bytes(&b->model->v, slots);
+  // + the work-queue counter of the persistent kernel + the buffers of the cost-ordered queue
+  const size_t sort_bytes = b->k->warp_sort_bytes(b->nenv);
+  e = cudaMalloc(&b->d_jscratch, bytes + 256 + sort_bytes);
+  if (e != cudaSuccess) return cuda_fail(e, "warp-engine scratch cudaMalloc");
+  b->d_warp_counter = (char*)b->d_jscratch + bytes;
+  b->d_warp_sort = (char*)b->d_warp_counter + 256;
+  if ((e = cudaMemset(b->d_warp_sort, 0, sort_bytes)) != cudaSuccess) return cuda_fail(e, "warp-engine queue cudaMemset");
+  b->warp = true; b->warp_wpb = wpb; b->warp_blocks = blocks; b->warp_slots = slots;
+  return B2_OK;
+}
+// The model's image for this batch's device and precision (kind 0: lane engine, 1: warp engine): uploaded on first use
+// (b2_batch_create does that for the kinds the batch will launch) and again after a disable-mask change.
+static int image_of(b2_batch* b, int kind, const void** out) {
+  const b2_model* m = b->model;
+  const int pi = b->pi, dev = b->device;
+  std::lock_guard<std::mutex> lock(m->image_mu);
+  if (!m->image[dev][pi][kind] || m->image_serial[dev][pi][kind] != m->serial) {
+    const size_t bytes = kind == 1 ? b->k->warp_image_bytes() : b->k->image_bytes(m->cls);
+    std::vector<unsigned char> host(bytes);
+    if (kind == 1) b->k->warp_image_fill(&m->v, m->disabled.data(), host.data());
+    else b->k->image_fill(m->cls, &m->v, m->disabled.data(), host.data());
+    void* d = nullptr;
+    cudaError_t e = cudaMalloc(&d, bytes);
+    if (e != cudaSuccess) return cuda_fail(e, "model image cudaMalloc");
+    if ((e = cudaMemcpy(d, host.data(), bytes, cudaMemcpyHostToDevice)) != cudaSuccess) { cudaFree(d); return cuda_fail(e, "model image upload"); }
+    if (m->image[dev][pi][kind]) m->retired_images.emplace_back(dev, m->image[dev][pi][kind]);  // kernels in flight may still read it
+    m->image[dev][pi][kind] = d;
+    m->image_serial[dev][pi][kind] = m->serial;
+  }
+  *out = m->image[dev][pi][kind];
+  return B2_OK;
+}
+// Every launch starts here: selects the batch's device and hands out its model's current lane-engine image and, when the
+// batch runs on the warp engine and `warp` is given, its warp-engine image.
+static int batch_images(b2_batch* b, const void** lane, const void** warp = nullptr) {
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+  int rc = image_of(b, 0, lane);
+  if (!rc && warp && b->warp) rc = image_of(b, 1, warp);
+  return rc;
+}
+// the warp engine takes the launches it supports, unless the model has specialised kernels
+static bool on_warp_engine(const b2_batch* b) { return b->warp && !b->model->spec; }
+
+#define B2_CHECK_STATE(fn)                                                                         \
+  if (!b || !st || !st->qpos || !st->qvel || (b->model->v.nu && !st->ctrl)) return fail(B2_ERR_ARG, fn ": null batch/state pointer")
 
 extern "C" {
 
@@ -133,7 +201,7 @@ int b2_model_create(const void* blob, size_t nbytes, b2_model** out) {
   else { delete m; return fail(B2_ERR_CAPACITY, "b2_model_create: model exceeds the largest compiled size class"); }
   m->disabled.assign(v.actuator_disabled, v.actuator_disabled + v.nu);
   m->serial = g_serial.fetch_add(1);
-  m->spec = b2::find_spec(b2::fnv1a(blob, nbytes), nbytes);
+  set_spec(m, b2::find_spec(b2::fnv1a(blob, nbytes), nbytes));
   *out = m;
   return B2_OK;
 }
@@ -152,10 +220,12 @@ void b2_model_destroy(b2_model* m) {
 
 int b2_model_set_actuator_disabled(b2_model* m, const int* disabled, int nu) {
   if (!m || (nu && !disabled) || nu != m->v.nu) return fail(B2_ERR_ARG, "b2_model_set_actuator_disabled: bad arguments");
+  // an unchanged mask keeps the images: launches never upload one then (an upload cannot run inside a graph capture)
+  if (std::equal(disabled, disabled + nu, m->disabled.begin())) return B2_OK;
   m->disabled.assign(disabled, disabled + nu);
   m->serial = g_serial.fetch_add(1);  // the device images are rebuilt on their next use
   for (int i = 0; i < nu; i++)
-    if (disabled[i] != m->v.actuator_disabled[i]) m->spec = nullptr;  // the specialisation bakes the mask in
+    if (disabled[i] != m->v.actuator_disabled[i]) set_spec(m, nullptr);  // the specialisation bakes the mask in
   return B2_OK;
 }
 
@@ -168,12 +238,13 @@ int b2_batch_create(const b2_model* model, int nenv, int device, int precision, 
   if (device < 0 || device >= ndev || device >= 16) return fail(B2_ERR_ARG, "b2_batch_create: device index out of range");
   b2_batch* b = new (std::nothrow) b2_batch();
   if (!b) return fail(B2_ERR_ARG, "out of host memory");
-  b->model = model; b->nenv = nenv; b->device = device; b->precision = precision; b->esz = precision == B2_F64 ? 8 : 4;
+  b->model = model; b->nenv = nenv; b->device = device; b->precision = precision;
+  b->pi = precision == B2_F64 ? 0 : 1; b->k = kernels(precision); b->esz = precision == B2_F64 ? 8 : 4;
   // everything the step path needs on the device is set up here, so that b2_step / b2_linearize only launch: the model's
   // images (shared by all batches of the model on this device) and, for large models, the warp engine's plan and scratch
-  const void* image = nullptr;
-  int rc = b2_batch_setup(b, &image);
-  if (rc) { b2_batch_destroy(b); return rc; }
+  const void *lane = nullptr, *warp = nullptr;
+  int rc = prepare_warp(b);
+  if (rc || (rc = batch_images(b, &lane, &warp))) { b2_batch_destroy(b); return rc; }
   *out = b;
   return B2_OK;
 }
@@ -188,203 +259,83 @@ void b2_batch_destroy(b2_batch* b) {
 int b2_batch_size_class(const b2_batch* b) { return b ? b->model->cls : -1; }
 const char* b2_batch_kernel_variant(const b2_batch* b) {
   if (!b) return "";
-  const b2::SpecKernels* k = b->model->spec;
-  if (k) return k->name;
-  if (b->warp_mode == 1 || (b->warp_mode < 0 && b->model->cls == 2 && warp_engine_supports(b->model->v))) return "generic-warp";
-  return "generic";
+  if (b->model->spec) return b->model->spec->name;
+  return b->warp ? "generic-warp" : "generic";
 }
 
-}  // extern "C"
-
-static inline const b2::SpecKernels* active_spec(const b2_batch* b) { return b->model->spec; }
-static inline int prec_index(const b2_batch* b) { return b->precision == B2_F64 ? 0 : 1; }
-
-static int lane_image(b2_batch* b, const void** image);
-
-// decide once per batch whether the large-model warp engine is used; plan its launch and scratch
-static int prepare_warp(b2_batch* b) {
-  cudaError_t e0 = cudaSetDevice(b->device);
-  if (e0 != cudaSuccess) return cuda_fail(e0, "cudaSetDevice");
-  if (b->warp_mode >= 0) return B2_OK;
-  b->warp_mode = 0;
-  if (b->model->cls != 2 || !warp_engine_supports(b->model->v)) return B2_OK;
-  const bool f64 = b->precision == B2_F64;
-  int wpb = 0, blocks = 0;
-  const int slots = f64 ? b2::b2k_warp_plan_f64(&b->model->v, b->nenv, &wpb, &blocks)
-                        : b2::b2k_warp_plan_f32(&b->model->v, b->nenv, &wpb, &blocks);
-  if (slots <= 0) return B2_OK;  // not enough shared memory: stay on the lane engine
-  const size_t bytes = f64 ? b2::b2k_warp_scratch_bytes_f64(&b->model->v, slots) : b2::b2k_warp_scratch_bytes_f32(&b->model->v, slots);
-  // + the work-queue counter of the persistent kernel + the buffers of the cost-ordered queue
-  const size_t sort_bytes = f64 ? b2::b2k_warp_sort_bytes_f64(b->nenv) : b2::b2k_warp_sort_bytes_f32(b->nenv);
-  cudaError_t e = cudaMalloc(&b->d_jscratch, bytes + 256 + sort_bytes);
-  if (e != cudaSuccess) return cuda_fail(e, "warp-engine scratch cudaMalloc");
-  b->d_warp_counter = (char*)b->d_jscratch + bytes;
-  b->d_warp_sort = (char*)b->d_warp_counter + 256;
-  if ((e = cudaMemset(b->d_warp_sort, 0, sort_bytes)) != cudaSuccess) return cuda_fail(e, "warp-engine queue cudaMemset");
-  b->warp_mode = 1; b->warp_wpb = wpb; b->warp_blocks = blocks; b->warp_slots = slots;
-  return B2_OK;
-}
-// The model's image for this batch's device and precision (kind 0: lane engine, 1: warp engine): uploaded on first use
-// (b2_batch_create does that for the kinds the batch will launch) and again after a disable-mask change.
-static int image_of(b2_batch* b, int kind, const void** out) {
-  const b2_model* m = b->model;
-  const int pi = b->precision == B2_F64 ? 0 : 1, dev = b->device;
-  std::lock_guard<std::mutex> lock(m->image_mu);
-  if (!m->image[dev][pi][kind] || m->image_serial[dev][pi][kind] != m->serial) {
-    cudaError_t e = cudaSetDevice(dev);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    const size_t bytes = kind == 1 ? (pi == 0 ? b2::b2k_warp_image_bytes_f64() : b2::b2k_warp_image_bytes_f32())
-                                   : (pi == 0 ? b2::b2k_image_bytes_f64(m->cls) : b2::b2k_image_bytes_f32(m->cls));
-    std::vector<unsigned char> host(bytes);
-    if (kind == 1) {
-      if (pi == 0) b2::b2k_warp_image_fill_f64(&m->v, m->disabled.data(), host.data());
-      else b2::b2k_warp_image_fill_f32(&m->v, m->disabled.data(), host.data());
-    } else {
-      if (pi == 0) b2::b2k_image_fill_f64(m->cls, &m->v, m->disabled.data(), host.data());
-      else b2::b2k_image_fill_f32(m->cls, &m->v, m->disabled.data(), host.data());
-    }
-    void* d = nullptr;
-    e = cudaMalloc(&d, bytes);
-    if (e != cudaSuccess) return cuda_fail(e, "model image cudaMalloc");
-    if ((e = cudaMemcpy(d, host.data(), bytes, cudaMemcpyHostToDevice)) != cudaSuccess) { cudaFree(d); return cuda_fail(e, "model image upload"); }
-    if (m->image[dev][pi][kind]) m->retired_images.emplace_back(dev, m->image[dev][pi][kind]);  // kernels in flight may still read it
-    m->image[dev][pi][kind] = d;
-    m->image_serial[dev][pi][kind] = m->serial;
-  }
-  *out = m->image[dev][pi][kind];
-  return B2_OK;
-}
-static int warp_image_of(b2_batch* b, const void** out) { return image_of(b, 1, out); }
-extern "C" { static int do_lqr_control(b2_batch* b, const b2_state* st, int count, void* stream); }
-
-static int launch_generic_step(b2_batch* b, const b2_state* st, const b2_derived* derived, int count, int nsteps, const void* gain,
-                               void* stream, const b2_state* park = nullptr) {
+static int do_lqr_control(b2_batch* b, const b2_state* st, int count, void* stream) {
   const void* lane = nullptr;
-  int rc = lane_image(b, &lane);
+  int rc = batch_images(b, &lane);
   if (rc) return rc;
-  if ((rc = prepare_warp(b))) return rc;
-  const bool f64 = b->precision == B2_F64;
-  if (b->warp_mode == 1 && count == b->nenv && gain) {  // the warp engine has no in-kernel control law: separate launch
-    if ((rc = do_lqr_control(b, st, count, stream))) return rc;
-    gain = nullptr;
-  }
-  if (b->warp_mode == 1 && count == b->nenv) {
-    const void* image = nullptr;
-    if ((rc = warp_image_of(b, &image))) return rc;
-    if (b->warp_wpb > 1 && nsteps > 0) g_launches += 2;  // the queue's histogram and scatter kernels
-    return f64 ? b2::b2k_warp_step_f64(image, &b->model->v, st, derived, b->nenv, nsteps, b->d_jscratch, b->d_warp_counter, b->d_warp_sort, b->warp_wpb, b->warp_blocks, park, stream)
-               : b2::b2k_warp_step_f32(image, &b->model->v, st, derived, b->nenv, nsteps, b->d_jscratch, b->d_warp_counter, b->d_warp_sort, b->warp_wpb, b->warp_blocks, park, stream);
-  }
-  return f64 ? b2::b2k_step_f64(lane, b->model->cls, st, derived, count, b->nenv, nsteps, gain, park, stream)
-             : b2::b2k_step_f32(lane, b->model->cls, st, derived, count, b->nenv, nsteps, gain, park, stream);
+  return launched(b->k->lqr_control(lane, b->model->cls, st, count, b->nenv, b->d_gain, stream), "b2_lqr_control launch");
 }
-
-// selects the batch's device and hands out the lane-engine image of its model
-static int b2_batch_setup(b2_batch* b, const void** image) {
-  int rc = prepare_warp(b);
-  if (rc || (rc = image_of(b, 0, image))) return rc;
-  if (b->warp_mode == 1) rc = image_of(b, 1, image);
-  return rc;
-}
-static int lane_image(b2_batch* b, const void** image) {
-  cudaError_t e = cudaSetDevice(b->device);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-  return image_of(b, 0, image);
-}
-
-#define B2_CHECK_STATE(fn)                                                                         \
-  if (!b || !st || !st->qpos || !st->qvel || (b->model->v.nu && !st->ctrl)) return fail(B2_ERR_ARG, fn ": null batch/state pointer")
-
-extern "C" {
 
 // count envs (a leading chunk of the arrays `st` points at; the env stride is always b->nenv)
 static int do_step(b2_batch* b, const b2_state* st, int count, int nsteps, const b2_derived* derived, void* stream,
                    const void* gain = nullptr, const b2_state* park = nullptr) {
-  int rc;
-  if (const b2::SpecKernels* k = active_spec(b)) {
-    cudaError_t e = cudaSetDevice(b->device);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    rc = k->step[prec_index(b)](st, derived, count, b->nenv, nsteps, gain, park, stream);
+  const void *lane = nullptr, *warp = nullptr;
+  int rc = batch_images(b, &lane, &warp);
+  if (rc) return rc;
+  const b2_model* m = b->model;
+  if (on_warp_engine(b) && count == b->nenv) {
+    // the warp engine has no in-kernel control law: separate launch
+    if (gain && (rc = do_lqr_control(b, st, count, stream))) return rc;
+    if (b->warp_wpb > 1 && nsteps > 0) g_launches += 2;  // the queue's histogram and scatter kernels
+    rc = b->k->warp_step(warp, &m->v, st, derived, b->nenv, nsteps, b->d_jscratch, b->d_warp_counter, b->d_warp_sort, b->warp_wpb,
+                         b->warp_blocks, park, stream);
   } else {
-    rc = launch_generic_step(b, st, derived, count, nsteps, gain, stream, park);
-    if (rc < 0) return rc;
+    rc = m->lane[b->pi]->step(lane, m->cls, st, derived, count, b->nenv, nsteps, gain, park, stream);
   }
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "step launch") : B2_OK;
+  return launched(rc, "step launch");
 }
 // b2_rollout.  Lane engine (specialised or generic kernels): one k_rollout launch.  Warp engine: the contract's loop itself,
 // one warp step per control row -- a humanoid step of a full batch takes milliseconds, so a launch per step costs nothing,
 // and every step re-orders the warp engine's cost-ordered queue as b2_step does.
 static int do_rollout(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj,
                       const b2_derived* derived, void* stream) {
-  const b2m_view& v = b->model->v;
-  int rc;
-  if (const b2::SpecKernels* k = active_spec(b)) {
-    cudaError_t e = cudaSetDevice(b->device);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    rc = k->rollout[prec_index(b)](st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);
-  } else {
-    const void* lane = nullptr;
-    if ((rc = lane_image(b, &lane)) || (rc = prepare_warp(b))) return rc;
-    if (b->warp_mode == 1) {  // the warp engine runs no model with sensors: sensor_traj is null here
-      const size_t N = (size_t)b->nenv, es = b->esz, ctrl_bytes = v.nu * N * es, qpos_bytes = v.nq * N * es, qvel_bytes = v.nv * N * es;
-      cudaStream_t s = (cudaStream_t)stream;
-      for (int t = 0; t < nsteps; t++) {
-        cudaError_t e = cudaSuccess;
-        if (ctrl_seq && ctrl_bytes) e = cudaMemcpyAsync(st->ctrl, (const char*)ctrl_seq + t * ctrl_bytes, ctrl_bytes, cudaMemcpyDefault, s);
-        if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: control row copy");
-        if ((rc = do_step(b, st, b->nenv, 1, t == nsteps - 1 ? derived : nullptr, stream))) return rc;
-        if (qpos_traj) e = cudaMemcpyAsync((char*)qpos_traj + t * qpos_bytes, st->qpos, qpos_bytes, cudaMemcpyDefault, s);
-        if (e == cudaSuccess && qvel_traj) e = cudaMemcpyAsync((char*)qvel_traj + t * qvel_bytes, st->qvel, qvel_bytes, cudaMemcpyDefault, s);
-        if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: trajectory row copy");
-      }
-      return B2_OK;
+  const b2_model* m = b->model;
+  const b2m_view& v = m->v;
+  const void* lane = nullptr;
+  int rc = batch_images(b, &lane);
+  if (rc) return rc;
+  if (on_warp_engine(b)) {  // the warp engine runs no model with sensors: sensor_traj is null here
+    const size_t N = (size_t)b->nenv, es = b->esz, ctrl_bytes = v.nu * N * es, qpos_bytes = v.nq * N * es, qvel_bytes = v.nv * N * es;
+    cudaStream_t s = (cudaStream_t)stream;
+    for (int t = 0; t < nsteps; t++) {
+      cudaError_t e = cudaSuccess;
+      if (ctrl_seq && ctrl_bytes) e = cudaMemcpyAsync(st->ctrl, (const char*)ctrl_seq + t * ctrl_bytes, ctrl_bytes, cudaMemcpyDefault, s);
+      if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: control row copy");
+      if ((rc = do_step(b, st, b->nenv, 1, t == nsteps - 1 ? derived : nullptr, stream))) return rc;
+      if (qpos_traj) e = cudaMemcpyAsync((char*)qpos_traj + t * qpos_bytes, st->qpos, qpos_bytes, cudaMemcpyDefault, s);
+      if (e == cudaSuccess && qvel_traj) e = cudaMemcpyAsync((char*)qvel_traj + t * qvel_bytes, st->qvel, qvel_bytes, cudaMemcpyDefault, s);
+      if (e != cudaSuccess) return cuda_fail(e, "b2_rollout: trajectory row copy");
     }
-    rc = b->precision == B2_F64 ? b2::b2k_rollout_f64(lane, b->model->cls, st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream)
-                                : b2::b2k_rollout_f32(lane, b->model->cls, st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);
+    return B2_OK;
   }
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "rollout launch") : B2_OK;
+  rc = m->lane[b->pi]->rollout(lane, m->cls, st, derived, b->nenv, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);
+  return launched(rc, "rollout launch");
 }
 // C / D (b2_linearize_sensors): the sensor Jacobians from the same rollouts; either one non-null selects the sensor variant
 // of the FD kernel, which has no control law and no env advance
 static int do_linearize(b2_batch* b, const b2_state* st, int count, double eps, int centered, void* A, void* B, void* stream,
                         const void* gain = nullptr, const b2_state* shadow = nullptr, void* C = nullptr, void* D = nullptr) {
   const bool sensors = C || D;
-  int rc;
-  if (const b2::SpecKernels* k = active_spec(b)) {
-    cudaError_t e = cudaSetDevice(b->device);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    const int p = prec_index(b);
-    rc = sensors ? k->linearize_sensors[p](st, count, b->nenv, eps, centered, A, B, C, D, stream)
-                 : k->linearize[p](st, count, b->nenv, eps, centered, A, B, gain, shadow, stream);
-  } else {
-    const void* lane = nullptr;
-    if ((rc = lane_image(b, &lane))) return rc;
-    if ((rc = prepare_warp(b))) return rc;
-    // large models on the warp engine: one warp per (column, env) rollout pair (the warp engine runs no model with sensors)
-    if (b->warp_mode == 1 && count == b->nenv && !gain && !shadow && !sensors) {
-      const void* image = nullptr;
-      if ((rc = warp_image_of(b, &image))) return rc;
-      rc = b->precision == B2_F64
-               ? b2::b2k_warp_linearize_f64(image, &b->model->v, st, b->nenv, eps, centered, A, B, b->d_jscratch, b->d_warp_counter, b->warp_wpb, b->warp_blocks, stream)
-               : b2::b2k_warp_linearize_f32(image, &b->model->v, st, b->nenv, eps, centered, A, B, b->d_jscratch, b->d_warp_counter, b->warp_wpb, b->warp_blocks, stream);
-      g_launches++;
-      return rc ? cuda_fail((cudaError_t)rc, "warp linearize launch") : B2_OK;
-    }
-    // FD tasks per env: see k_linearize (Euler: one thread per group of velocity / control columns + one per position column)
-    const b2m_view& v = b->model->v;
-    const int ntask = b2::fd_task_count(v.integrator, v.nv, v.nu);
-    const bool f64 = b->precision == B2_F64;
-    if (sensors)
-      rc = f64 ? b2::b2k_linearize_sensors_f64(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, C, D, stream)
-               : b2::b2k_linearize_sensors_f32(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, C, D, stream);
-    else
-      rc = f64 ? b2::b2k_linearize_f64(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream)
-               : b2::b2k_linearize_f32(lane, b->model->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream);
+  const void *lane = nullptr, *warp = nullptr;
+  int rc = batch_images(b, &lane, &warp);
+  if (rc) return rc;
+  const b2_model* m = b->model;
+  // large models on the warp engine: one warp per (column, env) rollout pair (the warp engine runs no model with sensors)
+  if (on_warp_engine(b) && count == b->nenv && !gain && !shadow && !sensors) {
+    rc = b->k->warp_linearize(warp, &m->v, st, b->nenv, eps, centered, A, B, b->d_jscratch, b->d_warp_counter, b->warp_wpb, b->warp_blocks,
+                              stream);
+    return launched(rc, "warp linearize launch");
   }
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "linearize launch") : B2_OK;
+  // FD tasks per env: see k_linearize (Euler: one thread per group of velocity / control columns + one per position column)
+  const int ntask = b2::fd_task_count(m->v.integrator, m->v.nv, m->v.nu);
+  const b2::LaneKernels* lk = m->lane[b->pi];
+  rc = sensors ? lk->linearize_sensors(lane, m->cls, st, count, b->nenv, ntask, eps, centered, A, B, C, D, stream)
+               : lk->linearize(lane, m->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream);
+  return launched(rc, "linearize launch");
 }
 
 int b2_step(b2_batch* b, const b2_state* st, int nsteps, const b2_derived* derived, void* stream) {
@@ -420,8 +371,7 @@ int b2_linearize_sensors(b2_batch* b, const b2_state* st, double eps, int center
   const b2m_view& v = b->model->v;
   // without sensors (or without C / D to fill) this is b2_linearize; the warp engine only runs models without sensors
   if (v.nsensordata == 0 || (!C && !D)) return (A || B) ? do_linearize(b, st, b->nenv, eps, centered, A, B, stream) : B2_OK;
-  if (const b2::SpecKernels* k = active_spec(b))
-    if (!k->linearize_sensors[prec_index(b)]) return fail(B2_ERR_ARG, "b2_linearize_sensors: specialised kernel set has no sensor variant");
+  if (!b->model->lane[b->pi]->linearize_sensors) return fail(B2_ERR_ARG, "b2_linearize_sensors: specialised kernel set has no sensor variant");
   return do_linearize(b, st, b->nenv, eps, centered, A, B, stream, nullptr, nullptr, C, D);
 }
 
@@ -431,31 +381,20 @@ int b2_jacobian(b2_batch* b, const b2_state* st, int kind, int objid, void* jacp
   const int limit = kind == B2_JAC_SITE ? v.nsite : v.nbody;
   if (kind < B2_JAC_SITE || kind > B2_JAC_SUBTREECOM || objid < 0 || objid >= limit)
     return fail(B2_ERR_ARG, "b2_jacobian: kind/objid out of range");
-  int rc;
-  if (const b2::SpecKernels* k = active_spec(b)) {
-    cudaError_t e = cudaSetDevice(b->device);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    rc = k->jacobian[prec_index(b)](st, b->nenv, kind, objid, jacp, jacr, stream);
-  } else {
-    const void* lane = nullptr;
-    if ((rc = lane_image(b, &lane))) return rc;
-    rc = b->precision == B2_F64 ? b2::b2k_jacobian_f64(lane, b->model->cls, st, b->nenv, kind, objid, jacp, jacr, stream)
-                                : b2::b2k_jacobian_f32(lane, b->model->cls, st, b->nenv, kind, objid, jacp, jacr, stream);
-  }
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_jacobian launch") : B2_OK;
+  const void* lane = nullptr;
+  int rc = batch_images(b, &lane);
+  if (rc) return rc;
+  rc = b->model->lane[b->pi]->jacobian(lane, b->model->cls, st, b->nenv, kind, objid, jacp, jacr, stream);
+  return launched(rc, "b2_jacobian launch");
 }
 
 int b2_inverse(b2_batch* b, const b2_state* st, const void* qacc, void* qfrc_inverse, void* actuator_moment, void* stream) {
   B2_CHECK_STATE("b2_inverse");
   if (!qfrc_inverse) return fail(B2_ERR_ARG, "b2_inverse: qfrc_inverse is NULL");
   const void* lane = nullptr;
-  int rc = lane_image(b, &lane);  // one-shot setup call: always the generic kernels
+  int rc = batch_images(b, &lane);  // one-shot setup call: always the generic kernels
   if (rc) return rc;
-  rc = b->precision == B2_F64 ? b2::b2k_inverse_f64(lane, b->model->cls, st, b->nenv, qacc, qfrc_inverse, actuator_moment, stream)
-                              : b2::b2k_inverse_f32(lane, b->model->cls, st, b->nenv, qacc, qfrc_inverse, actuator_moment, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_inverse launch") : B2_OK;
+  return launched(b->k->inverse(lane, b->model->cls, st, b->nenv, qacc, qfrc_inverse, actuator_moment, stream), "b2_inverse launch");
 }
 
 int b2_lqr_set_gain(b2_batch* b, const double* K, const double* qpos_ref, const double* ctrl_ref) {
@@ -475,16 +414,6 @@ int b2_lqr_set_gain(b2_batch* b, const double* K, const double* qpos_ref, const 
   return B2_OK;
 }
 
-static int do_lqr_control(b2_batch* b, const b2_state* st, int count, void* stream) {
-  const void* lane = nullptr;
-  int rc = lane_image(b, &lane);
-  if (rc) return rc;
-  rc = b->precision == B2_F64 ? b2::b2k_lqr_control_f64(lane, b->model->cls, st, count, b->nenv, b->d_gain, stream)
-                              : b2::b2k_lqr_control_f32(lane, b->model->cls, st, count, b->nenv, b->d_gain, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_lqr_control launch") : B2_OK;
-}
-
 int b2_lqr_control(b2_batch* b, const b2_state* st, void* stream) {
   B2_CHECK_STATE("b2_lqr_control");
   if (!b->d_gain) return fail(B2_ERR_ARG, "b2_lqr_control: call b2_lqr_set_gain first");
@@ -496,7 +425,9 @@ static int shadow_state(b2_batch* b, b2_state* out) {
   const b2m_view& v = b->model->v;
   const size_t N = (size_t)b->nenv, es = b->esz, nu1 = v.nu ? v.nu : 1;
   if (!b->d_shadow) {
-    cudaError_t e = cudaMalloc(&b->d_shadow, (v.nq + 2 * (size_t)v.nv + nu1) * N * es);
+    cudaError_t e = cudaSetDevice(b->device);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+    e = cudaMalloc(&b->d_shadow, (v.nq + 2 * (size_t)v.nv + nu1) * N * es);
     if (e != cudaSuccess) return cuda_fail(e, "shadow state cudaMalloc");
   }
   char* p = (char*)b->d_shadow;
@@ -521,32 +452,26 @@ int b2_control_tick(b2_batch* b, const b2_state* st, const b2_derived* derived, 
   const void* gain = use_lqr ? b->d_gain : nullptr;
   const b2m_view& v = b->model->v;
   b->shadow_has_prestep = false;
-  if (!active_spec(b)) {
-    int rc = prepare_warp(b);
-    if (rc) return rc;
-    if (b->warp_mode == 1) {
-      // large models: control-law launch, FD on the warp engine, step on the warp engine.  Without a `derived`
-      // argument the pre-step state is parked in the shadow arrays for b2_refresh_derived, as in the fused form.
-      if (gain && (rc = do_lqr_control(b, st, b->nenv, stream))) return rc;
-      if ((rc = do_linearize(b, st, b->nenv, eps, centered, A, B, stream))) return rc;
-      if (!derived && st->qacc_warmstart) {  // the step kernel parks the pre-step state itself
-        b2_state shadow;
-        if ((rc = shadow_state(b, &shadow)) || (rc = do_step(b, st, b->nenv, 1, nullptr, stream, nullptr, &shadow))) return rc;
-        b->shadow_has_prestep = true;
-        return B2_OK;
-      }
-      return do_step(b, st, b->nenv, 1, derived, stream);
+  if (on_warp_engine(b)) {
+    // large models: control-law launch, FD on the warp engine, step on the warp engine.  Without a `derived`
+    // argument the pre-step state is parked in the shadow arrays for b2_refresh_derived, as in the fused form.
+    int rc;
+    if (gain && (rc = do_lqr_control(b, st, b->nenv, stream))) return rc;
+    if ((rc = do_linearize(b, st, b->nenv, eps, centered, A, B, stream))) return rc;
+    if (!derived && st->qacc_warmstart) {  // the step kernel parks the pre-step state itself
+      b2_state shadow;
+      if ((rc = shadow_state(b, &shadow)) || (rc = do_step(b, st, b->nenv, 1, nullptr, stream, nullptr, &shadow))) return rc;
+      b->shadow_has_prestep = true;
+      return B2_OK;
     }
+    return do_step(b, st, b->nenv, 1, derived, stream);
   }
   if (!derived && v.integrator == 0 && st->qacc_warmstart && (v.nu == 0 || st->ctrl)) {
     b2_state shadow;
     int rc = shadow_state(b, &shadow);
     if (rc) return rc;
     if ((rc = do_linearize(b, st, b->nenv, eps, centered, A, B, stream, gain, &shadow))) return rc;
-    rc = b->precision == B2_F64 ? b2::b2k_commit_state_f64(st, &shadow, b->nenv, b->nenv, v.nq, v.nv, v.nu, stream)
-                                : b2::b2k_commit_state_f32(st, &shadow, b->nenv, b->nenv, v.nq, v.nv, v.nu, stream);
-    g_launches++;
-    if (rc) return cuda_fail((cudaError_t)rc, "commit launch");
+    if ((rc = launched(b->k->commit_state(st, &shadow, b->nenv, b->nenv, v.nq, v.nv, v.nu, stream), "commit launch"))) return rc;
     b->shadow_has_prestep = true;
     return B2_OK;
   }
@@ -559,9 +484,6 @@ int b2_step_lazy(b2_batch* b, const b2_state* st, void* stream) {
   B2_CHECK_STATE("b2_step_lazy");
   if (!st->qacc_warmstart) return fail(B2_ERR_ARG, "b2_step_lazy: state.qacc_warmstart is required");
   int rc;
-  if (!active_spec(b)) {
-    if ((rc = prepare_warp(b))) return rc;
-  }
   // the step kernel (lane or warp engine) has the pre-step state at hand and writes it to the shadow arrays itself
   b2_state shadow;
   if ((rc = shadow_state(b, &shadow))) return rc;
@@ -584,24 +506,18 @@ int b2_refresh_derived(b2_batch* b, const b2_derived* derived, void* stream) {
 int b2_integrate_pos(b2_batch* b, void* qpos, const void* qvel, double dt, void* stream) {
   if (!b || !qpos || !qvel) return fail(B2_ERR_ARG, "b2_integrate_pos: null pointer");
   const void* lane = nullptr;
-  int rc = lane_image(b, &lane);
+  int rc = batch_images(b, &lane);
   if (rc) return rc;
-  rc = b->precision == B2_F64 ? b2::b2k_integrate_pos_f64(lane, b->model->cls, qpos, qvel, dt, b->nenv, stream)
-                              : b2::b2k_integrate_pos_f32(lane, b->model->cls, qpos, qvel, dt, b->nenv, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_integrate_pos launch") : B2_OK;
+  return launched(b->k->integrate_pos(lane, b->model->cls, qpos, qvel, dt, b->nenv, stream), "b2_integrate_pos launch");
 }
 
 int b2_differentiate_pos(b2_batch* b, void* out, double dt, const void* q1, const void* q2, void* stream) {
   if (!b || !out || !q1 || !q2) return fail(B2_ERR_ARG, "b2_differentiate_pos: null pointer");
   if (dt == 0) return fail(B2_ERR_ARG, "b2_differentiate_pos: dt must be nonzero");
   const void* lane = nullptr;
-  int rc = lane_image(b, &lane);
+  int rc = batch_images(b, &lane);
   if (rc) return rc;
-  rc = b->precision == B2_F64 ? b2::b2k_differentiate_pos_f64(lane, b->model->cls, out, dt, q1, q2, b->nenv, stream)
-                              : b2::b2k_differentiate_pos_f32(lane, b->model->cls, out, dt, q1, q2, b->nenv, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_differentiate_pos launch") : B2_OK;
+  return launched(b->k->differentiate_pos(lane, b->model->cls, out, dt, q1, q2, b->nenv, stream), "b2_differentiate_pos launch");
 }
 
 // Host-buffer step.  The env range is cut into chunks that flow through a small pool of streams:
@@ -640,12 +556,10 @@ int b2_step_host(b2_batch* b, const b2_state* hs, int nsteps, int linearize, dou
     direct = mapped(host_A, &map_A) && (!host_B || mapped(host_B, &map_B));
   }
   if (linearize && !direct && ((e = need(&b->d_A, nx * nx * N * es)) || (e = need(&b->d_B, nx * nu1 * N * es)))) return cuda_fail(e, "b2_step_host: cudaMalloc");
-  int rc = prepare_warp(b);
-  if (rc) return rc;
   // chunking: warp-engine batches and small batches go through in one piece
   // two chunks measured best at N = 65536 (1.72e8 vs 1.55e8 with 4, 0.94e8 with 16): every extra chunk adds ~11 copy nodes
   // (an async call overlaps with the other batch's call instead: one chunk measured best there, 1.93e8 vs 1.89e8)
-  const int nchunk = (b->warp_mode == 1 || N < 4096 || async) ? 1 : 2;
+  const int nchunk = (b->warp || N < 4096 || async) ? 1 : 2;
   if (!b->pipe_ready) {
     for (int i = 0; i < 3; i++) if ((e = cudaStreamCreateWithFlags(&b->pipe[i], cudaStreamNonBlocking))) return cuda_fail(e, "cudaStreamCreate");
     for (int i = 0; i < 3; i++) if ((e = cudaEventCreateWithFlags(&b->pipe_ev[i], cudaEventDisableTiming))) return cuda_fail(e, "cudaEventCreate");
@@ -740,12 +654,9 @@ int b2_lqr_control_env(b2_batch* b, const b2_state* st, const void* K_env, void*
   if (!b->d_gain) return fail(B2_ERR_ARG, "b2_lqr_control_env: call b2_lqr_set_gain first (qpos_ref / ctrl_ref come from it)");
   if (!K_env) return fail(B2_ERR_ARG, "b2_lqr_control_env: K_env is NULL");
   const void* lane = nullptr;
-  int rc = lane_image(b, &lane);
+  int rc = batch_images(b, &lane);
   if (rc) return rc;
-  rc = b->precision == B2_F64 ? b2::b2k_lqr_control_env_f64(lane, b->model->cls, st, b->nenv, b->nenv, b->d_gain, K_env, stream)
-                              : b2::b2k_lqr_control_env_f32(lane, b->model->cls, st, b->nenv, b->nenv, b->d_gain, K_env, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_lqr_control_env launch") : B2_OK;
+  return launched(b->k->lqr_control_env(lane, b->model->cls, st, b->nenv, b->nenv, b->d_gain, K_env, stream), "b2_lqr_control_env launch");
 }
 
 int b2_random_controls(b2_batch* b, const b2_state* st, double lo, double hi, unsigned long long seed, int watch_row, double watch_min,
@@ -760,11 +671,8 @@ int b2_random_controls(b2_batch* b, const b2_state* st, double lo, double hi, un
     if ((e = cudaMalloc(&b->d_rng_ctr, sizeof(unsigned) * (size_t)b->nenv)) || (e = cudaMemset(b->d_rng_ctr, 0, sizeof(unsigned) * (size_t)b->nenv)))
       return cuda_fail(e, "b2_random_controls: draw counters");
   }
-  const int rc = b->precision == B2_F64
-                     ? b2::b2k_random_controls_f64(st, b->nenv, v.nq, v.nv, v.nu, lo, hi, seed, b->d_rng_ctr, watch_row, watch_min, reset_qpos, reset_qvel, stream)
-                     : b2::b2k_random_controls_f32(st, b->nenv, v.nq, v.nv, v.nu, lo, hi, seed, b->d_rng_ctr, watch_row, watch_min, reset_qpos, reset_qvel, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_random_controls launch") : B2_OK;
+  return launched(b->k->random_controls(st, b->nenv, v.nq, v.nv, v.nu, lo, hi, seed, b->d_rng_ctr, watch_row, watch_min, reset_qpos, reset_qvel, stream),
+                  "b2_random_controls launch");
 }
 
 // Batched discrete LQR synthesis (see include/b2mj.h).  Q, R are host arrays shared by all envs; R is inverted here.
@@ -813,8 +721,7 @@ int b2_dlqr(int device, int precision, const void* A, const void* B, const doubl
       cache.emplace_back(std::move(key), dqr);
     }
   }
-  const int rc = precision == B2_F64 ? b2::b2k_dare_f64(A, B, dqr, nx, nu, nenv, max_doublings, tol, K, P, status, stream)
-                                     : b2::b2k_dare_f32(A, B, dqr, nx, nu, nenv, max_doublings, tol, K, P, status, stream);
+  const int rc = kernels(precision)->dare(A, B, dqr, nx, nu, nenv, max_doublings, tol, K, P, status, stream);
   g_launches++;
   if (rc == (int)cudaErrorInvalidValue) return fail(B2_ERR_CAPACITY, "b2_dlqr: nx too large for the shared-memory workspace of one SM");
   return rc ? cuda_fail((cudaError_t)rc, "b2_dlqr launch") : B2_OK;
@@ -853,11 +760,8 @@ int b2_recorder_record(b2_recorder* r, double time, void* out_slot, void* stream
   if (!r || !out_slot) return fail(B2_ERR_ARG, "b2_recorder_record: null pointer");
   cudaError_t e = cudaSetDevice(r->batch->device);
   if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-  const int rc = r->batch->precision == B2_F64
-                     ? b2::b2k_record_rows_f64(r->d_cols, r->ncol, r->d_index, r->nsel, r->batch->nenv, time, out_slot, stream)
-                     : b2::b2k_record_rows_f32(r->d_cols, r->ncol, r->d_index, r->nsel, r->batch->nenv, time, out_slot, stream);
-  g_launches++;
-  return rc ? cuda_fail((cudaError_t)rc, "b2_recorder_record launch") : B2_OK;
+  return launched(r->batch->k->record_rows(r->d_cols, r->ncol, r->d_index, r->nsel, r->batch->nenv, time, out_slot, stream),
+                  "b2_recorder_record launch");
 }
 void b2_recorder_destroy(b2_recorder* r) {
   if (!r) return;
@@ -868,7 +772,7 @@ void b2_recorder_destroy(b2_recorder* r) {
 
 int b2_warp_queue_histogram(b2_batch* b, int* hist16, void* stream) {
   if (!b || !hist16) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: null pointer");
-  if (b->warp_mode != 1) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: batch does not run on the warp engine's ordered queue");
+  if (!b->warp) return fail(B2_ERR_ARG, "b2_warp_queue_histogram: batch does not run on the warp engine's ordered queue");
   cudaError_t e = cudaSetDevice(b->device);
   if (!e) e = cudaStreamSynchronize((cudaStream_t)stream);
   int bins[64] = {0};
@@ -882,7 +786,7 @@ int b2_fp_peak(int precision, int device, double* tflops) {
   if (!tflops || (precision != B2_F64 && precision != B2_F32)) return fail(B2_ERR_ARG, "b2_fp_peak: bad arguments");
   cudaError_t e = cudaSetDevice(device);
   if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-  const double v = precision == B2_F64 ? b2::b2k_fma_peak_f64(nullptr) : b2::b2k_fma_peak_f32(nullptr);
+  const double v = kernels(precision)->fma_peak(nullptr);
   g_launches += 6;
   if (v < 0) return fail(B2_ERR_CUDA, "b2_fp_peak: kernel failed");
   *tflops = v;

@@ -1,7 +1,6 @@
 // Generic (runtime-model) instantiation of the lane-engine kernels for ONE arithmetic type.
 // Included by b2_kernels_f64.cu and b2_kernels_f32.cu with B2_REAL / B2_SUFFIX defined; each
-// translation unit owns its own __constant__ model images (one per size class), so the two
-// precisions do not share the 64 KB constant bank.
+// translation unit exports its launchers as one Kernels table (b2_kernels.h), kernels_f64 or kernels_f32.
 #include <cuda_runtime.h>
 
 #include <cstdio>
@@ -77,16 +76,16 @@ __global__ void __launch_bounds__(256) k_fma_peak(real* out, int iters, real a, 
 #define B2_FN(name) B2_CAT(name, B2_SUFFIX)
 
 // the lane engine's model image of a size class: size, and fill on the host (uploaded once per model by the C-ABI layer)
-size_t B2_FN(b2k_image_bytes)(int cls) {
+static size_t b2k_image_bytes(int cls) {
   size_t n = 0;
   B2_DISPATCH(cls, n = sizeof(DevModel<real, DD>));
   return n;
 }
-void B2_FN(b2k_image_fill)(int cls, const b2m_view* v, const int* disabled, void* host) {
+static void b2k_image_fill(int cls, const b2m_view* v, const int* disabled, void* host) {
   B2_DISPATCH(cls, fill_dev_model(*reinterpret_cast<DevModel<real, DD>*>(host), *v, disabled));
 }
 // returns measured TFLOP/s (2 flops per FMA) or a negative cudaError
-double B2_FN(b2k_fma_peak)(void* stream) {
+static double b2k_fma_peak(void* stream) {
   int dev = 0, sms = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -113,7 +112,7 @@ double B2_FN(b2k_fma_peak)(void* stream) {
   const double flops = 2.0 * 8.0 * iters * (double)threads * blocks;
   return flops / (best * 1e-3) / 1e12;
 }
-int B2_FN(b2k_step)(const void* image, int cls, const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain,
+static int b2k_step(const void* image, int cls, const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain,
                     const b2_state* park, void* stream) {
   int rc = 0;
   B2_DISPATCH(cls, (rc = launch_step<real, DD, RuntimeModel<DD>>(image, st, out, count, N, nsteps, gain, park, stream)));
@@ -152,12 +151,12 @@ static int warp_occupancy(K kern, int wpb, size_t smem, int* per_sm) {
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kern, wpb * 32, smem) != cudaSuccess || *per_sm < 1) return -1;
   return 0;
 }
-size_t B2_FN(b2k_warp_image_bytes)() { return sizeof(WarpImage<real>); }
-void B2_FN(b2k_warp_image_fill)(const b2m_view* v, const int* disabled, void* host) {
+static size_t b2k_warp_image_bytes() { return sizeof(WarpImage<real>); }
+static void b2k_warp_image_fill(const b2m_view* v, const int* disabled, void* host) {
   fill_warp_image(*reinterpret_cast<WarpImage<real>*>(host), *v, disabled);
 }
 // chooses warps-per-block / grid so that every SM is filled; returns the number of warp slots (scratch slots)
-int B2_FN(b2k_warp_plan)(const b2m_view* v, int N, int* out_wpb, int* out_blocks) {
+static int b2k_warp_plan(const b2m_view* v, int N, int* out_wpb, int* out_blocks) {
   int dev = 0, sms = 0, smem_max = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -174,12 +173,12 @@ int B2_FN(b2k_warp_plan)(const b2m_view* v, int N, int* out_wpb, int* out_blocks
   *out_wpb = wpb; *out_blocks = blocks;
   return blocks * wpb;
 }
-size_t B2_FN(b2k_warp_scratch_bytes)(const b2m_view* v, int slots) {
+static size_t b2k_warp_scratch_bytes(const b2m_view* v, int slots) {
   return (size_t)slots * warp_slot_reals(v->nv) * sizeof(real);
 }
 // bytes of the cost-ordered queue's buffers behind the work-queue counter: [hist | cursor] (2 kCostBins ints), cost[N], perm[N]
-size_t B2_FN(b2k_warp_sort_bytes)(int N) { return (2 * kCostBins + 2 * (size_t)N) * sizeof(int); }
-int B2_FN(b2k_warp_step)(const void* image, const b2m_view* v, const b2_state* st, const b2_derived* out, int N, int nsteps, void* jscratch,
+static size_t b2k_warp_sort_bytes(int N) { return (2 * kCostBins + 2 * (size_t)N) * sizeof(int); }
+static int b2k_warp_step(const void* image, const b2m_view* v, const b2_state* st, const b2_derived* out, int N, int nsteps, void* jscratch,
                          void* counter, void* sortbuf, int wpb, int blocks, const b2_state* park, void* stream) {
   const size_t smem = warp_block_smem(v, wpb, 0);
   cudaStream_t s = (cudaStream_t)stream;
@@ -202,7 +201,7 @@ int B2_FN(b2k_warp_step)(const void* image, const b2m_view* v, const b2_state* s
   return (int)cudaGetLastError();
 }
 // FD linearisation on the warp engine: same scratch slots as the step plan (wpb warps per block)
-int B2_FN(b2k_warp_linearize)(const void* image, const b2m_view* v, const b2_state* st, int N, double eps, int centered, void* A, void* B,
+static int b2k_warp_linearize(const void* image, const b2m_view* v, const b2_state* st, int N, double eps, int centered, void* A, void* B,
                               void* jscratch, void* counter, int wpb, int blocks, void* stream) {
   const size_t smem = warp_block_smem(v, wpb, 2 * (v->nq + v->nv));
   int per_sm = 0, dev = 0, sms = 0, rc = 0;
@@ -218,7 +217,7 @@ int B2_FN(b2k_warp_linearize)(const void* image, const b2m_view* v, const b2_sta
   return (int)cudaGetLastError();
 }
 // ntask: FD tasks per env (fd_task_count of the model)
-int B2_FN(b2k_linearize)(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A, void* B,
+static int b2k_linearize(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A, void* B,
                          const void* gain, const b2_state* shadow, void* stream) {
   int rc = 0;
   B2_DISPATCH(cls, (rc = launch_linearize<real, DD, RuntimeModel<DD>>(image, st, count, N, ntask, eps, centered, A, B, gain, shadow, nullptr,
@@ -226,38 +225,38 @@ int B2_FN(b2k_linearize)(const void* image, int cls, const b2_state* st, int cou
   return rc;
 }
 // (A, B) and the sensor Jacobians from the same rollouts (k_linearize<..., SENS = true>); no control law, no env advance
-int B2_FN(b2k_linearize_sensors)(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A,
+static int b2k_linearize_sensors(const void* image, int cls, const b2_state* st, int count, int N, int ntask, double eps, int centered, void* A,
                                  void* B, void* dsdx, void* dsdu, void* stream) {
   int rc = 0;
   B2_DISPATCH(cls, (rc = launch_linearize<real, DD, RuntimeModel<DD>, true>(image, st, count, N, ntask, eps, centered, A, B, nullptr, nullptr,
                                                                             dsdx, dsdu, stream)));
   return rc;
 }
-int B2_FN(b2k_commit_state)(const b2_state* st, const b2_state* shadow, int count, int N, int nq, int nv, int nu, void* stream) {
+static int b2k_commit_state(const b2_state* st, const b2_state* shadow, int count, int N, int nq, int nv, int nu, void* stream) {
   int bx = (count + 255) / 256;
   if (bx > 148 * 8) bx = 148 * 8;
   k_commit_state<real><<<dim3(bx, nq + 2 * nv + nu), 256, 0, (cudaStream_t)stream>>>(to_dev<real>(st), to_dev<real>(shadow), count, N, nq, nv, nu);
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_jacobian)(const void* image, int cls, const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {
+static int b2k_jacobian(const void* image, int cls, const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {
   int rc = 0;
   B2_DISPATCH(cls, (rc = launch_jacobian<real, DD, RuntimeModel<DD>>(image, st, N, kind, objid, jacp, jacr, stream)));
   return rc;
 }
-int B2_FN(b2k_inverse)(const void* image, int cls, const b2_state* st, int N, const void* qacc, void* qfrc, void* moment, void* stream) {
+static int b2k_inverse(const void* image, int cls, const b2_state* st, int N, const void* qacc, void* qfrc, void* moment, void* stream) {
   const int threads = 128, blocks = (N + threads - 1) / threads;
   B2_DISPATCH(cls, (k_inverse<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
                        to_dev<real>(st), N, (const real*)qacc, (real*)qfrc, (real*)moment, image)));
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_lqr_control)(const void* image, int cls, const b2_state* st, int count, int N, const void* gain, void* stream) {
+static int b2k_lqr_control(const void* image, int cls, const b2_state* st, int count, int N, const void* gain, void* stream) {
   const int threads = 128, blocks = (count + threads - 1) / threads;
   B2_DISPATCH(cls, (k_lqr_control<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
                        to_dev<real>(st), count, N, (const real*)gain, image)));
   return (int)cudaGetLastError();
 }
 // batched DARE / LQR gains: one warp per env, as many warps per block as the shared-memory workspace allows (at most four)
-int B2_FN(b2k_dare)(const void* A, const void* B, const void* qr /* device: Q, R, Rinv */, int nx, int nu, int N, int max_doublings,
+static int b2k_dare(const void* A, const void* B, const void* qr /* device: Q, R, Rinv */, int nx, int nu, int N, int max_doublings,
                     double tol, void* K, void* P, int* status, void* stream) {
   const real* qd = (const real*)qr;
   // small systems: one env per thread, compile-time sizes
@@ -284,42 +283,51 @@ int B2_FN(b2k_dare)(const void* A, const void* B, const void* qr /* device: Q, R
       (const real*)A, (const real*)B, q, q + nx * nx, q + nx * nx + nu * nu, nx, nu, N, max_doublings, (real)tol, (real*)K, (real*)P, status);
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_lqr_control_env)(const void* image, int cls, const b2_state* st, int count, int N, const void* gain, const void* K_env, void* stream) {
+static int b2k_lqr_control_env(const void* image, int cls, const b2_state* st, int count, int N, const void* gain, const void* K_env, void* stream) {
   const int threads = 128, blocks = (count + threads - 1) / threads;
   B2_DISPATCH(cls, (k_lqr_control_env<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
                        to_dev<real>(st), count, N, (const real*)gain, (const real*)K_env, image)));
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_random_controls)(const b2_state* st, int N, int nq, int nv, int nu, double lo, double hi, unsigned long long seed, void* ctr,
+static int b2k_random_controls(const b2_state* st, int N, int nq, int nv, int nu, double lo, double hi, unsigned long long seed, void* ctr,
                                int watch_row, double watch_min, const void* reset_qpos, const void* reset_qvel, void* stream) {
   k_random_controls<real><<<(N + 255) / 256, 256, 0, (cudaStream_t)stream>>>(to_dev<real>(st), N, nq, nv, nu, (real)lo, (real)hi, seed,
                                                                              (unsigned*)ctr, watch_row, (real)watch_min,
                                                                              (const real*)reset_qpos, (const real*)reset_qvel);
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_record_rows)(const void* cols, int ncol, const int* env_index, int nsel, int N, double time, void* out, void* stream) {
+static int b2k_record_rows(const void* cols, int ncol, const int* env_index, int nsel, int N, double time, void* out, void* stream) {
   const int threads = 128;
   k_record_rows<real><<<dim3((nsel + threads - 1) / threads, ncol), threads, 0, (cudaStream_t)stream>>>(
       (const RecordColDev*)cols, env_index, nsel, N, (real)time, (real*)out);
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_integrate_pos)(const void* image, int cls, void* qpos, const void* qvel, double dt, int N, void* stream) {
+static int b2k_integrate_pos(const void* image, int cls, void* qpos, const void* qvel, double dt, int N, void* stream) {
   const int threads = 128, blocks = (N + threads - 1) / threads;
   B2_DISPATCH(cls, (k_integrate_pos<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
                        (real*)qpos, (const real*)qvel, (real)dt, N, image)));
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_differentiate_pos)(const void* image, int cls, void* out, double dt, const void* q1, const void* q2, int N, void* stream) {
+static int b2k_differentiate_pos(const void* image, int cls, void* out, double dt, const void* q1, const void* q2, int N, void* stream) {
   const int threads = 128, blocks = (N + threads - 1) / threads;
   B2_DISPATCH(cls, (k_differentiate_pos<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
                        (real*)out, (real)dt, (const real*)q1, (const real*)q2, N, image)));
   return (int)cudaGetLastError();
 }
-int B2_FN(b2k_rollout)(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq,
+static int b2k_rollout(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq,
                        void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {
   int rc = 0;
   B2_DISPATCH(cls, (rc = launch_rollout<real, DD, RuntimeModel<DD>>(image, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream)));
   return rc;
 }
+
+// in the member order of Kernels (b2_kernels.h)
+const Kernels B2_FN(kernels) = {
+    {b2k_step, b2k_linearize, b2k_linearize_sensors, b2k_jacobian, b2k_rollout},
+    b2k_inverse, b2k_lqr_control, b2k_lqr_control_env, b2k_integrate_pos, b2k_differentiate_pos,
+    b2k_commit_state, b2k_random_controls, b2k_record_rows, b2k_dare, b2k_fma_peak,
+    b2k_image_bytes, b2k_image_fill,
+    b2k_warp_plan, b2k_warp_scratch_bytes, b2k_warp_image_bytes, b2k_warp_image_fill, b2k_warp_sort_bytes, b2k_warp_step, b2k_warp_linearize,
+};
 
 }  // namespace b2

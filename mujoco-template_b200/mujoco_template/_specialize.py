@@ -5,7 +5,7 @@ accessors return compile-time constants (function-local ``constexpr`` tables), e
 capacity constants, launchers for the step / linearize / jacobian / rollout kernels instantiated with that
 provider, and a registrar keyed by the FNV-1a hash of the model blob.  ``libb2mj.so`` picks the
 specialised kernels automatically when ``b2_model_create`` sees a blob with a registered hash;
-any other model runs on the generic (constant-memory) kernels.
+any other model runs on the generic kernels.
 
 Run by ``__graft_entry__.build()`` for the example models before ``make``.
 """
@@ -124,7 +124,7 @@ def emit_spec(compiled: dict, name: str) -> str:
     # generated sources of sensorless models do not change with it
     has_sensors = int(c["nsensordata"]) > 0
     A('#include "../b2_kernel_templates.cuh"')
-    A('#include "../b2_spec_registry.h"')
+    A('#include "../b2_kernels.h"')
     A("")
     A("namespace b2 {")
     A("namespace {")
@@ -150,33 +150,35 @@ def emit_spec(compiled: dict, name: str) -> str:
         A(f"  static B2_DEV T {k}(int i) {{ static constexpr T t[{one(v.size)}] = {{{body}}}; return t[i]; }}")
     A("};")
     A("")
-    # launchers: b2_kernel_templates.cuh's launch_* own block size and grid; the FD task count is the kernel's own rule,
-    # evaluated on the host from the provider's constexpr accessors
+    # launchers with the LaneKernels signatures (b2_kernels.h): b2_kernel_templates.cuh's launch_* own block size and grid;
+    # the static provider needs no model image, and the caller passes the FD task count
+    lane = "const void*, int, const b2_state* st"
     for T, suf in (("double", ""), ("float", "32")):
         M = f"{T}, SDims, SModel<{T}>"
-        ntask = f"fd_task_count(SModel<{T}>::integrator(), SModel<{T}>::nv(), SModel<{T}>::nu())"
-        A(f"int spec_step{suf}(const b2_state* st, const b2_derived* out, int count, int N, int nsteps, const void* gain, const b2_state* park, void* stream) {{")
+        A(f"int spec_step{suf}({lane}, const b2_derived* out, int count, int N, int nsteps, const void* gain, const b2_state* park, void* stream) {{")
         A(f"  return launch_step<{M}>(nullptr, st, out, count, N, nsteps, gain, park, stream);")
         A("}")
-        A(f"int spec_linearize{suf}(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, const void* gain, const b2_state* shadow, void* stream) {{")
-        A(f"  return launch_linearize<{M}>(nullptr, st, count, N, {ntask}, eps, centered, A, B, gain, shadow, nullptr, nullptr, stream);")
+        A(f"int spec_linearize{suf}({lane}, int count, int N, int ntask, double eps, int centered, void* A, void* B, const void* gain, const b2_state* shadow, void* stream) {{")
+        A(f"  return launch_linearize<{M}>(nullptr, st, count, N, ntask, eps, centered, A, B, gain, shadow, nullptr, nullptr, stream);")
         A("}")
         if has_sensors:
             # (A, B) plus the sensor Jacobians from the same rollouts: no control law, no advance
-            A(f"int spec_linearize_sensors{suf}(const b2_state* st, int count, int N, double eps, int centered, void* A, void* B, void* dsdx, void* dsdu, void* stream) {{")
-            A(f"  return launch_linearize<{M}, true>(nullptr, st, count, N, {ntask}, eps, centered, A, B, nullptr, nullptr, dsdx, dsdu, stream);")
+            A(f"int spec_linearize_sensors{suf}({lane}, int count, int N, int ntask, double eps, int centered, void* A, void* B, void* dsdx, void* dsdu, void* stream) {{")
+            A(f"  return launch_linearize<{M}, true>(nullptr, st, count, N, ntask, eps, centered, A, B, nullptr, nullptr, dsdx, dsdu, stream);")
             A("}")
-        A(f"int spec_jacobian{suf}(const b2_state* st, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {{")
+        A(f"int spec_jacobian{suf}({lane}, int N, int kind, int objid, void* jacp, void* jacr, void* stream) {{")
         A(f"  return launch_jacobian<{M}>(nullptr, st, N, kind, objid, jacp, jacr, stream);")
         A("}")
     # the rollout kernels come after all the others: cicc's inlining, and so the other kernels' code, depends on kernel order
     for T, suf in (("double", ""), ("float", "32")):
-        A(f"int spec_rollout{suf}(const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {{")
+        A(f"int spec_rollout{suf}({lane}, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {{")
         A(f"  return launch_rollout<{T}, SDims, SModel<{T}>>(nullptr, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);")
         A("}")
-    sens_init = "{spec_linearize_sensors, spec_linearize_sensors32}" if has_sensors else "{nullptr, nullptr}"
-    A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{spec_step, spec_step32}}, '
-      f'{{spec_linearize, spec_linearize32}}, {{spec_jacobian, spec_jacobian32}}, {sens_init}, {{spec_rollout, spec_rollout32}}}};')
+    lanes = []
+    for suf in ("", "32"):
+        sens = f"spec_linearize_sensors{suf}" if has_sensors else "nullptr"
+        lanes.append(f"{{spec_step{suf}, spec_linearize{suf}, {sens}, spec_jacobian{suf}, spec_rollout{suf}}}")
+    A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{{lanes[0]}, {lanes[1]}}}}};')
     A("struct Registrar { Registrar() { register_spec(&kSpec); } } registrar;")
     A("}  // namespace")
     A("}  // namespace b2")

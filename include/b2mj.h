@@ -16,7 +16,8 @@
  *    default stream) unless stated otherwise.  Device memory is allocated in b2_model_create /
  *    b2_batch_create (model images, warp-engine scratch) and on the FIRST call of the entry points
  *    that need extra buffers (b2_control_tick / b2_step_lazy: shadow state; b2_step_host: staging;
- *    b2_lqr_set_gain); b2_step, b2_rollout, b2_forward, b2_linearize, b2_linearize_sensors and b2_jacobian never allocate.
+ *    b2_lqr_set_gain); b2_step, b2_rollout, b2_forward, b2_linearize, b2_linearize_sensors,
+ *    b2_linearize_rollout and b2_jacobian never allocate.
  *  - No process-wide model state: a model's constants live in per-model device images handed to
  *    every launch, so batches of different models can be driven from different threads and streams,
  *    and a captured CUDA graph replays with the model it was captured with.  One b2_batch must not be
@@ -134,6 +135,31 @@ int b2_linearize(b2_batch* batch, const b2_state* state, double eps, int centere
  * follow B's ctrlrange rules.  Any of A, B, C, D may be NULL, but not all four.  Without sensors this is b2_linearize.
  * State is not modified; never allocates. */
 int b2_linearize_sensors(b2_batch* batch, const b2_state* state, double eps, int centered, void* A, void* B, void* C, void* D,
+                         void* stream);
+
+/* Linearisation along a rollout (iLQR / DDP, time-varying LQR about a nominal trajectory, the linear model of MPC): the
+ * transition and sensor Jacobians at every step of an open-loop control sequence.  Exactly the loop, on a COPY s of state,
+ *     X[0] <- s
+ *     for t = 0 .. nsteps-1:  s.ctrl <- ctrl_seq[t];  b2_linearize_sensors(s, eps, centered, A[t], B[t], C[t], D[t]);
+ *                             b2_step(s, 1);  X[t+1] <- s
+ * On the lane engine it is two launches for any nsteps: the nominal rollout, then the FD of every step at once.
+ * ctrl_seq    (nsteps, nu, nenv) as in b2_rollout; NULL = hold state.ctrl
+ * A, B        (nsteps, 2nv, 2nv, nenv), (nsteps, 2nv, nu, nenv): b2_linearize's layout with the step outermost
+ * C, D        (nsteps, nsensordata, 2nv, nenv), (nsteps, nsensordata, nu, nenv); ignored when the model has no sensors.
+ *             Any of A, B, C, D may be NULL, but not all four.
+ * qpos_traj   (nsteps+1, nq, nenv), required: row 0 is x0, row t+1 the state after step t -- the nominal the FD reads
+ * qvel_traj   (nsteps+1, nv, nenv), required: likewise
+ * warm_traj   (nsteps+1, nv, nenv): the qacc_warmstart each step starts from (row 0: state.qacc_warmstart); required when
+ *             state.qacc_warmstart is non-NULL, ignored when it is NULL (every step then starts from zeros, as b2_step)
+ * sensor_traj (nsteps, nsensordata, nenv): the nominal reading of step t, as b2_rollout records it; may be NULL; ignored
+ *             when the model has no sensors
+ * State is not modified, except that flags get every bit the loop would set OR-ed in.  A diverged env is frozen from the
+ * step that detects it, as in b2_rollout: its remaining state and warm rows repeat the frozen state, its remaining sensor
+ * rows are NaN, and its later Jacobians are the FD about the frozen state.  Offsets are 64-bit; never allocates; capturable
+ * in a CUDA graph.  nsteps < 1, a NULL qpos_traj / qvel_traj, a NULL warm_traj with a warm start, or all four Jacobians
+ * NULL: B2_ERR_ARG; eps <= 0: B2_ERR_LINEARIZE. */
+int b2_linearize_rollout(b2_batch* batch, const b2_state* state, int nsteps, const void* ctrl_seq, double eps, int centered,
+                         void* A, void* B, void* C, void* D, void* qpos_traj, void* qvel_traj, void* warm_traj, void* sensor_traj,
                          void* stream);
 
 /* Replaces mj.mj_jacSite / mj_jacBody / mj_jacBodyCom / mj_jacSubtreeCom

@@ -337,6 +337,48 @@ static int do_linearize(b2_batch* b, const b2_state* st, int count, double eps, 
                : lk->linearize(lane, m->cls, st, count, b->nenv, ntask, eps, centered, A, B, gain, shadow, stream);
   return launched(rc, "linearize launch");
 }
+// b2_linearize_rollout.  Lane engine: the nominal rollout, then one FD launch over every (step, env).  Warp engine (no
+// sensors): the contract's loop itself on the trajectory rows, which serve as the working state -- a humanoid FD launch
+// takes milliseconds, so a launch pair per step costs nothing.  warm_traj is null exactly when the state has no warm start.
+static int do_linearize_rollout(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_seq, double eps, int centered, void* A, void* B,
+                                void* C, void* D, void* qpos_traj, void* qvel_traj, void* warm_traj, void* sensor_traj, void* stream) {
+  const b2_model* m = b->model;
+  const b2m_view& v = m->v;
+  const void* lane = nullptr;
+  int rc = batch_images(b, &lane);
+  if (rc) return rc;
+  if (on_warp_engine(b)) {
+    const size_t N = (size_t)b->nenv, es = b->esz, ndx = 2 * (size_t)v.nv, qpos_bytes = v.nq * N * es, qvel_bytes = v.nv * N * es;
+    const size_t ctrl_bytes = v.nu * N * es, A_bytes = ndx * ndx * N * es, B_bytes = ndx * v.nu * N * es;
+    cudaStream_t s = (cudaStream_t)stream;
+    // row t of the trajectories as a state, with the controls of step t (the warp kernels only read state.ctrl)
+    auto row = [&](int t) {
+      return b2_state{(char*)qpos_traj + t * qpos_bytes, (char*)qvel_traj + t * qvel_bytes,
+                      ctrl_seq ? (char*)ctrl_seq + t * ctrl_bytes : st->ctrl, warm_traj ? (char*)warm_traj + t * qvel_bytes : nullptr, st->flags};
+    };
+    auto copy_row = [&](const b2_state& dst, const b2_state& src) {
+      cudaError_t e = cudaMemcpyAsync(dst.qpos, src.qpos, qpos_bytes, cudaMemcpyDefault, s);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(dst.qvel, src.qvel, qvel_bytes, cudaMemcpyDefault, s);
+      if (e == cudaSuccess && warm_traj) e = cudaMemcpyAsync(dst.qacc_warmstart, src.qacc_warmstart, qvel_bytes, cudaMemcpyDefault, s);
+      return e == cudaSuccess ? B2_OK : cuda_fail(e, "b2_linearize_rollout: trajectory row copy");
+    };
+    if ((rc = copy_row(row(0), *st))) return rc;
+    for (int t = 0; t < nsteps; t++) {
+      const b2_state x = row(t);
+      if ((A || B) && (rc = do_linearize(b, &x, b->nenv, eps, centered, A ? (char*)A + t * A_bytes : nullptr, B ? (char*)B + t * B_bytes : nullptr, stream)))
+        return rc;
+      b2_state next = row(t + 1);
+      next.ctrl = x.ctrl;
+      if ((rc = copy_row(next, x)) || (rc = do_step(b, &next, b->nenv, 1, nullptr, stream))) return rc;
+    }
+    return B2_OK;
+  }
+  const int ntask = b2::fd_task_count(v.integrator, v.nv, v.nu);
+  rc = m->lane[b->pi]->linearize_rollout(lane, m->cls, st, b->nenv, ntask, nsteps, ctrl_seq, eps, centered, A, B, C, D, qpos_traj, qvel_traj,
+                                         warm_traj, sensor_traj, stream);
+  if (A || B || C || D) g_launches++;  // the FD launch
+  return launched(rc, "linearize_rollout launch");
+}
 
 int b2_step(b2_batch* b, const b2_state* st, int nsteps, const b2_derived* derived, void* stream) {
   B2_CHECK_STATE("b2_step");
@@ -373,6 +415,20 @@ int b2_linearize_sensors(b2_batch* b, const b2_state* st, double eps, int center
   if (v.nsensordata == 0 || (!C && !D)) return (A || B) ? do_linearize(b, st, b->nenv, eps, centered, A, B, stream) : B2_OK;
   if (!b->model->lane[b->pi]->linearize_sensors) return fail(B2_ERR_ARG, "b2_linearize_sensors: specialised kernel set has no sensor variant");
   return do_linearize(b, st, b->nenv, eps, centered, A, B, stream, nullptr, nullptr, C, D);
+}
+
+int b2_linearize_rollout(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_seq, double eps, int centered, void* A, void* B, void* C,
+                         void* D, void* qpos_traj, void* qvel_traj, void* warm_traj, void* sensor_traj, void* stream) {
+  if (nsteps < 1) return fail(B2_ERR_ARG, "b2_linearize_rollout: nsteps must be >= 1");
+  if (!qpos_traj || !qvel_traj) return fail(B2_ERR_ARG, "b2_linearize_rollout: qpos_traj and qvel_traj are required");
+  if (st && st->qacc_warmstart && !warm_traj) return fail(B2_ERR_ARG, "b2_linearize_rollout: warm_traj is required with a warm start");
+  if (!A && !B && !C && !D) return fail(B2_ERR_ARG, "b2_linearize_rollout: A, B, C and D are all NULL");
+  if (!(eps > 0)) return fail(B2_ERR_LINEARIZE, "b2_linearize_rollout: eps must be > 0");
+  B2_CHECK_STATE("b2_linearize_rollout");
+  const b2m_view& v = b->model->v;
+  const bool sens = v.nsensordata != 0;
+  return do_linearize_rollout(b, st, nsteps, v.nu ? ctrl_seq : nullptr, eps, centered, A, B, sens ? C : nullptr, sens ? D : nullptr,
+                              qpos_traj, qvel_traj, st->qacc_warmstart ? warm_traj : nullptr, sens ? sensor_traj : nullptr, stream);
 }
 
 int b2_jacobian(b2_batch* b, const b2_state* st, int kind, int objid, void* jacp, void* jacr, void* stream) {

@@ -694,4 +694,142 @@ auto launch_rollout(const void* image, const b2_state* st, const b2_derived* out
   return (int)cudaGetLastError();
 }
 
+// Linearisation along a rollout (b2_linearize_rollout), launch 1 of 2: the nominal trajectory.  k_rollout's step loop,
+// reading x0 from the state and writing nothing back to it but flags: row 0 of qpos_traj (nsteps+1, nq, N), qvel_traj and
+// warm_traj (nsteps+1, nv, N) is x0, row s+1 the state after step s, and row s of warm_traj the qacc_warmstart step s starts
+// from.  warm_traj null: no warm start, every step starts from zeros as b2_step does without one.  sensor_traj
+// (nsteps, nsensordata, N) as in k_rollout.  A diverged env is frozen as in k_rollout: its remaining state and warm rows
+// repeat the state it is frozen in, its remaining sensor rows are NaN.  (A kernel of its own, so k_rollout stays as it is.)
+template <typename T, class D, class M>
+__global__ void __launch_bounds__(128, 1) k_nominal_traj(StateDev<T> st, int N, int nsteps, const T* __restrict__ ctrl_seq, T* qpos_traj,
+                                                         T* qvel_traj, T* warm_traj, T* sensor_traj, const void* image = nullptr) {
+  model_load<M>(image, 0);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  RowStore<T, D> rows;
+  LaneEnv<T, D, M> env(rows);
+  constexpr bool kLate = LaneEnv<T, D, M>::kLateMass;
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu(), nsd = M::nsensor() > 0 ? M::nsensordata() : 0;
+  load_state(env, st, N, e);
+  auto store_row = [&](int r) {
+    B2_UNROLL
+    for (int k = 0; k < nq; k++) qpos_traj[((size_t)r * nq + k) * N + e] = env.qpos[k];
+    B2_UNROLL
+    for (int k = 0; k < nv; k++) qvel_traj[((size_t)r * nv + k) * N + e] = env.qvel[k];
+    if (warm_traj) { B2_UNROLL for (int k = 0; k < nv; k++) warm_traj[((size_t)r * nv + k) * N + e] = env.warm[k]; }
+  };
+  store_row(0);
+  int s = 0;
+  B2_NOUNROLL
+  for (; s < nsteps; s++) {
+    if (ctrl_seq) { B2_UNROLL for (int k = 0; k < nu; k++) env.ctrl[k] = ctrl_seq[((size_t)s * nu + k) * N + e]; }
+    if (!warm_traj) { B2_UNROLL for (int k = 0; k < nv; k++) env.warm[k] = T(0); }
+    env.check_state();
+    if (env.flags & 3) break;
+    env.template forward_position<kLate>();
+    env.forward_velocity();
+    env.template forward_acc<kLate>();
+    B2_UNROLL
+    for (int k = 0; k < nv; k++) if (!(fabs(env.qacc[k]) <= T(1e10))) env.flags |= 4;
+    if (sensor_traj && nsd > 0) {
+      T sd[D::NSD];
+      env.sensors(sd);
+      B2_UNROLL
+      for (int k = 0; k < nsd; k++) sensor_traj[((size_t)s * nsd + k) * N + e] = sd[k];
+    }
+    if (M::integrator() == 1) env.rk4(); else env.euler();
+    store_row(s + 1);
+  }
+  // frozen at step s (s == nsteps when the env never diverged)
+  B2_NOUNROLL
+  for (int r = s; r < nsteps; r++) {
+    store_row(r + 1);
+    if (sensor_traj && nsd > 0) { B2_UNROLL for (int k = 0; k < nsd; k++) sensor_traj[((size_t)r * nsd + k) * N + e] = T(__int_as_float(0x7fc00000)); }
+  }
+  if (st.flags && env.flags) st.flags[e] |= env.flags;
+}
+
+// Launch 2 of 2: the FD columns of every step of the nominal trajectory in one launch, one thread per (task, step, env) --
+// k_linearize's task decomposition and fd_column, task-major (the long group tasks of Euler models start first), then step,
+// env fastest.  A thread's nominal state is row t of the trajectory arrays, its controls row t of ctrl_seq (null: the
+// state's held controls); its outputs are step t of A (nsteps, 2nv, 2nv, N), B (nsteps, 2nv, nu, N) and, with SENS,
+// dsdx (nsteps, nsensordata, 2nv, N) and dsdu (nsteps, nsensordata, nu, N).  No control law, no env advance.
+template <typename T, class D, class M, bool SENS = false>
+__global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize_traj(StateDev<T> st, int N, int nsteps, T eps, int centered,
+                                                                                      const T* __restrict__ ctrl_seq, T* qpos_traj, T* qvel_traj,
+                                                                                      T* warm_traj, T* A, T* B, T* dsdx, T* dsdu,
+                                                                                      const void* image = nullptr) {
+  model_load<M>(image, 0);
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu(), ndx = 2 * nv;
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int ntask = fd_task_count(M::integrator(), nv, nu);
+  const long long per_task = (long long)nsteps * N, total = per_task * ntask;
+  if (idx >= total) return;
+  // 32-bit division when the launch fits (a 64-bit one is ~100 instructions)
+  int e, t, task;
+  if (total <= 0x7fffffffLL) {
+    const unsigned u = (unsigned)idx, r = u % (unsigned)per_task;
+    task = (int)(u / (unsigned)per_task); t = (int)(r / (unsigned)N); e = (int)(r - (unsigned)t * (unsigned)N);
+  } else {
+    const long long r = idx % per_task;
+    task = (int)(idx / per_task); t = (int)(r / N); e = (int)(r - (long long)t * N);
+  }
+  RowStore<T, D> rows;
+  LaneEnv<T, D, M> env(rows);
+  T u0[D::NU];
+  B2_UNROLL
+  for (int k = 0; k < nu; k++) u0[k] = ctrl_seq ? ctrl_seq[((size_t)t * nu + k) * N + e] : st.ctrl[(size_t)k * N + e];
+  typedef typename std::conditional<SENS, NominalWithSensors<T>, NominalInMemory<T>>::type Nominal;
+  Nominal nom;
+  nom.st.qpos = qpos_traj + (size_t)t * nq * N;
+  nom.st.qvel = qvel_traj + (size_t)t * nv * N;
+  nom.st.warm = warm_traj ? warm_traj + (size_t)t * nv * N : nullptr;
+  nom.st.ctrl = nullptr;
+  nom.st.flags = nullptr;
+  nom.N = N; nom.e = e; nom.u0 = u0;
+  if constexpr (SENS) {
+    const size_t nsd = M::nsensordata();
+    nom.dsdx = dsdx ? dsdx + (size_t)t * nsd * ndx * N : nullptr;
+    nom.dsdu = dsdu ? dsdu + (size_t)t * nsd * nu * N : nullptr;
+  }
+  T* At = A ? A + (size_t)t * ndx * ndx * N : nullptr;
+  T* Bt = B ? B + (size_t)t * ndx * nu * N : nullptr;
+  const bool grouped = M::integrator() == 0;  // not a constant expression for the runtime provider
+  const int groups = fd_group_count(nv, nu);
+  int c0 = task, c1 = task + 1;
+  if (grouped) {
+    if (task < groups) { c0 = nv + task * B2_FD_GROUP; c1 = c0 + B2_FD_GROUP < ndx + nu ? c0 + B2_FD_GROUP : ndx + nu; }
+    else { c0 = task - groups; c1 = c0 + 1; }
+  }
+  bool pos_valid = false, vel_valid = false;
+  const T inv_eps = T(1) / eps;
+  // mj_checkPos / mj_checkVel once on the nominal state, as k_linearize does
+  B2_UNROLL
+  for (int k = 0; k < nq; k++) env.qpos[k] = nom.q(k);
+  B2_UNROLL
+  for (int k = 0; k < nv; k++) env.qvel[k] = nom.v(k);
+  env.check_state();
+  B2_NOUNROLL
+  for (int c = c0; c < c1; c++) fd_column(env, nom, c, false, eps, inv_eps, centered, N, e, At, Bt, pos_valid, vel_valid);
+  if (st.flags && env.flags) atomicOr(st.flags + e, env.flags);
+}
+// Both launches of b2_linearize_rollout.  ntask: FD tasks per env (fd_task_count of the model).  The FD launch is skipped
+// when there is no Jacobian to write.
+template <typename T, class D, class M, bool SENS = false>
+auto launch_linearize_rollout(const void* image, const b2_state* st, int N, int ntask, int nsteps, const void* ctrl_seq, double eps,
+                              int centered, void* A, void* B, void* dsdx, void* dsdu, void* qpos_traj, void* qvel_traj, void* warm_traj,
+                              void* sensor_traj, void* stream) {
+  const StateDev<T> s = to_dev<T>(st);
+  k_nominal_traj<T, D, M><<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(s, N, nsteps, (const T*)ctrl_seq, (T*)qpos_traj, (T*)qvel_traj,
+                                                                             (T*)warm_traj, (T*)sensor_traj, image);
+  cudaError_t rc = cudaGetLastError();
+  if (rc != cudaSuccess || !(A || B || dsdx || dsdu)) return (int)rc;
+  const long long total = (long long)nsteps * N * ntask;
+  const unsigned blocks = (unsigned)((total + B2_LIN_THREADS - 1) / B2_LIN_THREADS);
+  k_linearize_traj<T, D, M, SENS><<<blocks, B2_LIN_THREADS, 0, (cudaStream_t)stream>>>(s, N, nsteps, (T)eps, centered, (const T*)ctrl_seq,
+                                                                                        (T*)qpos_traj, (T*)qvel_traj, (T*)warm_traj, (T*)A,
+                                                                                        (T*)B, (T*)dsdx, (T*)dsdu, image);
+  return (int)cudaGetLastError();
+}
+
 }  // namespace b2

@@ -29,6 +29,12 @@ struct LaneKernels {
   // b2_rollout: per-step controls and the recorded trajectory of every env in one launch (k_rollout)
   int (*rollout)(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_seq,
                  void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream);
+  // b2_linearize_rollout: the nominal trajectory (k_nominal_traj), then the FD of every step in one launch
+  // (k_linearize_traj); dsdx / dsdu non-null selects the sensor variant, which a specialised set has only for models with
+  // sensors
+  int (*linearize_rollout)(const void* image, int cls, const b2_state* st, int N, int ntask, int nsteps, const void* ctrl_seq, double eps,
+                           int centered, void* A, void* B, void* dsdx, void* dsdu, void* qpos_traj, void* qvel_traj, void* warm_traj,
+                           void* sensor_traj, void* stream);
 };
 
 // The generic kernels of one precision (b2_kernels_impl.cuh).

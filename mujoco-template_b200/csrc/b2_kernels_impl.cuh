@@ -320,10 +320,22 @@ static int b2k_rollout(const void* image, int cls, const b2_state* st, const b2_
   B2_DISPATCH(cls, (rc = launch_rollout<real, DD, RuntimeModel<DD>>(image, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream)));
   return rc;
 }
+static int b2k_linearize_rollout(const void* image, int cls, const b2_state* st, int N, int ntask, int nsteps, const void* ctrl_seq, double eps,
+                                 int centered, void* A, void* B, void* dsdx, void* dsdu, void* qpos_traj, void* qvel_traj, void* warm_traj,
+                                 void* sensor_traj, void* stream) {
+  int rc = 0;
+  if (!dsdx && !dsdu)
+    B2_DISPATCH(cls, (rc = launch_linearize_rollout<real, DD, RuntimeModel<DD>>(image, st, N, ntask, nsteps, ctrl_seq, eps, centered, A, B,
+                                                                               nullptr, nullptr, qpos_traj, qvel_traj, warm_traj, sensor_traj, stream)))
+  else
+    B2_DISPATCH(cls, (rc = launch_linearize_rollout<real, DD, RuntimeModel<DD>, true>(image, st, N, ntask, nsteps, ctrl_seq, eps, centered, A, B,
+                                                                                     dsdx, dsdu, qpos_traj, qvel_traj, warm_traj, sensor_traj, stream)))
+  return rc;
+}
 
 // in the member order of Kernels (b2_kernels.h)
 const Kernels B2_FN(kernels) = {
-    {b2k_step, b2k_linearize, b2k_linearize_sensors, b2k_jacobian, b2k_rollout},
+    {b2k_step, b2k_linearize, b2k_linearize_sensors, b2k_jacobian, b2k_rollout, b2k_linearize_rollout},
     b2k_inverse, b2k_lqr_control, b2k_lqr_control_env, b2k_integrate_pos, b2k_differentiate_pos,
     b2k_commit_state, b2k_random_controls, b2k_record_rows, b2k_dare, b2k_fma_peak,
     b2k_image_bytes, b2k_image_fill,

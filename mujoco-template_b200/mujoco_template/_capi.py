@@ -23,7 +23,7 @@ _lib: C.CDLL | None = None
 # every symbol include/b2mj.h declares (tests check the shared object exports all of them)
 EXPORTED_SYMBOLS = (
     "b2_model_create", "b2_model_destroy", "b2_model_set_actuator_disabled", "b2_batch_create",
-    "b2_batch_destroy", "b2_step", "b2_rollout", "b2_forward", "b2_linearize", "b2_linearize_sensors", "b2_jacobian", "b2_integrate_pos",
+    "b2_batch_destroy", "b2_step", "b2_rollout", "b2_forward", "b2_linearize", "b2_linearize_sensors", "b2_linearize_rollout", "b2_jacobian", "b2_integrate_pos",
     "b2_differentiate_pos", "b2_inverse", "b2_lqr_set_gain", "b2_lqr_control", "b2_control_tick", "b2_refresh_derived", "b2_step_lazy", "b2_step_host", "b2_step_host_wait", "b2_stream_synchronize", "b2_launch_count",
     "b2_batch_size_class", "b2_last_error", "b2_version", "b2_fp_peak", "b2_batch_kernel_variant",
     "b2_recorder_create", "b2_recorder_record", "b2_recorder_destroy", "b2_dlqr", "b2_random_controls", "b2_warp_queue_histogram", "b2_lqr_control_env",
@@ -80,6 +80,7 @@ def lib() -> C.CDLL:
     L.b2_forward.argtypes = [vp, C.POINTER(State), C.POINTER(Derived), vp]
     L.b2_linearize.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp]
     L.b2_linearize_sensors.argtypes = [vp, C.POINTER(State), d, i, vp, vp, vp, vp, vp]
+    L.b2_linearize_rollout.argtypes = [vp, C.POINTER(State), i, vp, d, i, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.b2_jacobian.argtypes = [vp, C.POINTER(State), i, i, vp, vp, vp]
     L.b2_inverse.argtypes = [vp, C.POINTER(State), vp, vp, vp, vp]
     L.b2_lqr_set_gain.argtypes = [vp, C.POINTER(d), C.POINTER(d), C.POINTER(d)]
@@ -183,6 +184,14 @@ class NativeBatch:
                           D_: int | None, stream: int = 0) -> None:
         """``b2_linearize_sensors``: (A, B) and the sensor Jacobians C = d sensordata / dx, D = d sensordata / du."""
         check(self._L.b2_linearize_sensors(self.handle, C.byref(state), float(eps), int(bool(centered)), A, B, C_, D_, stream))
+
+    def linearize_rollout(self, state: State, nsteps: int, ctrl_seq: int | None, eps: float, centered: bool, A: int | None,
+                          B: int | None, C_: int | None, D_: int | None, qpos_traj: int, qvel_traj: int, warm_traj: int | None,
+                          sensor_traj: int | None, stream: int = 0) -> None:
+        """``b2_linearize_rollout``: (A, B, C, D) at every step of the open-loop rollout under ``ctrl_seq`` (nsteps, nu, nenv)
+        (None: held controls), about the nominal trajectory it records into the (nsteps+1, dim, nenv) arrays."""
+        check(self._L.b2_linearize_rollout(self.handle, C.byref(state), int(nsteps), ctrl_seq, float(eps), int(bool(centered)), A, B,
+                                           C_, D_, qpos_traj, qvel_traj, warm_traj, sensor_traj, stream))
 
     def jacobian(self, state: State, kind: int, objid: int, jacp: int, jacr: int | None, stream: int = 0) -> None:
         check(self._L.b2_jacobian(self.handle, C.byref(state), int(kind), int(objid), jacp, jacr, stream))

@@ -379,6 +379,33 @@ class NativeBackend:
                      *[t.data_ptr() if t.numel() else None for t in bufs])
         return tuple(bufs)
 
+    def linearize_rollout(self, ctrl_seq, nsteps: int, eps: float, centered: bool, sensors: bool, out=None):
+        """(A, B) -- and with ``sensors`` (C, D) -- at every step of the open-loop rollout under ``ctrl_seq``
+        (``b2_linearize_rollout``): the loop ``ctrl <- ctrl_seq[t]; linearize_sensors; step(1)`` on a copy of the state,
+        which is left as it is (flags apart).  ``ctrl_seq``: a (nsteps, nu, nenv) tensor, or None (the controls held).
+
+        Returns (A, B, C, D, qpos, qvel, warm, sensordata) of shapes (T, 2nv, 2nv, nenv), (T, 2nv, nu, nenv),
+        (T, nsensordata, 2nv, nenv), (T, nsensordata, nu, nenv), (T+1, nq, nenv), (T+1, nv, nenv), (T+1, nv, nenv) and
+        (T, nsensordata, nenv): the Jacobians of step t and the nominal trajectory they linearise about (row 0 is the
+        state, row t+1 the state after step t, warm the warm start each step starts from).  C, D and sensordata are None
+        unless ``sensors`` and the model has sensors; warm is None when the state has no warm start.  Fresh buffers unless
+        ``out`` gives all eight (fixed addresses under graph capture); an entry of ``out`` may be None (not written)."""
+        torch, m = self.torch, self.model
+        T, nx, ns = int(nsteps), 2 * m.nv, m.nsensordata
+        if out is None:
+            mk = ((lambda *shape: torch.zeros(shape, dtype=self.dtype).pin_memory()) if self.host_mapped else
+                  (lambda *shape: torch.empty(shape, device=f"cuda:{self.device}", dtype=self.dtype)))
+            sens = bool(sensors) and ns > 0
+            out = (mk(T, nx, nx, self.nenv), mk(T, nx, m.nu, self.nenv),
+                   mk(T, ns, nx, self.nenv) if sens else None, mk(T, ns, m.nu, self.nenv) if sens else None,
+                   mk(T + 1, m.nq, self.nenv), mk(T + 1, m.nv, self.nenv),
+                   mk(T + 1, m.nv, self.nenv) if self._ptr("qacc_warmstart") else None, mk(T, ns, self.nenv) if sens else None)
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
+        A, B, C_, D_, q, v, w, s = out
+        self._launch("linearize_rollout", self.batch.linearize_rollout, self.state_struct(), T, ptr(ctrl_seq) if m.nu else None,
+                     eps, centered, ptr(A), ptr(B), ptr(C_), ptr(D_), ptr(q), ptr(v), ptr(w), ptr(s))
+        return tuple(out)
+
     def jacobian(self, kind: int, objid: int, want_rot: bool):
         torch, m = self.torch, self.model
         mk = (lambda: torch.zeros((3, m.nv, self.nenv), dtype=self.dtype).pin_memory()) if self.host_mapped else (

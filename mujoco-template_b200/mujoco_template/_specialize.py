@@ -174,10 +174,20 @@ def emit_spec(compiled: dict, name: str) -> str:
         A(f"int spec_rollout{suf}({lane}, const b2_derived* out, int N, int nsteps, const void* ctrl_seq, void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {{")
         A(f"  return launch_rollout<{T}, SDims, SModel<{T}>>(nullptr, st, out, N, nsteps, ctrl_seq, qpos_traj, qvel_traj, sensor_traj, stream);")
         A("}")
+    # ... and the linearisation along a rollout after them; its sensor variant only for models with sensors (the C-ABI
+    # passes no dsdx / dsdu for a model without)
+    for T, suf in (("double", ""), ("float", "32")):
+        M = f"{T}, SDims, SModel<{T}>"
+        A(f"int spec_linearize_rollout{suf}({lane}, int N, int ntask, int nsteps, const void* ctrl_seq, double eps, int centered, void* A, void* B, void* dsdx, void* dsdu, void* qpos_traj, void* qvel_traj, void* warm_traj, void* sensor_traj, void* stream) {{")
+        call = "(nullptr, st, N, ntask, nsteps, ctrl_seq, eps, centered, A, B, {}, qpos_traj, qvel_traj, warm_traj, sensor_traj, stream);"
+        if has_sensors:
+            A(f"  if (dsdx || dsdu) return launch_linearize_rollout<{M}, true>" + call.format("dsdx, dsdu"))
+        A(f"  return launch_linearize_rollout<{M}>" + call.format("nullptr, nullptr"))
+        A("}")
     lanes = []
     for suf in ("", "32"):
         sens = f"spec_linearize_sensors{suf}" if has_sensors else "nullptr"
-        lanes.append(f"{{spec_step{suf}, spec_linearize{suf}, {sens}, spec_jacobian{suf}, spec_rollout{suf}}}")
+        lanes.append(f"{{spec_step{suf}, spec_linearize{suf}, {sens}, spec_jacobian{suf}, spec_rollout{suf}, spec_linearize_rollout{suf}}}")
     A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{{lanes[0]}, {lanes[1]}}}}};')
     A("struct Registrar { Registrar() { register_spec(&kSpec); } } registrar;")
     A("}  // namespace")

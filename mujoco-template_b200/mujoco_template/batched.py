@@ -338,26 +338,8 @@ class BatchedEnv:
         leaves it), as permuted views of fresh ``(T, dim, nenv)`` buffers.  An env that diverges is flagged and frozen: its
         remaining rows repeat its frozen state, and its remaining sensor rows are NaN.  Otherwise returns None.
         ``data.time`` advances by T timesteps and the derived arrays are those of the last step."""
-        backend, m = self.data.backend, self.model
-        seq = None
-        if controls is not None:
-            import torch
-
-            if m.nu == 0:
-                raise ConfigError("rollout(controls=...): the model has no actuators (nu=0)")
-            if not isinstance(controls, torch.Tensor) or controls.dim() != 3 or controls.shape[0] != self.nenv or controls.shape[2] != m.nu:
-                raise ConfigError(f"rollout(controls=...): expected a (nenv={self.nenv}, T, nu={m.nu}) tensor, got "
-                                  f"{tuple(controls.shape) if isinstance(controls, torch.Tensor) else type(controls).__name__}")
-            ref = self.data.qpos
-            if controls.device != ref.device or controls.dtype != ref.dtype:
-                raise ConfigError(f"rollout(controls=...): expected {ref.dtype} on {ref.device}, got {controls.dtype} on {controls.device}")
-            if nsteps is not None and int(nsteps) != controls.shape[1]:
-                raise ConfigError(f"rollout: nsteps={nsteps} disagrees with the {controls.shape[1]} rows of controls")
-            nsteps = controls.shape[1]
-            seq = controls.permute(1, 2, 0).contiguous()  # (T, nu, nenv); no copy for a permuted (T, nu, nenv) buffer
-        if nsteps is None or int(nsteps) < 1:
-            raise ConfigError("nsteps must be >= 1")
-        nsteps = int(nsteps)
+        backend = self.data.backend
+        seq, nsteps = self._control_sequence("rollout", controls, nsteps)
         out = None
         if seq is None and not record:
             backend.step(nsteps)
@@ -371,6 +353,51 @@ class BatchedEnv:
         if out[2] is not None:
             traj["sensordata"] = out[2].permute(2, 0, 1)
         return traj
+
+    def _control_sequence(self, what: str, controls, nsteps):
+        """Validates a ``(nenv, T, nu)`` control tensor and ``nsteps``; returns the controls as a ``(T, nu, nenv)`` layout
+        (None without controls) and T."""
+        m = self.model
+        seq = None
+        if controls is not None:
+            import torch
+
+            if m.nu == 0:
+                raise ConfigError(f"{what}(controls=...): the model has no actuators (nu=0)")
+            if not isinstance(controls, torch.Tensor) or controls.dim() != 3 or controls.shape[0] != self.nenv or controls.shape[2] != m.nu:
+                raise ConfigError(f"{what}(controls=...): expected a (nenv={self.nenv}, T, nu={m.nu}) tensor, got "
+                                  f"{tuple(controls.shape) if isinstance(controls, torch.Tensor) else type(controls).__name__}")
+            ref = self.data.qpos
+            if controls.device != ref.device or controls.dtype != ref.dtype:
+                raise ConfigError(f"{what}(controls=...): expected {ref.dtype} on {ref.device}, got {controls.dtype} on {controls.device}")
+            if nsteps is not None and int(nsteps) != controls.shape[1]:
+                raise ConfigError(f"{what}: nsteps={nsteps} disagrees with the {controls.shape[1]} rows of controls")
+            nsteps = controls.shape[1]
+            seq = controls.permute(1, 2, 0).contiguous()  # (T, nu, nenv); no copy for a permuted (T, nu, nenv) buffer
+        if nsteps is None or int(nsteps) < 1:
+            raise ConfigError("nsteps must be >= 1")
+        return seq, int(nsteps)
+
+    def linearize_rollout(self, controls=None, nsteps: int | None = None, *, eps: float | None = None, centered: bool = True,
+                          sensors: bool = False):
+        """Transition Jacobians at every step of an open-loop control sequence (iLQR / DDP, time-varying LQR about a
+        nominal trajectory): the loop ``ctrl <- controls[:, t]; linearize(); step(1)`` run on a copy of the state, in two
+        kernel launches on the lane engine for any T.  ``controls`` and ``nsteps`` as in ``rollout`` (without controls the
+        current ones are held).  The controller is not called, and neither the state, ``data.time`` nor the
+        control-decimation counter moves (only flags are OR-ed in, as the loop would).
+
+        Returns a dict of ``(nenv, ...)`` views of fresh buffers: ``"qpos": (nenv, T+1, nq)`` and ``"qvel": (nenv, T+1, nv)``
+        -- the nominal trajectory, row 0 the current state and row t+1 the state after step t -- and ``"A": (nenv, T, 2nv,
+        2nv)``, ``"B": (nenv, T, 2nv, nu)``, the Jacobians about row t.  ``sensors=True`` on a model with sensors adds
+        ``"C": (nenv, T, nsensordata, 2nv)``, ``"D": (nenv, T, nsensordata, nu)`` and the nominal readings
+        ``"sensordata": (nenv, T, nsensordata)``.  An env that diverges is frozen as in ``rollout``."""
+        seq, nsteps = self._control_sequence("linearize_rollout", controls, nsteps)
+        eps = self.lin_eps if eps is None else float(eps)
+        A, B, C, D, qpos, qvel, _, sd = self.data.backend.linearize_rollout(seq, nsteps, eps, centered, sensors)
+        out = {"qpos": qpos.permute(2, 0, 1), "qvel": qvel.permute(2, 0, 1), "A": A.permute(3, 0, 1, 2), "B": B.permute(3, 0, 1, 2)}
+        if C is not None:
+            out.update(C=C.permute(3, 0, 1, 2), D=D.permute(3, 0, 1, 2), sensordata=sd.permute(2, 0, 1))
+        return out
 
     def passive(self, *, duration: float | None = None, max_steps: int | None = None, hooks=None,
                 return_obs: bool = True) -> Iterator[StepResult]:

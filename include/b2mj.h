@@ -16,7 +16,7 @@
  *    default stream) unless stated otherwise.  Device memory is allocated in b2_model_create /
  *    b2_batch_create (model images, warp-engine scratch) and on the FIRST call of the entry points
  *    that need extra buffers (b2_control_tick / b2_step_lazy: shadow state; b2_step_host: staging;
- *    b2_lqr_set_gain); b2_step, b2_rollout, b2_forward, b2_linearize, b2_linearize_sensors,
+ *    b2_lqr_set_gain); b2_step, b2_rollout, b2_rollout_feedback, b2_forward, b2_linearize, b2_linearize_sensors,
  *    b2_linearize_rollout and b2_jacobian never allocate.
  *  - No process-wide model state: a model's constants live in per-model device images handed to
  *    every launch, so batches of different models can be driven from different threads and streams,
@@ -162,6 +162,28 @@ int b2_linearize_rollout(b2_batch* batch, const b2_state* state, int nsteps, con
                          void* A, void* B, void* C, void* D, void* qpos_traj, void* qvel_traj, void* warm_traj, void* sensor_traj,
                          void* stream);
 
+/* Closed-loop rollout under a time-varying LQR law (the forward pass of iLQR / DDP, time-varying LQR tracking of a nominal
+ * trajectory).  Exactly the loop, for t = 0 .. nsteps-1,
+ *     state.ctrl <- clip(ctrl_nom[t] + alpha[e] k[t] - K[t] [qpos (-) qpos_nom[t] ; qvel - qvel_nom[t]], ctrlrange);
+ *     b2_step(batch, state, 1, t == nsteps-1 ? derived : NULL)
+ * with the state recorded after each step as in b2_rollout.  (-) is b2_differentiate_pos(dt = 1, qpos_nom[t] -> qpos): the
+ * tangent-space deviation of b2_lqr_control and of b2_linearize's A.  Clipping applies to ctrl-limited actuators only.
+ * ctrl_nom    (nsteps, nu, nenv), required
+ * qpos_nom    (>= nsteps, nq, nenv), qvel_nom (>= nsteps, nv, nenv): row t is the nominal state of step t; required.  Rows
+ *             0 .. nsteps-1 are read, so b2_linearize_rollout's (nsteps+1)-row trajectories serve as they are.
+ * K           (nsteps, nu, 2nv, nenv): b2_tvlqr's layout; required
+ * k           (nsteps, nu, nenv): feedforward terms; NULL = zero
+ * alpha       (nenv): step size per env (an iLQR line search is per env), in the batch's precision; NULL = 1
+ * ctrl_traj   (nsteps, nu, nenv): the control applied at step t; may be NULL
+ * qpos_traj, qvel_traj, sensor_traj, derived: as in b2_rollout; may be NULL.
+ * State, flags, derived arrays and diverged envs behave as in b2_rollout; a frozen env's remaining ctrl_traj rows are NaN and
+ * its state.ctrl keeps the last control it was given (otherwise state.ctrl holds the control of step nsteps-1).  On the
+ * lane engine it is one launch; offsets are 64-bit; never allocates; capturable in a CUDA graph.  nsteps < 1, a NULL
+ * required pointer or a model without actuators: B2_ERR_ARG. */
+int b2_rollout_feedback(b2_batch* batch, const b2_state* state, int nsteps, const void* ctrl_nom, const void* qpos_nom,
+                        const void* qvel_nom, const void* K, const void* k, const void* alpha, void* ctrl_traj, void* qpos_traj,
+                        void* qvel_traj, void* sensor_traj, const b2_derived* derived, void* stream);
+
 /* Replaces mj.mj_jacSite / mj_jacBody / mj_jacBodyCom / mj_jacSubtreeCom
  * (reference mujoco_template/jacobians.py:44,55,67,79).  jacp/jacr: (3, nv, nenv); jacr may be NULL. */
 int b2_jacobian(b2_batch* batch, const b2_state* state, int kind, int objid, void* jacp, void* jacr, void* stream);
@@ -252,6 +274,34 @@ int b2_random_controls(b2_batch* batch, const b2_state* state, double lo, double
  * status (device, nenv ints, may be NULL): doublings used, negative if a pivot underflowed.  Not tied to a batch. */
 int b2_dlqr(int device, int precision, const void* A, const void* B, const double* Q, const double* R, int nx, int nu, int nenv,
             int max_doublings, double tol, void* K, void* P, int* status, void* stream);
+
+/* Finite-horizon time-varying LQR about a trajectory, batched: the Riccati backward pass of TV-LQR, iLQR and DDP (without
+ * second-order dynamics terms) for every env from its own (A_t, B_t), t = 0 .. nsteps-1.  Deviations are in A's tangent
+ * space, dx = [q (-) qbar ; v - vbar] (nx = 2nv for b2_linearize_rollout's output), du = u - ubar, and u = -K dx as in
+ * b2_dlqr.  The cost is
+ *     J = sum_t [1/2 dx_t'Q dx_t + q_t'dx_t + 1/2 du_t'R du_t + r_t'du_t] + 1/2 dx_T'Qf dx_T + q_T'dx_T
+ * and, from P = Qf, s = q_T, for t = nsteps-1 .. 0:
+ *     Qx = q_t + A's   Qu = r_t + B's   Qxx = Q + A'PA   Quu = R + B'PB   Qux = B'PA
+ *     K_t = (Quu + reg I)^-1 Qux,   k_t = -(Quu + reg I)^-1 Qu          (Cholesky of Quu + reg I)
+ *     P <- Qxx + K'Quu K - K'Qux - Qux'K  (symmetrised),   s <- Qx - K'Qu - K'Quu k + Qux'k
+ *     dV0 += k'Qu,   dV1 += 1/2 k'Quu k
+ * so that the closed-loop control is ubar_t + alpha k_t - K_t dx_t (b2_rollout_feedback), and for a linear system
+ * alpha dV0 + alpha^2 dV1 is the change of J that step size alpha brings.  reg = 0 without q / r is plain TV-LQR; for a
+ * constant (A, B) and a long horizon K_0 and P0 approach b2_dlqr's K and P.
+ * DEVICE arrays, env fastest (element (t, i, j, e) at base[((t*rows + i)*cols + j)*nenv + e]):
+ *     A (nsteps, nx, nx, nenv), B (nsteps, nx, nu, nenv)  -- b2_linearize_rollout's layout, read in place
+ *     q (nsteps+1, nx, nenv), r (nsteps, nu, nenv)         -- may be NULL (zeros)
+ *     K (nsteps, nu, nx, nenv) required;  k (nsteps, nu, nenv), P0 (nx, nx, nenv), dV (2, nenv) may be NULL
+ *     status (nenv ints, may be NULL): 0, or -(t+1) when Quu_t + reg I is not positive definite (the first such t from the
+ *     end); that env's rows <= t of K and k, its P0 and its dV are then NaN.
+ * Q, Qf (nx x nx) and R (nu x nu): HOST arrays, row-major, shared by all envs; kept on the device by content as b2_dlqr
+ * keeps its weights, so that repeated calls neither allocate nor copy and can be captured in a CUDA graph.  One launch:
+ * a thread per env for (nx, nu) = (2, 1), (4, 1), (4, 2), otherwise a warp per env with its matrices in shared memory.
+ * Offsets are 64-bit.  Not tied to a batch.  nsteps, nx, nu or nenv < 1, reg < 0, a bad precision or a NULL A, B, Q, R, Qf
+ * or K: B2_ERR_ARG; an (nx, nu) whose workspace exceeds an SM's shared memory: B2_ERR_CAPACITY. */
+int b2_tvlqr(int device, int precision, int nsteps, int nx, int nu, int nenv, const void* A, const void* B, const double* Q,
+             const double* R, const double* Qf, const void* q, const void* r, double reg, void* K, void* k, void* P0, void* dV,
+             int* status, void* stream);
 
 /* Batched recorder sink: one CSV row per selected env and step, in the reference's column layout
  * (reference logging.py:81-247: time_s, qpos.., qvel.., ctrl.., probe columns).  A recorder is a column table

@@ -379,6 +379,37 @@ static int do_linearize_rollout(b2_batch* b, const b2_state* st, int nsteps, con
   if (A || B || C || D) g_launches++;  // the FD launch
   return launched(rc, "linearize_rollout launch");
 }
+// b2_rollout_feedback.  Lane engine: one k_rollout_feedback launch.  Warp engine: the contract's loop itself, as do_rollout
+// runs it, with a law launch (which also records the control row) in front of every warp step.
+static int do_rollout_feedback(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_nom, const void* qpos_nom, const void* qvel_nom,
+                               const void* K, const void* k, const void* alpha, void* ctrl_traj, void* qpos_traj, void* qvel_traj,
+                               void* sensor_traj, const b2_derived* derived, void* stream) {
+  const b2_model* m = b->model;
+  const b2m_view& v = m->v;
+  const void* lane = nullptr;
+  int rc = batch_images(b, &lane);
+  if (rc) return rc;
+  if (on_warp_engine(b)) {  // no sensors on the warp engine
+    const size_t N = (size_t)b->nenv, es = b->esz, ctrl_bytes = v.nu * N * es, qpos_bytes = v.nq * N * es, qvel_bytes = v.nv * N * es;
+    const size_t K_bytes = ctrl_bytes * 2 * v.nv;
+    cudaStream_t s = (cudaStream_t)stream;
+    for (int t = 0; t < nsteps; t++) {
+      rc = b->k->tvlqr_law(lane, m->cls, st, b->nenv, (const char*)ctrl_nom + t * ctrl_bytes, (const char*)qpos_nom + t * qpos_bytes,
+                           (const char*)qvel_nom + t * qvel_bytes, (const char*)K + t * K_bytes, k ? (const char*)k + t * ctrl_bytes : nullptr,
+                           alpha, ctrl_traj ? (char*)ctrl_traj + t * ctrl_bytes : nullptr, stream);
+      if ((rc = launched(rc, "b2_rollout_feedback: law launch"))) return rc;
+      if ((rc = do_step(b, st, b->nenv, 1, t == nsteps - 1 ? derived : nullptr, stream))) return rc;
+      cudaError_t e = cudaSuccess;
+      if (qpos_traj) e = cudaMemcpyAsync((char*)qpos_traj + t * qpos_bytes, st->qpos, qpos_bytes, cudaMemcpyDefault, s);
+      if (e == cudaSuccess && qvel_traj) e = cudaMemcpyAsync((char*)qvel_traj + t * qvel_bytes, st->qvel, qvel_bytes, cudaMemcpyDefault, s);
+      if (e != cudaSuccess) return cuda_fail(e, "b2_rollout_feedback: trajectory row copy");
+    }
+    return B2_OK;
+  }
+  rc = m->lane[b->pi]->rollout_feedback(lane, m->cls, st, derived, b->nenv, nsteps, ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, ctrl_traj,
+                                        qpos_traj, qvel_traj, sensor_traj, stream);
+  return launched(rc, "rollout_feedback launch");
+}
 
 int b2_step(b2_batch* b, const b2_state* st, int nsteps, const b2_derived* derived, void* stream) {
   B2_CHECK_STATE("b2_step");
@@ -429,6 +460,18 @@ int b2_linearize_rollout(b2_batch* b, const b2_state* st, int nsteps, const void
   const bool sens = v.nsensordata != 0;
   return do_linearize_rollout(b, st, nsteps, v.nu ? ctrl_seq : nullptr, eps, centered, A, B, sens ? C : nullptr, sens ? D : nullptr,
                               qpos_traj, qvel_traj, st->qacc_warmstart ? warm_traj : nullptr, sens ? sensor_traj : nullptr, stream);
+}
+
+int b2_rollout_feedback(b2_batch* b, const b2_state* st, int nsteps, const void* ctrl_nom, const void* qpos_nom, const void* qvel_nom,
+                        const void* K, const void* k, const void* alpha, void* ctrl_traj, void* qpos_traj, void* qvel_traj, void* sensor_traj,
+                        const b2_derived* derived, void* stream) {
+  if (nsteps < 1) return fail(B2_ERR_ARG, "b2_rollout_feedback: nsteps must be >= 1");
+  if (!ctrl_nom || !qpos_nom || !qvel_nom || !K) return fail(B2_ERR_ARG, "b2_rollout_feedback: ctrl_nom, qpos_nom, qvel_nom and K are required");
+  B2_CHECK_STATE("b2_rollout_feedback");
+  const b2m_view& v = b->model->v;
+  if (v.nu == 0) return fail(B2_ERR_ARG, "b2_rollout_feedback: the model has no actuators");
+  return do_rollout_feedback(b, st, nsteps, ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, ctrl_traj, qpos_traj, qvel_traj,
+                             v.nsensordata ? sensor_traj : nullptr, derived, stream);
 }
 
 int b2_jacobian(b2_batch* b, const b2_state* st, int kind, int objid, void* jacp, void* jacr, void* stream) {
@@ -731,6 +774,40 @@ int b2_random_controls(b2_batch* b, const b2_state* st, double lo, double hi, un
                   "b2_random_controls launch");
 }
 
+}  // extern "C"
+
+// The weight blocks of b2_dlqr (Q, R, R^-1) and b2_tvlqr (Q, R, Qf), converted to the call's precision, live on the device for
+// as long as the process does, keyed by their contents: repeated calls with the same weights (a controller that
+// re-synthesises its gains every tick, an iLQR iteration) neither allocate nor copy, and the calls can be captured into a
+// CUDA graph once the block exists.  The calling thread's current device must be `device`.
+static int resident_weights(int device, int precision, int nx, int nu, const std::vector<double>& vals, const char* who, void** out) {
+  const size_t esz = precision == B2_F64 ? 8 : 4;
+  std::vector<unsigned char> host(vals.size() * esz);
+  for (size_t i = 0; i < vals.size(); i++) {
+    if (precision == B2_F64) ((double*)host.data())[i] = vals[i]; else ((float*)host.data())[i] = (float)vals[i];
+  }
+  static std::mutex mu;
+  static std::vector<std::pair<std::vector<unsigned char>, void*>> cache;  // key: bytes, then device, precision and sizes
+  std::vector<unsigned char> key(host);
+  const int head[4] = {device, precision, nx, nu};
+  key.insert(key.end(), (const unsigned char*)head, (const unsigned char*)head + sizeof(head));
+  std::lock_guard<std::mutex> lock(mu);
+  for (auto& kv : cache) if (kv.first == key) { *out = kv.second; return B2_OK; }
+  void* d = nullptr;
+  cudaError_t e;
+  if ((e = cudaMalloc(&d, host.size())) != cudaSuccess) return cuda_fail(e, (std::string(who) + ": cudaMalloc").c_str());
+  if ((e = cudaMemcpy(d, host.data(), host.size(), cudaMemcpyHostToDevice)) != cudaSuccess) {
+    cudaFree(d);
+    return cuda_fail(e, (std::string(who) + ": upload").c_str());
+  }
+  if (cache.size() >= 64) { cudaFree(cache.front().second); cache.erase(cache.begin()); }
+  cache.emplace_back(std::move(key), d);
+  *out = d;
+  return B2_OK;
+}
+
+extern "C" {
+
 // Batched discrete LQR synthesis (see include/b2mj.h).  Q, R are host arrays shared by all envs; R is inverted here.
 int b2_dlqr(int device, int precision, const void* A, const void* B, const double* Q, const double* R, int nx, int nu, int nenv,
             int max_doublings, double tol, void* K, void* P, int* status, void* stream) {
@@ -751,36 +828,35 @@ int b2_dlqr(int device, int precision, const void* A, const void* B, const doubl
     for (int k = 0; k < 2 * nu; k++) aug[(size_t)c * 2 * nu + k] *= inv;
     for (int r = 0; r < nu; r++) if (r != c) { const double f = aug[(size_t)r * 2 * nu + c]; for (int k = 0; k < 2 * nu; k++) aug[(size_t)r * 2 * nu + k] -= f * aug[(size_t)c * 2 * nu + k]; }
   }
-  const size_t nqr = (size_t)nx * nx + 2 * (size_t)nu * nu, esz = precision == B2_F64 ? 8 : 4;
-  std::vector<unsigned char> host(nqr * esz);
-  for (size_t i = 0; i < nqr; i++) {
-    const double x = i < (size_t)nx * nx ? Q[i] : (i < (size_t)nx * nx + (size_t)nu * nu ? R[i - (size_t)nx * nx]
-                                                   : aug[((i - (size_t)nx * nx - (size_t)nu * nu) / nu) * 2 * nu + nu + (i - (size_t)nx * nx - (size_t)nu * nu) % nu]);
-    if (precision == B2_F64) ((double*)host.data())[i] = x; else ((float*)host.data())[i] = (float)x;
-  }
-  // The (Q, R, R^-1) block lives on the device for as long as the process does, keyed by its contents: repeated calls with the
-  // same weights (a controller that re-synthesises its gains every tick) neither allocate nor copy, and the call can be
-  // captured into a CUDA graph once the block exists.
+  std::vector<double> qr(Q, Q + (size_t)nx * nx);
+  qr.insert(qr.end(), R, R + (size_t)nu * nu);
+  for (int i = 0; i < nu; i++) qr.insert(qr.end(), aug.begin() + (size_t)i * 2 * nu + nu, aug.begin() + (size_t)(i + 1) * 2 * nu);
   void* dqr = nullptr;
-  {
-    static std::mutex mu;
-    static std::vector<std::pair<std::vector<unsigned char>, void*>> cache;  // key: device, sizes, bytes
-    std::vector<unsigned char> key(host);
-    const int head[4] = {device, precision, nx, nu};
-    key.insert(key.end(), (const unsigned char*)head, (const unsigned char*)head + sizeof(head));
-    std::lock_guard<std::mutex> lock(mu);
-    for (auto& kv : cache) if (kv.first == key) { dqr = kv.second; break; }
-    if (!dqr) {
-      if ((e = cudaMalloc(&dqr, nqr * esz)) != cudaSuccess) return cuda_fail(e, "b2_dlqr: cudaMalloc");
-      if ((e = cudaMemcpy(dqr, host.data(), nqr * esz, cudaMemcpyHostToDevice)) != cudaSuccess) { cudaFree(dqr); return cuda_fail(e, "b2_dlqr: upload"); }
-      if (cache.size() >= 64) { cudaFree(cache.front().second); cache.erase(cache.begin()); }
-      cache.emplace_back(std::move(key), dqr);
-    }
-  }
+  if (int rc = resident_weights(device, precision, nx, nu, qr, "b2_dlqr", &dqr)) return rc;
   const int rc = kernels(precision)->dare(A, B, dqr, nx, nu, nenv, max_doublings, tol, K, P, status, stream);
   g_launches++;
   if (rc == (int)cudaErrorInvalidValue) return fail(B2_ERR_CAPACITY, "b2_dlqr: nx too large for the shared-memory workspace of one SM");
   return rc ? cuda_fail((cudaError_t)rc, "b2_dlqr launch") : B2_OK;
+}
+
+// Finite-horizon time-varying LQR / iLQR backward pass (see include/b2mj.h).  Q, R, Qf are host arrays shared by all envs.
+int b2_tvlqr(int device, int precision, int nsteps, int nx, int nu, int nenv, const void* A, const void* B, const double* Q, const double* R,
+             const double* Qf, const void* q, const void* r, double reg, void* K, void* k, void* P0, void* dV, int* status, void* stream) {
+  if (nsteps < 1 || nx < 1 || nu < 1 || nenv < 1) return fail(B2_ERR_ARG, "b2_tvlqr: nsteps, nx, nu and nenv must be >= 1");
+  if (!(reg >= 0)) return fail(B2_ERR_ARG, "b2_tvlqr: reg must be >= 0");
+  if (precision != B2_F64 && precision != B2_F32) return fail(B2_ERR_ARG, "b2_tvlqr: precision must be 64 or 32");
+  if (!A || !B || !Q || !R || !Qf || !K) return fail(B2_ERR_ARG, "b2_tvlqr: A, B, Q, R, Qf and K are required");
+  cudaError_t e = cudaSetDevice(device);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
+  std::vector<double> w(Q, Q + (size_t)nx * nx);
+  w.insert(w.end(), R, R + (size_t)nu * nu);
+  w.insert(w.end(), Qf, Qf + (size_t)nx * nx);
+  void* dw = nullptr;
+  if (int rc = resident_weights(device, precision, nx, nu, w, "b2_tvlqr", &dw)) return rc;
+  const int rc = kernels(precision)->tvlqr(A, B, dw, q, r, nsteps, nx, nu, nenv, reg, K, k, P0, dV, status, stream);
+  g_launches++;
+  if (rc == (int)cudaErrorInvalidValue) return fail(B2_ERR_CAPACITY, "b2_tvlqr: nx, nu too large for the shared-memory workspace of one SM");
+  return rc ? cuda_fail((cudaError_t)rc, "b2_tvlqr launch") : B2_OK;
 }
 
 struct b2_recorder {

@@ -357,3 +357,294 @@ __global__ void __launch_bounds__(64) k_dare_small(const T* __restrict__ Ag, con
 }
 
 }  // namespace b2
+
+namespace b2 {
+
+// ---- Finite-horizon time-varying LQR / the backward pass of iLQR (b2_tvlqr, see include/b2mj.h for the recursion).
+// A (nsteps, nx, nx, N), B (nsteps, nx, nu, N), q (nsteps+1, nx, N), r (nsteps, nu, N), K (nsteps, nu, nx, N),
+// k (nsteps, nu, N), P0 (nx, nx, N), dV (2, N): env fastest.  W: Q (nx x nx), R (nu x nu), Qf (nx x nx), row-major, shared
+// by all envs.  q, r, k, P0, dV and status may be null.  A step whose Quu + reg I is not positive definite gets NaN gains;
+// they make P, and so every earlier step, NaN as well, so only the first failure (the largest t) is recorded.
+
+// Thread per env for the sizes k_dare_small covers: every matrix in registers, nu <= 2 (closed-form Cholesky).
+template <typename T, int NX, int NU>
+__global__ void __launch_bounds__(64) k_tvlqr_small(const T* __restrict__ Ag, const T* __restrict__ Bg, const T* __restrict__ W,
+                                                    const T* __restrict__ qg, const T* __restrict__ rg, int nsteps, int N, T reg, T* Kg,
+                                                    T* kg, T* P0g, T* dVg, int* status) {
+  static_assert(NU == 1 || NU == 2, "closed-form Cholesky");
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  constexpr int NN = NX * NX;
+  const T *Q = W, *R = W + NN, *Qf = W + NN + NU * NU;
+  const T nan = T(__int_as_float(0x7fc00000));
+  T P[NN], s[NX];
+#pragma unroll
+  for (int k = 0; k < NN; k++) P[k] = Qf[k];
+#pragma unroll
+  for (int i = 0; i < NX; i++) s[i] = qg ? qg[((size_t)nsteps * NX + i) * N + e] : T(0);
+  T dv0 = 0, dv1 = 0;
+  int failed = 0;
+#pragma unroll 1
+  for (int t = nsteps - 1; t >= 0; t--) {
+    T A[NN], B[NX * NU], PA[NN], PB[NX * NU];
+#pragma unroll
+    for (int k = 0; k < NN; k++) A[k] = Ag[((size_t)t * NN + k) * N + e];
+#pragma unroll
+    for (int k = 0; k < NX * NU; k++) B[k] = Bg[((size_t)t * NX * NU + k) * N + e];
+    small_mul<T, NX>(PA, P, A);
+#pragma unroll
+    for (int i = 0; i < NX; i++)
+#pragma unroll
+      for (int a = 0; a < NU; a++) { T v = 0;
+#pragma unroll
+        for (int j = 0; j < NX; j++) v += P[i * NX + j] * B[j * NU + a];
+        PB[i * NU + a] = v; }
+    T Qx[NX], Qu[NU], Quu[NU * NU], Qux[NU * NX];
+#pragma unroll
+    for (int i = 0; i < NX; i++) { T v = qg ? qg[((size_t)t * NX + i) * N + e] : T(0);
+#pragma unroll
+      for (int j = 0; j < NX; j++) v += A[j * NX + i] * s[j];
+      Qx[i] = v; }
+#pragma unroll
+    for (int a = 0; a < NU; a++) {
+      T v = rg ? rg[((size_t)t * NU + a) * N + e] : T(0);
+#pragma unroll
+      for (int j = 0; j < NX; j++) v += B[j * NU + a] * s[j];
+      Qu[a] = v;
+#pragma unroll
+      for (int b = 0; b < NU; b++) { T w = R[a * NU + b];
+#pragma unroll
+        for (int j = 0; j < NX; j++) w += B[j * NU + a] * PB[j * NU + b];
+        Quu[a * NU + b] = w; }
+#pragma unroll
+      for (int i = 0; i < NX; i++) { T w = 0;
+#pragma unroll
+        for (int j = 0; j < NX; j++) w += B[j * NU + a] * PA[j * NX + i];
+        Qux[a * NX + i] = w; }
+    }
+    small_mul_tn<T, NX>(P, A, PA);  // P <- Qxx = Q + A'PA
+#pragma unroll
+    for (int k = 0; k < NN; k++) P[k] += Q[k];
+    // K = (Quu + reg I)^-1 Qux, k = -(Quu + reg I)^-1 Qu by the Cholesky factor L L' of Quu + reg I (lower triangle)
+    T K[NU * NX], kk[NU];
+    bool ok;
+    if constexpr (NU == 1) {
+      const T d = Quu[0] + reg;
+      ok = d > T(0);
+      const T inv = T(1) / d;
+#pragma unroll
+      for (int i = 0; i < NX; i++) K[i] = inv * Qux[i];
+      kk[0] = -inv * Qu[0];
+    } else {
+      const T l11 = sqrt(Quu[0] + reg), l21 = Quu[2] / l11, d2 = Quu[3] + reg - l21 * l21, l22 = sqrt(d2);
+      ok = Quu[0] + reg > T(0) && d2 > T(0);
+      auto solve = [&](T y1, T y2, T& x1, T& x2) {
+        const T z1 = y1 / l11, z2 = (y2 - l21 * z1) / l22;
+        x2 = z2 / l22; x1 = (z1 - l21 * x2) / l11;
+      };
+#pragma unroll
+      for (int i = 0; i < NX; i++) solve(Qux[i], Qux[NX + i], K[i], K[NX + i]);
+      solve(-Qu[0], -Qu[1], kk[0], kk[1]);
+    }
+    if (!ok) {
+      if (!failed) failed = t + 1;
+#pragma unroll
+      for (int k = 0; k < NU * NX; k++) K[k] = nan;
+#pragma unroll
+      for (int a = 0; a < NU; a++) kk[a] = nan;
+    }
+    // P <- Qxx + K'(Quu K - Qux) - Qux'K (symmetrised);  s <- Qx - K'(Qu + Quu k) + Qux'k
+    T M[NU * NX], w[NU];
+#pragma unroll
+    for (int a = 0; a < NU; a++) {
+      T v = Qu[a];
+#pragma unroll
+      for (int b = 0; b < NU; b++) v += Quu[a * NU + b] * kk[b];
+      w[a] = v;
+      dv0 += kk[a] * Qu[a];
+      dv1 += T(0.5) * kk[a] * (v - Qu[a]);
+#pragma unroll
+      for (int i = 0; i < NX; i++) { T m = -Qux[a * NX + i];
+#pragma unroll
+        for (int b = 0; b < NU; b++) m += Quu[a * NU + b] * K[b * NX + i];
+        M[a * NX + i] = m; }
+    }
+    T Pn[NN];
+#pragma unroll
+    for (int i = 0; i < NX; i++) {
+#pragma unroll
+      for (int j = 0; j < NX; j++) { T v = P[i * NX + j];
+#pragma unroll
+        for (int a = 0; a < NU; a++) v += K[a * NX + i] * M[a * NX + j] - Qux[a * NX + i] * K[a * NX + j];
+        Pn[i * NX + j] = v; }
+      T v = Qx[i];
+#pragma unroll
+      for (int a = 0; a < NU; a++) v += Qux[a * NX + i] * kk[a] - K[a * NX + i] * w[a];
+      s[i] = v;
+    }
+#pragma unroll
+    for (int i = 0; i < NX; i++)
+#pragma unroll
+      for (int j = 0; j < NX; j++) P[i * NX + j] = T(0.5) * (Pn[i * NX + j] + Pn[j * NX + i]);
+#pragma unroll
+    for (int k = 0; k < NU * NX; k++) Kg[((size_t)t * NU * NX + k) * N + e] = K[k];
+    if (kg) {
+#pragma unroll
+      for (int a = 0; a < NU; a++) kg[((size_t)t * NU + a) * N + e] = kk[a];
+    }
+  }
+  if (P0g) {
+#pragma unroll
+    for (int k = 0; k < NN; k++) P0g[(size_t)k * N + e] = P[k];
+  }
+  if (dVg) { dVg[e] = dv0; dVg[(size_t)N + e] = dv1; }
+  if (status) status[e] = -failed;
+}
+
+// shared-memory reals one env of k_tvlqr needs: P, A, a scratch nx x nx; B, P B (later Quu K - Qux), Qux, K; Quu and its
+// Cholesky factor; s, Qx; Qu, k, Qu + Quu k
+__host__ __device__ inline size_t tvlqr_ws_reals(int nx, int nu) {
+  return ((size_t)3 * nx * nx + (size_t)4 * nx * nu + (size_t)2 * nu * nu + 2 * (size_t)nx + 3 * (size_t)nu + 1) & ~(size_t)1;
+}
+
+// Warp per env, the env's matrices in shared memory; wpb (= blockDim.x / 32) consecutive envs per block.  The block stages
+// A_t, B_t, q_t and r_t of its envs together, env fastest, so that a load of one matrix element of wpb envs uses whole
+// 32-byte sectors (FP64, wpb = 4) where a warp loading its own env alone would use a quarter of each.
+template <typename T>
+__global__ void __launch_bounds__(128) k_tvlqr(const T* __restrict__ Ag, const T* __restrict__ Bg, const T* __restrict__ W,
+                                               const T* __restrict__ qg, const T* __restrict__ rg, int nsteps, int nx, int nu, int N, T reg,
+                                               T* Kg, T* kg, T* P0g, T* dVg, int* status) {
+  extern __shared__ double b2_tvlqr_smem[];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+  const int e0 = blockIdx.x * wpb, e = e0 + wib;
+  const bool active = e < N;
+  const int nn = nx * nx, xu = nx * nu, uu = nu * nu;
+  const size_t per = tvlqr_ws_reals(nx, nu);
+  T* ws = reinterpret_cast<T*>(b2_tvlqr_smem) + (size_t)wib * per;
+  T *P = ws, *A = P + nn, *S = A + nn, *Bm = S + nn, *PB = Bm + xu, *Qux = PB + xu, *K = Qux + xu, *Quu = K + xu, *L = Quu + uu,
+    *s = L + uu, *Qx = s + nx, *Qu = Qx + nx, *kk = Qu + nu, *w = kk + nu;
+  const T *Q = W, *R = W + nn, *Qf = W + nn + uu;
+  const T nan = T(__int_as_float(0x7fc00000));
+  // q_t and r_t are staged into Qx and Qu
+  auto stage = [&](const T* src, int off, int count) {
+    T* base = reinterpret_cast<T*>(b2_tvlqr_smem);
+    for (int idx = threadIdx.x; idx < count * wpb; idx += blockDim.x) {
+      const int j = idx % wpb, k = idx / wpb;
+      if (e0 + j < N) base[(size_t)j * per + off + k] = src ? src[(size_t)k * N + e0 + j] : T(0);
+    }
+  };
+  stage(qg ? qg + (size_t)nsteps * nx * N : nullptr, (int)(s - ws), nx);
+  for (int k = lane; k < nn; k += 32) P[k] = Qf[k];
+  T dv0 = 0, dv1 = 0;
+  int failed = 0;
+  for (int t = nsteps - 1; t >= 0; t--) {
+    __syncthreads();  // every warp is done with the previous step's A, B, Qx, Qu
+    stage(Ag + (size_t)t * nn * N, (int)(A - ws), nn);
+    stage(Bg + (size_t)t * xu * N, (int)(Bm - ws), xu);
+    stage(qg ? qg + (size_t)t * nx * N : nullptr, (int)(Qx - ws), nx);
+    stage(rg ? rg + (size_t)t * nu * N : nullptr, (int)(Qu - ws), nu);
+    __syncthreads();
+    if (!active) continue;
+    dare_matmul(S, P, false, A, false, nx, lane);  // S = P A
+    for (int x = lane; x < xu; x += 32) {  // PB = P B
+      const int i = x / nu, a = x - i * nu;
+      T v = 0;
+      for (int j = 0; j < nx; j++) v += P[i * nx + j] * Bm[j * nu + a];
+      PB[x] = v;
+    }
+    __syncwarp();
+    for (int x = lane; x < xu; x += 32) {  // Qux = B'PA
+      const int a = x / nx, i = x - a * nx;
+      T v = 0;
+      for (int j = 0; j < nx; j++) v += Bm[j * nu + a] * S[j * nx + i];
+      Qux[x] = v;
+    }
+    for (int x = lane; x < uu; x += 32) {  // Quu = R + B'PB
+      const int a = x / nu, b = x - a * nu;
+      T v = R[x];
+      for (int j = 0; j < nx; j++) v += Bm[j * nu + a] * PB[j * nu + b];
+      Quu[x] = v;
+    }
+    for (int i = lane; i < nx + nu; i += 32) {  // Qx = q + A's, Qu = r + B's
+      T v = 0;
+      if (i < nx) { for (int j = 0; j < nx; j++) v += A[j * nx + i] * s[j]; Qx[i] += v; }
+      else { const int a = i - nx; for (int j = 0; j < nx; j++) v += Bm[j * nu + a] * s[j]; Qu[a] += v; }
+    }
+    for (int x = lane; x < nn; x += 32) {  // P <- Qxx = Q + A'PA
+      const int i = x / nx, j = x - i * nx;
+      T v = Q[x];
+      for (int q = 0; q < nx; q++) v += A[q * nx + i] * S[q * nx + j];
+      P[x] = v;
+    }
+    __syncwarp();
+    // Cholesky L L' = Quu + reg I, column by column (lower triangle)
+    bool ok = true;
+    for (int c = 0; c < nu; c++) {
+      T d = Quu[c * nu + c] + reg;
+      for (int k = 0; k < c; k++) d -= L[c * nu + k] * L[c * nu + k];
+      ok = ok && d > T(0);
+      const T lcc = sqrt(d);
+      for (int i = c + 1 + lane; i < nu; i += 32) {
+        T v = Quu[i * nu + c];
+        for (int k = 0; k < c; k++) v -= L[i * nu + k] * L[c * nu + k];
+        L[i * nu + c] = v / lcc;
+      }
+      if (lane == 0) L[c * nu + c] = lcc;
+      __syncwarp();
+    }
+    // K = L'^-1 L^-1 Qux and k = -L'^-1 L^-1 Qu: one right-hand side per lane, solved in place
+    for (int c = lane; c <= nx; c += 32) {
+      T* y = c < nx ? K + c : kk;
+      const int ys = c < nx ? nx : 1;
+      for (int a = 0; a < nu; a++) {
+        T v = c < nx ? Qux[a * nx + c] : -Qu[a];
+        for (int b = 0; b < a; b++) v -= L[a * nu + b] * y[b * ys];
+        y[a * ys] = ok ? v / L[a * nu + a] : nan;
+      }
+      for (int a = nu - 1; a >= 0; a--) {
+        T v = y[a * ys];
+        for (int b = a + 1; b < nu; b++) v -= L[b * nu + a] * y[b * ys];
+        y[a * ys] = ok ? v / L[a * nu + a] : nan;
+      }
+    }
+    if (!ok && !failed) failed = t + 1;
+    __syncwarp();
+    for (int x = lane; x < xu; x += 32) {  // PB <- Quu K - Qux
+      const int a = x / nx, i = x - a * nx;
+      T v = -Qux[x];
+      for (int b = 0; b < nu; b++) v += Quu[a * nu + b] * K[b * nx + i];
+      PB[x] = v;
+    }
+    for (int a = lane; a < nu; a += 32) {  // w = Qu + Quu k
+      T v = Qu[a];
+      for (int b = 0; b < nu; b++) v += Quu[a * nu + b] * kk[b];
+      w[a] = v;
+    }
+    __syncwarp();
+    for (int x = lane; x < nn; x += 32) {  // S = Qxx + K'(Quu K - Qux) - Qux'K
+      const int i = x / nx, j = x - i * nx;
+      T v = P[x];
+      for (int a = 0; a < nu; a++) v += K[a * nx + i] * PB[a * nx + j] - Qux[a * nx + i] * K[a * nx + j];
+      S[x] = v;
+    }
+    for (int i = lane; i < nx; i += 32) {  // s = Qx - K'w + Qux'k
+      T v = Qx[i];
+      for (int a = 0; a < nu; a++) v += Qux[a * nx + i] * kk[a] - K[a * nx + i] * w[a];
+      s[i] = v;
+    }
+    for (int a = 0; a < nu; a++) { dv0 += kk[a] * Qu[a]; dv1 += T(0.5) * kk[a] * (w[a] - Qu[a]); }
+    for (int x = lane; x < xu; x += 32) Kg[((size_t)t * xu + x) * N + e] = K[x];
+    if (kg) for (int a = lane; a < nu; a += 32) kg[((size_t)t * nu + a) * N + e] = kk[a];
+    __syncwarp();
+    for (int x = lane; x < nn; x += 32) { const int i = x / nx, j = x - i * nx; P[x] = T(0.5) * (S[x] + S[j * nx + i]); }
+    __syncwarp();
+  }
+  if (!active) return;
+  if (P0g) for (int x = lane; x < nn; x += 32) P0g[(size_t)x * N + e] = P[x];
+  if (lane == 0) {
+    if (dVg) { dVg[e] = dv0; dVg[(size_t)N + e] = dv1; }
+    if (status) status[e] = -failed;
+  }
+}
+
+}  // namespace b2

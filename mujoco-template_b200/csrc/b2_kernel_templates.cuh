@@ -832,4 +832,131 @@ auto launch_linearize_rollout(const void* image, const b2_state* st, int N, int 
   return (int)cudaGetLastError();
 }
 
+
+// u = clip(ubar + alpha k - K [q (-) qbar ; v - vbar], ctrlrange) for one env whose state is in registers: the
+// time-varying law of b2_rollout_feedback.  (-) is mj_differentiatePos(qbar -> q), as in lqr_law.  ubar (nu, N), qbar
+// (nq, N), vbar (nv, N), K (nu, 2nv, N) and k (nu, N; may be null) are one step's rows, env fastest.
+template <typename T, class D, class M>
+B2_DEV void tvlqr_law(const LaneEnv<T, D, M>& env, const T* q, const T* v, const T* __restrict__ ubar, const T* __restrict__ qbar,
+                      const T* __restrict__ vbar, const T* __restrict__ K, const T* __restrict__ k, T alpha, int N, int e, T* u_out) {
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu();
+  T qr[D::NQ], x[2 * D::NV];
+  B2_UNROLL
+  for (int i = 0; i < nq; i++) qr[i] = qbar[(size_t)i * N + e];
+  env.differentiate_pos(x, T(1), qr, q);
+  B2_UNROLL
+  for (int i = 0; i < nv; i++) x[nv + i] = v[i] - vbar[(size_t)i * N + e];
+  B2_UNROLL
+  for (int a = 0; a < nu; a++) {
+    T u = ubar[(size_t)a * N + e];
+    if (k) u += alpha * k[(size_t)a * N + e];
+    B2_UNROLL
+    for (int j = 0; j < 2 * nv; j++) u -= K[((size_t)a * 2 * nv + j) * N + e] * x[j];
+    if (M::actuator_ctrllimited(a)) u = tclip(u, M::actuator_ctrlrange(2 * a), M::actuator_ctrlrange(2 * a + 1));
+    u_out[a] = u;
+  }
+}
+
+// Closed-loop rollout (b2_rollout_feedback): for s = 0 .. nsteps-1, ctrl <- tvlqr_law at step s's rows of the nominal
+// trajectory and gains, one mj_step, record -- k_rollout's step loop with the law in front of each step.  ctrl_nom
+// (nsteps, nu, N), qpos_nom / qvel_nom (>= nsteps rows of nq / nv), K (nsteps, nu, 2nv, N), k (nsteps, nu, N) or null,
+// alpha (N) or null (1); ctrl_traj (nsteps, nu, N) records the applied controls, the other trajectories as in k_rollout.
+// A diverged env is frozen as in k_rollout; its remaining control rows are NaN, and state.ctrl keeps the last control it
+// was given.  A kernel of its own, so k_rollout stays as it is.
+template <typename T, class D, class M>
+__global__ void __launch_bounds__(128, 1) k_rollout_feedback(StateDev<T> st, DerivedDev<T> out, int want_derived, int N, int nsteps,
+                                                             const T* __restrict__ ctrl_nom, const T* __restrict__ qpos_nom,
+                                                             const T* __restrict__ qvel_nom, const T* __restrict__ K, const T* __restrict__ k,
+                                                             const T* __restrict__ alpha, T* ctrl_traj, T* qpos_traj, T* qvel_traj,
+                                                             T* sensor_traj, const void* image = nullptr) {
+  model_load<M>(image, 0);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  RowStore<T, D> rows;
+  LaneEnv<T, D, M> env(rows);
+  constexpr bool kLate = LaneEnv<T, D, M>::kLateMass;
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu(), nsd = M::nsensor() > 0 ? M::nsensordata() : 0;
+  load_state(env, st, N, e);
+  const T a = alpha ? alpha[e] : T(1);
+  int s = 0;
+  B2_NOUNROLL
+  for (; s < nsteps; s++) {
+    env.check_state();
+    if (env.flags & 3) break;
+    tvlqr_law(env, env.qpos, env.qvel, ctrl_nom + (size_t)s * nu * N, qpos_nom + (size_t)s * nq * N, qvel_nom + (size_t)s * nv * N,
+              K + (size_t)s * nu * 2 * nv * N, k ? k + (size_t)s * nu * N : nullptr, a, N, e, env.ctrl);
+    if (ctrl_traj) { B2_UNROLL for (int i = 0; i < nu; i++) ctrl_traj[((size_t)s * nu + i) * N + e] = env.ctrl[i]; }
+    env.template forward_position<kLate>();
+    env.forward_velocity();
+    env.template forward_acc<kLate>();
+    B2_UNROLL
+    for (int i = 0; i < nv; i++) if (!(fabs(env.qacc[i]) <= T(1e10))) env.flags |= 4;
+    if (sensor_traj && nsd > 0) {
+      T sd[D::NSD];
+      env.sensors(sd);
+      B2_UNROLL
+      for (int i = 0; i < nsd; i++) sensor_traj[((size_t)s * nsd + i) * N + e] = sd[i];
+    }
+    if (want_derived && s == nsteps - 1) store_derived(env, out, N, e);
+    if (M::integrator() == 1) env.rk4(); else env.euler();
+    if (qpos_traj) { B2_UNROLL for (int i = 0; i < nq; i++) qpos_traj[((size_t)s * nq + i) * N + e] = env.qpos[i]; }
+    if (qvel_traj) { B2_UNROLL for (int i = 0; i < nv; i++) qvel_traj[((size_t)s * nv + i) * N + e] = env.qvel[i]; }
+  }
+  // frozen at step s (s == nsteps when the env never diverged)
+  const T nan = T(__int_as_float(0x7fc00000));
+  B2_NOUNROLL
+  for (int r = s; r < nsteps; r++) {
+    if (qpos_traj) { B2_UNROLL for (int i = 0; i < nq; i++) qpos_traj[((size_t)r * nq + i) * N + e] = env.qpos[i]; }
+    if (qvel_traj) { B2_UNROLL for (int i = 0; i < nv; i++) qvel_traj[((size_t)r * nv + i) * N + e] = env.qvel[i]; }
+    if (sensor_traj && nsd > 0) { B2_UNROLL for (int i = 0; i < nsd; i++) sensor_traj[((size_t)r * nsd + i) * N + e] = nan; }
+    if (ctrl_traj) { B2_UNROLL for (int i = 0; i < nu; i++) ctrl_traj[((size_t)r * nu + i) * N + e] = nan; }
+  }
+  B2_UNROLL
+  for (int i = 0; i < nq; i++) st.qpos[(size_t)i * N + e] = env.qpos[i];
+  B2_UNROLL
+  for (int i = 0; i < nv; i++) st.qvel[(size_t)i * N + e] = env.qvel[i];
+  if (st.warm) { B2_UNROLL for (int i = 0; i < nv; i++) st.warm[(size_t)i * N + e] = env.warm[i]; }
+  B2_UNROLL
+  for (int i = 0; i < nu; i++) st.ctrl[(size_t)i * N + e] = env.ctrl[i];
+  if (st.flags && env.flags) st.flags[e] |= env.flags;
+}
+template <typename T, class D, class M>
+auto launch_rollout_feedback(const void* image, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_nom,
+                             const void* qpos_nom, const void* qvel_nom, const void* K, const void* k, const void* alpha, void* ctrl_traj,
+                             void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {
+  const int threads = 128, blocks = (N + threads - 1) / threads;
+  k_rollout_feedback<T, D, M><<<blocks, threads, 0, (cudaStream_t)stream>>>(
+      to_dev<T>(st), to_dev<T>(out), out != nullptr, N, nsteps, (const T*)ctrl_nom, (const T*)qpos_nom, (const T*)qvel_nom, (const T*)K,
+      (const T*)k, (const T*)alpha, (T*)ctrl_traj, (T*)qpos_traj, (T*)qvel_traj, (T*)sensor_traj, image);
+  return (int)cudaGetLastError();
+}
+
+// One step's law of b2_rollout_feedback on its own (the warp engine runs the loop on the host: this launch, one warp
+// step, row copies): state.ctrl <- tvlqr_law, also written to ctrl_row (nu, N) when given.  An env whose state fails
+// mj_checkPos / mj_checkVel is the one the step freezes: its ctrl is left alone and its ctrl_row is NaN.
+template <typename T, class D, class M>
+__global__ void __launch_bounds__(128) k_tvlqr_law(StateDev<T> st, int N, const T* __restrict__ ubar, const T* __restrict__ qbar,
+                                                   const T* __restrict__ vbar, const T* __restrict__ K, const T* __restrict__ k,
+                                                   const T* __restrict__ alpha, T* ctrl_row, const void* image = nullptr) {
+  model_load<M>(image, 0);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  RowStore<T, D> rows;
+  LaneEnv<T, D, M> env(rows);
+  const int nu = M::nu();
+  for (int i = 0; i < M::nq(); i++) env.qpos[i] = st.qpos[(size_t)i * N + e];
+  for (int i = 0; i < M::nv(); i++) env.qvel[i] = st.qvel[(size_t)i * N + e];
+  env.check_state();
+  if (env.flags & 3) {
+    if (ctrl_row) for (int i = 0; i < nu; i++) ctrl_row[(size_t)i * N + e] = T(__int_as_float(0x7fc00000));
+    return;
+  }
+  T u[D::NU];
+  tvlqr_law(env, env.qpos, env.qvel, ubar, qbar, vbar, K, k, alpha ? alpha[e] : T(1), N, e, u);
+  for (int i = 0; i < nu; i++) {
+    st.ctrl[(size_t)i * N + e] = u[i];
+    if (ctrl_row) ctrl_row[(size_t)i * N + e] = u[i];
+  }
+}
+
 }  // namespace b2

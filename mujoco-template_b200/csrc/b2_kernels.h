@@ -35,6 +35,10 @@ struct LaneKernels {
   int (*linearize_rollout)(const void* image, int cls, const b2_state* st, int N, int ntask, int nsteps, const void* ctrl_seq, double eps,
                            int centered, void* A, void* B, void* dsdx, void* dsdu, void* qpos_traj, void* qvel_traj, void* warm_traj,
                            void* sensor_traj, void* stream);
+  // b2_rollout_feedback: the time-varying LQR law in front of every step of a rollout, in one launch (k_rollout_feedback)
+  int (*rollout_feedback)(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_nom,
+                          const void* qpos_nom, const void* qvel_nom, const void* K, const void* k, const void* alpha, void* ctrl_traj,
+                          void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream);
 };
 
 // The generic kernels of one precision (b2_kernels_impl.cuh).
@@ -67,6 +71,13 @@ struct Kernels {
                    void* counter, void* sortbuf, int wpb, int blocks, const b2_state* park, void* stream);
   int (*warp_linearize)(const void* image, const b2m_view* v, const b2_state* st, int N, double eps, int centered, void* A, void* B,
                         void* jscratch, void* counter, int wpb, int blocks, void* stream);
+  // b2_tvlqr (model-independent): W = Q, R, Qf on the device; returns cudaErrorInvalidValue when one env's workspace does not
+  // fit the shared memory of an SM
+  int (*tvlqr)(const void* A, const void* B, const void* W, const void* q, const void* r, int nsteps, int nx, int nu, int N, double reg,
+               void* K, void* k, void* P0, void* dV, int* status, void* stream);
+  // one step's law of b2_rollout_feedback on the lane engine's model image (the warp engine's loop): pointers at step t's rows
+  int (*tvlqr_law)(const void* image, int cls, const b2_state* st, int N, const void* ubar, const void* qbar, const void* vbar,
+                   const void* K, const void* k, const void* alpha, void* ctrl_row, void* stream);
 };
 extern const Kernels kernels_f64, kernels_f32;
 

@@ -332,14 +332,58 @@ static int b2k_linearize_rollout(const void* image, int cls, const b2_state* st,
                                                                                      dsdx, dsdu, qpos_traj, qvel_traj, warm_traj, sensor_traj, stream)))
   return rc;
 }
+static int b2k_rollout_feedback(const void* image, int cls, const b2_state* st, const b2_derived* out, int N, int nsteps, const void* ctrl_nom,
+                                const void* qpos_nom, const void* qvel_nom, const void* K, const void* k, const void* alpha, void* ctrl_traj,
+                                void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {
+  int rc = 0;
+  B2_DISPATCH(cls, (rc = launch_rollout_feedback<real, DD, RuntimeModel<DD>>(image, st, out, N, nsteps, ctrl_nom, qpos_nom, qvel_nom, K, k,
+                                                                            alpha, ctrl_traj, qpos_traj, qvel_traj, sensor_traj, stream)));
+  return rc;
+}
+static int b2k_tvlqr_law(const void* image, int cls, const b2_state* st, int N, const void* ubar, const void* qbar, const void* vbar,
+                         const void* K, const void* k, const void* alpha, void* ctrl_row, void* stream) {
+  const int threads = 128, blocks = (N + threads - 1) / threads;
+  B2_DISPATCH(cls, (k_tvlqr_law<real, DD, RuntimeModel<DD>><<<blocks, threads, 0, (cudaStream_t)stream>>>(
+                       to_dev<real>(st), N, (const real*)ubar, (const real*)qbar, (const real*)vbar, (const real*)K, (const real*)k,
+                       (const real*)alpha, (real*)ctrl_row, image)));
+  return (int)cudaGetLastError();
+}
+// b2_tvlqr: a thread per env (compile-time sizes, registers) for the sizes k_dare_small covers, otherwise a warp per env
+// with its matrices in shared memory, as many warps (consecutive envs) per block as fit, at most four
+static int b2k_tvlqr(const void* A, const void* B, const void* W, const void* q, const void* r, int nsteps, int nx, int nu, int N, double reg,
+                     void* K, void* k, void* P0, void* dV, int* status, void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+#define B2_TVLQR_SMALL(NX_, NU_)                                                                                                      \
+  if (nx == NX_ && nu == NU_) {                                                                                                       \
+    k_tvlqr_small<real, NX_, NU_><<<(N + 63) / 64, 64, 0, s>>>((const real*)A, (const real*)B, (const real*)W, (const real*)q,        \
+                                                               (const real*)r, nsteps, N, (real)reg, (real*)K, (real*)k, (real*)P0,  \
+                                                               (real*)dV, status);                                                    \
+    return (int)cudaGetLastError();                                                                                                   \
+  }
+  B2_TVLQR_SMALL(2, 1) B2_TVLQR_SMALL(4, 1) B2_TVLQR_SMALL(4, 2)
+#undef B2_TVLQR_SMALL
+  int dev = 0, smem_max = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  const size_t per = tvlqr_ws_reals(nx, nu) * sizeof(real);
+  int wpb = (int)((size_t)smem_max / per);
+  if (wpb < 1) return (int)cudaErrorInvalidValue;
+  if (wpb > 4) wpb = 4;
+  cudaError_t e = cudaFuncSetAttribute(k_tvlqr<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(per * wpb));
+  if (e != cudaSuccess) return (int)e;
+  k_tvlqr<real><<<(N + wpb - 1) / wpb, wpb * 32, per * wpb, s>>>((const real*)A, (const real*)B, (const real*)W, (const real*)q, (const real*)r,
+                                                                 nsteps, nx, nu, N, (real)reg, (real*)K, (real*)k, (real*)P0, (real*)dV, status);
+  return (int)cudaGetLastError();
+}
 
 // in the member order of Kernels (b2_kernels.h)
 const Kernels B2_FN(kernels) = {
-    {b2k_step, b2k_linearize, b2k_linearize_sensors, b2k_jacobian, b2k_rollout, b2k_linearize_rollout},
+    {b2k_step, b2k_linearize, b2k_linearize_sensors, b2k_jacobian, b2k_rollout, b2k_linearize_rollout, b2k_rollout_feedback},
     b2k_inverse, b2k_lqr_control, b2k_lqr_control_env, b2k_integrate_pos, b2k_differentiate_pos,
     b2k_commit_state, b2k_random_controls, b2k_record_rows, b2k_dare, b2k_fma_peak,
     b2k_image_bytes, b2k_image_fill,
     b2k_warp_plan, b2k_warp_scratch_bytes, b2k_warp_image_bytes, b2k_warp_image_fill, b2k_warp_sort_bytes, b2k_warp_step, b2k_warp_linearize,
+    b2k_tvlqr, b2k_tvlqr_law,
 };
 
 }  // namespace b2

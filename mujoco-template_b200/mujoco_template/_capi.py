@@ -27,6 +27,7 @@ EXPORTED_SYMBOLS = (
     "b2_differentiate_pos", "b2_inverse", "b2_lqr_set_gain", "b2_lqr_control", "b2_control_tick", "b2_refresh_derived", "b2_step_lazy", "b2_step_host", "b2_step_host_wait", "b2_stream_synchronize", "b2_launch_count",
     "b2_batch_size_class", "b2_last_error", "b2_version", "b2_fp_peak", "b2_batch_kernel_variant",
     "b2_recorder_create", "b2_recorder_record", "b2_recorder_destroy", "b2_dlqr", "b2_random_controls", "b2_warp_queue_histogram", "b2_lqr_control_env",
+    "b2_tvlqr", "b2_rollout_feedback",
 )
 
 
@@ -98,6 +99,8 @@ def lib() -> C.CDLL:
     L.b2_warp_queue_histogram.argtypes = [vp, C.POINTER(C.c_int), vp]
     L.b2_dlqr.argtypes = [C.c_int, C.c_int, vp, vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.c_int,
                           C.c_double, vp, vp, vp, vp]
+    L.b2_tvlqr.argtypes = [i, i, i, i, i, i, vp, vp, C.POINTER(d), C.POINTER(d), C.POINTER(d), vp, vp, d, vp, vp, vp, vp, vp, vp]
+    L.b2_rollout_feedback.argtypes = [vp, C.POINTER(State), i, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(Derived), vp]
     L.b2_recorder_create.argtypes = [vp, C.POINTER(RecordCol), C.c_int, C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]
     L.b2_recorder_record.argtypes = [vp, C.c_double, vp, vp]
     L.b2_recorder_destroy.argtypes = [vp]
@@ -173,6 +176,14 @@ class NativeBatch:
         controls), recording the state (and sensordata) after every step into the (nsteps, dim, nenv) trajectory arrays."""
         check(self._L.b2_rollout(self.handle, C.byref(state), int(nsteps), ctrl_seq, qpos_traj, qvel_traj, sensor_traj,
                                  C.byref(derived) if derived is not None else None, stream))
+
+    def rollout_feedback(self, state: State, nsteps: int, ctrl_nom: int, qpos_nom: int, qvel_nom: int, K: int, k: int | None,
+                         alpha: int | None, ctrl_traj: int | None, qpos_traj: int | None, qvel_traj: int | None, sensor_traj: int | None,
+                         derived: Derived | None, stream: int = 0) -> None:
+        """``b2_rollout_feedback``: ``nsteps`` steps under ``u = clip(ctrl_nom[t] + alpha k[t] - K[t] [q (-) qpos_nom[t] ;
+        v - qvel_nom[t]])``, recording the applied controls and the state (and sensordata) after every step."""
+        check(self._L.b2_rollout_feedback(self.handle, C.byref(state), int(nsteps), ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, ctrl_traj,
+                                          qpos_traj, qvel_traj, sensor_traj, C.byref(derived) if derived is not None else None, stream))
 
     def forward(self, state: State, derived: Derived | None, stream: int = 0) -> None:
         check(self._L.b2_forward(self.handle, C.byref(state), C.byref(derived) if derived is not None else None, stream))
@@ -268,6 +279,16 @@ def dlqr(device: int, precision: int, A_ptr: int, B_ptr: int, Q, R, nx: int, nu:
     r = (C.c_double * (nu * nu))(*[float(x) for x in R])
     check(lib().b2_dlqr(int(device), int(precision), A_ptr, B_ptr, q, r, int(nx), int(nu), int(nenv), int(max_doublings), float(tol),
                         K_ptr, P_ptr, status_ptr, stream))
+
+
+def tvlqr(device: int, precision: int, nsteps: int, nx: int, nu: int, nenv: int, A_ptr: int, B_ptr: int, Q, R, Qf, q_ptr: int | None,
+          r_ptr: int | None, reg: float, K_ptr: int, k_ptr: int | None, P0_ptr: int | None, dV_ptr: int | None, status_ptr: int | None,
+          stream: int = 0) -> None:
+    """``b2_tvlqr``: batched finite-horizon Riccati backward pass on the device (device pointers in the env-fastest layout;
+    Q, R, Qf host arrays)."""
+    arr = lambda x, n: (C.c_double * n)(*[float(v) for v in x])  # noqa: E731
+    check(lib().b2_tvlqr(int(device), int(precision), int(nsteps), int(nx), int(nu), int(nenv), A_ptr, B_ptr, arr(Q, nx * nx), arr(R, nu * nu),
+                         arr(Qf, nx * nx), q_ptr, r_ptr, float(reg), K_ptr, k_ptr, P0_ptr, dV_ptr, status_ptr, stream))
 
 
 class NativeRecorder:

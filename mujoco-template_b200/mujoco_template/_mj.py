@@ -317,6 +317,26 @@ class NativeBackend:
                      self.derived_struct() if derived else None)
         return bufs if out is not None else None
 
+    def rollout_feedback(self, ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, nsteps: int, record: bool, out=None, derived: bool = True):
+        """Closed-loop rollout (``b2_rollout_feedback``): ``nsteps`` steps under the time-varying LQR law
+        ``u_t = clip(ctrl_nom[t] + alpha k[t] - K[t] [q (-) qpos_nom[t] ; v - qvel_nom[t]], ctrlrange)``.  Tensors in the
+        library's layouts: ``ctrl_nom`` (nsteps, nu, nenv), ``qpos_nom`` / ``qvel_nom`` (>= nsteps, dim, nenv), ``K``
+        (nsteps, nu, 2nv, nenv), ``k`` (nsteps, nu, nenv) or None, ``alpha`` (nenv,) or None (1).  With ``record`` returns
+        (ctrl_traj, qpos_traj, qvel_traj, sensor_traj) of shapes (nsteps, nu, nenv), (nsteps, nq, nenv), (nsteps, nv, nenv)
+        and (nsteps, nsensordata, nenv) (None without sensors); fresh buffers unless ``out`` gives them."""
+        torch, m = self.torch, self.model
+        T = int(nsteps)
+        if out is None and record:
+            mk = ((lambda dim: torch.zeros((T, dim, self.nenv), dtype=self.dtype).pin_memory()) if self.host_mapped else
+                  (lambda dim: torch.empty((T, dim, self.nenv), device=f"cuda:{self.device}", dtype=self.dtype)))
+            out = (mk(m.nu), mk(m.nq), mk(m.nv), mk(m.nsensordata) if m.nsensordata else None)
+        bufs = tuple(out) if out is not None else (None, None, None, None)
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
+        self.derived_stale = False
+        self._launch("rollout_feedback", self.batch.rollout_feedback, self.state_struct(), T, ptr(ctrl_nom), ptr(qpos_nom), ptr(qvel_nom),
+                     ptr(K), ptr(k), ptr(alpha), *map(ptr, bufs), self.derived_struct() if derived else None)
+        return bufs if out is not None else None
+
     def forward(self) -> None:
         self.derived_stale = False
         self._launch("forward", self.batch.forward, self.state_struct(), self.derived_struct())

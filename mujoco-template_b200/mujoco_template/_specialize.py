@@ -184,10 +184,16 @@ def emit_spec(compiled: dict, name: str) -> str:
             A(f"  if (dsdx || dsdu) return launch_linearize_rollout<{M}, true>" + call.format("dsdx, dsdu"))
         A(f"  return launch_linearize_rollout<{M}>" + call.format("nullptr, nullptr"))
         A("}")
+    # ... and the closed-loop rollout last
+    for T, suf in (("double", ""), ("float", "32")):
+        A(f"int spec_rollout_feedback{suf}({lane}, const b2_derived* out, int N, int nsteps, const void* ctrl_nom, const void* qpos_nom, const void* qvel_nom, const void* K, const void* k, const void* alpha, void* ctrl_traj, void* qpos_traj, void* qvel_traj, void* sensor_traj, void* stream) {{")
+        A(f"  return launch_rollout_feedback<{T}, SDims, SModel<{T}>>(nullptr, st, out, N, nsteps, ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, ctrl_traj, qpos_traj, qvel_traj, sensor_traj, stream);")
+        A("}")
     lanes = []
     for suf in ("", "32"):
         sens = f"spec_linearize_sensors{suf}" if has_sensors else "nullptr"
-        lanes.append(f"{{spec_step{suf}, spec_linearize{suf}, {sens}, spec_jacobian{suf}, spec_rollout{suf}, spec_linearize_rollout{suf}}}")
+        lanes.append(f"{{spec_step{suf}, spec_linearize{suf}, {sens}, spec_jacobian{suf}, spec_rollout{suf}, spec_linearize_rollout{suf}, "
+                     f"spec_rollout_feedback{suf}}}")
     A(f'const SpecKernels kSpec = {{"{name}", 0x{fnv1a(blob):016x}ull, {len(blob)}, {{{lanes[0]}, {lanes[1]}}}}};')
     A("struct Registrar { Registrar() { register_spec(&kSpec); } } registrar;")
     A("}  // namespace")

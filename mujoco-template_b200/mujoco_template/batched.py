@@ -354,6 +354,64 @@ class BatchedEnv:
             traj["sensordata"] = out[2].permute(2, 0, 1)
         return traj
 
+    def rollout_feedback(self, controls, K, qpos, qvel, *, k=None, alpha=None, record: bool = False):
+        """``T`` steps of every env under the time-varying LQR law about a nominal trajectory, in one kernel launch (the
+        warp engine of large models: two per step).  At step t the control is
+
+            u_t = clip(controls[:, t] + alpha k[:, t] - K[:, t] [q (-) qpos[:, t] ; v - qvel[:, t]], ctrlrange)
+
+        where (-) is ``mj_differentiatePos`` (the tangent space of ``linearize_rollout``'s ``A``) and the clip applies to
+        ctrl-limited actuators.  This is the forward pass of iLQR (``linearize_rollout`` -> ``batched_tvlqr`` ->
+        ``rollout_feedback``) and time-varying LQR tracking of a nominal trajectory.  The controller is not called.
+
+        ``controls`` ``(nenv, T, nu)`` is the nominal control sequence (validated as in ``rollout``); ``K`` ``(nenv, T, nu,
+        2nv)`` and ``k`` ``(nenv, T, nu)`` (None: zero) are ``batched_tvlqr``'s gains; ``qpos`` ``(nenv, T or T+1, nq)`` and
+        ``qvel`` ``(nenv, T or T+1, nv)`` the nominal states -- ``linearize_rollout``'s ``"qpos"`` / ``"qvel"`` as they are;
+        ``alpha`` a float or an ``(nenv,)`` tensor (per-env line search; None: 1).  All on the batch's device, in its
+        dtype; views of env-fastest storage are handed over without a copy.
+
+        ``data.time`` and the step counter advance by T as in ``rollout``; ``data.ctrl`` holds the last applied control.
+        ``record=True`` returns ``rollout``'s dict plus ``"ctrl": (nenv, T, nu)``, the applied controls (NaN from the step
+        an env is frozen at).  Otherwise returns None."""
+        import torch
+
+        m, n = self.model, self.nenv
+        seq, T = self._control_sequence("rollout_feedback", controls, None)
+        if seq is None:
+            raise ConfigError("rollout_feedback: controls (the nominal control sequence) are required")
+        ref = self.data.qpos
+        nx = 2 * m.nv
+
+        def layout(name, t, shapes):
+            if not isinstance(t, torch.Tensor) or tuple(t.shape) not in shapes:
+                got = tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__
+                raise ConfigError(f"rollout_feedback: {name} must have shape {' or '.join(map(str, shapes))}, got {got}")
+            if t.device != ref.device or t.dtype != ref.dtype:
+                raise ConfigError(f"rollout_feedback: {name}: expected {ref.dtype} on {ref.device}, got {t.dtype} on {t.device}")
+            return t.permute(*range(1, t.dim()), 0).contiguous()  # env fastest; no copy for a view of such storage
+
+        Ks = layout("K", K, [(n, T, m.nu, nx)])
+        ks = None if k is None else layout("k", k, [(n, T, m.nu)])
+        qs = layout("qpos", qpos, [(n, T, m.nq), (n, T + 1, m.nq)])
+        vs = layout("qvel", qvel, [(n, T, m.nv), (n, T + 1, m.nv)])
+        if alpha is None:
+            a = None
+        elif isinstance(alpha, torch.Tensor):
+            if tuple(alpha.shape) != (n,) or alpha.device != ref.device or alpha.dtype != ref.dtype:
+                raise ConfigError(f"rollout_feedback: alpha must be a float or a ({n},) {ref.dtype} tensor on {ref.device}")
+            a = alpha.contiguous()
+        else:
+            a = torch.full((n,), float(alpha), dtype=ref.dtype, device=ref.device)
+        out = self.data.backend.rollout_feedback(seq, qs, vs, Ks, ks, a, T, record)
+        self._advance_time(T)
+        self._substep += T
+        if not record:
+            return None
+        traj = {"qpos": out[1].permute(2, 0, 1), "qvel": out[2].permute(2, 0, 1), "ctrl": out[0].permute(2, 0, 1)}
+        if out[3] is not None:
+            traj["sensordata"] = out[3].permute(2, 0, 1)
+        return traj
+
     def _control_sequence(self, what: str, controls, nsteps):
         """Validates a ``(nenv, T, nu)`` control tensor and ``nsteps``; returns the controls as a ``(T, nu, nenv)`` layout
         (None without controls) and T."""

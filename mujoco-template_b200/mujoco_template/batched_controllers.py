@@ -81,6 +81,70 @@ def batched_dlqr_gain(A, B, Q, R, max_doublings: int = 40, tol: float = 1e-13, r
     return (K, P, status) if return_status else (K, P)
 
 
+def batched_tvlqr(A, B, Q, R, Qf=None, q=None, r=None, reg: float = 0.0):
+    """Finite-horizon time-varying LQR about a trajectory for a whole batch on the device (``b2_tvlqr``): the Riccati
+    backward pass of TV-LQR and iLQR, every env from its own ``(A_t, B_t)``.
+
+    ``A`` (N, T, nx, nx) and ``B`` (N, T, nx, nu) are CUDA tensors -- ``BatchedEnv.linearize_rollout``'s ``"A"`` / ``"B"``
+    are read in place; ``Q``, ``R`` and ``Qf`` (default ``Q``) are shared host matrices; ``q`` (N, T+1, nx) and ``r``
+    (N, T, nu) optional linear cost terms; ``reg`` >= 0 is added to the diagonal of Quu before its Cholesky factorisation.
+    With ``dx = [q (-) qbar ; v - vbar]`` and ``du = u - ubar`` the cost is
+
+        J = sum_t [1/2 dx'Q dx + q_t'dx + 1/2 du'R du + r_t'du] + 1/2 dx_T'Qf dx_T + q_T'dx_T
+
+    Returns ``(K, k, P0, dV, status)``: ``K`` (N, T, nu, nx) and ``k`` (N, T, nu) with ``u_t = ubar_t + alpha k_t - K_t
+    dx_t`` (``BatchedEnv.rollout_feedback``), ``P0`` (N, nx, nx) the cost-to-go Hessian at t = 0, ``dV`` (N, 2) the
+    expected cost change ``alpha dV[:, 0] + alpha**2 dV[:, 1]`` and ``status`` (N,) int32: 0, or -(t+1) when
+    ``Quu_t + reg I`` is not positive definite (that env's rows <= t, ``P0`` and ``dV`` are NaN).  All are views of
+    env-fastest storage.  See ``include/b2mj.h`` for the recursion."""
+    import torch
+
+    from . import _capi
+    from .exceptions import TemplateError
+
+    if not isinstance(A, torch.Tensor) or not isinstance(B, torch.Tensor):
+        raise ConfigError("batched_tvlqr: A and B must be tensors")
+    if A.device.type != "cuda":
+        raise TemplateError("batched_tvlqr: A and B must be CUDA tensors (this path has no CPU fallback)")
+    if A.dtype not in (torch.float64, torch.float32):
+        raise ConfigError("batched_tvlqr: float64 or float32 tensors expected")
+    if A.dim() != 4 or B.dim() != 4:
+        raise ConfigError("batched_tvlqr: A must be (N, T, nx, nx) and B (N, T, nx, nu)")
+    n, T, nx, nu = A.shape[0], A.shape[1], A.shape[2], B.shape[3]
+    if A.shape != (n, T, nx, nx) or B.shape != (n, T, nx, nu) or min(n, T, nx, nu) < 1:
+        raise ConfigError(f"batched_tvlqr: A must be (N, T, nx, nx) and B (N, T, nx, nu), got {tuple(A.shape)} and {tuple(B.shape)}")
+
+    def env_fastest(name, t, shape):
+        if not isinstance(t, torch.Tensor) or tuple(t.shape) != shape:
+            raise ConfigError(f"batched_tvlqr: {name} must be a tensor of shape {shape}")
+        if t.device != A.device or t.dtype != A.dtype:
+            raise ConfigError(f"batched_tvlqr: {name}: expected {A.dtype} on {A.device}, got {t.dtype} on {t.device}")
+        return t.permute(*range(1, t.dim()), 0).contiguous()  # no copy for a view of env-fastest storage
+
+    def host(name, M, k):
+        M = np.asarray(M.cpu() if hasattr(M, "cpu") else M, dtype=float)
+        if M.shape != (k, k):
+            raise ConfigError(f"batched_tvlqr: {name} must be ({k}, {k}), got {M.shape}")
+        return np.ascontiguousarray(M).reshape(-1)
+
+    As, Bs = env_fastest("A", A, (n, T, nx, nx)), env_fastest("B", B, (n, T, nx, nu))
+    qs = None if q is None else env_fastest("q", q, (n, T + 1, nx))
+    rs = None if r is None else env_fastest("r", r, (n, T, nu))
+    Qh, Rh = host("Q", Q, nx), host("R", R, nu)
+    Qfh = Qh if Qf is None else host("Qf", Qf, nx)
+    if not float(reg) >= 0:
+        raise ConfigError("batched_tvlqr: reg must be >= 0")
+    mk = lambda *shape: torch.empty(shape, dtype=A.dtype, device=A.device)  # noqa: E731
+    Ks, ks, Ps, dVs = mk(T, nu, nx, n), mk(T, nu, n), mk(nx, nx, n), mk(2, n)
+    status = torch.zeros(n, dtype=torch.int32, device=A.device)
+    ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+    with torch.cuda.device(A.device):
+        _capi.tvlqr(A.device.index, 64 if A.dtype == torch.float64 else 32, T, nx, nu, n, As.data_ptr(), Bs.data_ptr(), Qh, Rh, Qfh,
+                    ptr(qs), ptr(rs), float(reg), Ks.data_ptr(), ks.data_ptr(), Ps.data_ptr(), dVs.data_ptr(), status.data_ptr(),
+                    torch.cuda.current_stream(A.device).cuda_stream)
+    return Ks.permute(3, 0, 1, 2), ks.permute(2, 0, 1), Ps.permute(2, 0, 1), dVs.permute(1, 0), status
+
+
 class BatchedLQRController:
     def __init__(self, qpos_ref: np.ndarray | None = None, ctrl_ref: np.ndarray | None = None,
                  Q: np.ndarray | None = None, R: np.ndarray | None = None, eps: float = 1e-6,
@@ -264,4 +328,4 @@ class BatchedRandomController:
         b._launch("random_controls", b.batch.random_controls, b.state_struct(), self.lo, self.hi, self.seed, row, thr, rq, rv)
 
 
-__all__ = ["BatchedLQRController", "BatchedTVLQRController", "BatchedRandomController", "batched_dlqr_gain", "dlqr_gain"]
+__all__ = ["BatchedLQRController", "BatchedTVLQRController", "BatchedRandomController", "batched_dlqr_gain", "batched_tvlqr", "dlqr_gain"]

@@ -185,12 +185,17 @@ auto launch_step(const void* image, const b2_state* st, const b2_derived* out, i
 // The nominal state of a thread's env is re-read from the SoA arrays at the start of every rollout (L1/L2 hits) rather
 // than held in registers: ~14 fewer live registers across the physics, which is what the 168-register budget of three
 // resident blocks is short of.  The controls are the exception (they may come from the control law, not from st.ctrl).
+// (The addresses are left to the compiler: the specialised cartpole kernel keeps all six in registers already, and
+// per-thread base pointers with a stride of their own raised the drone group thread's spill loads; see DESIGN.md §3.)
 template <typename T>
 struct NominalInMemory {
   static constexpr bool kSens = false;
   StateDev<T> st;
   int N, e;
   const T* u0;
+  B2_DEV void set(const T* qpos, const T* qvel, const T* warm, int n, int ee) {
+    st.qpos = (T*)qpos; st.qvel = (T*)qvel; st.warm = (T*)warm; st.ctrl = nullptr; st.flags = nullptr; N = n; e = ee;
+  }
   B2_DEV T q(int k) const { return __ldg(st.qpos + (size_t)k * N + e); }
   B2_DEV T v(int k) const { return __ldg(st.qvel + (size_t)k * N + e); }
   B2_DEV T u(int k) const { return u0[k]; }
@@ -205,7 +210,6 @@ struct NominalWithSensors : NominalInMemory<T> {
   T *dsdx, *dsdu;
   mutable T* col;      // entry (0, c, e) of the current column in dsdx / dsdu, or null
   mutable int ncol;    // columns of that array
-  mutable bool first;  // no rollout of the column has stored its reading yet
 };
 
 // One column of the FD linearisation for env e -- c < nv: tangent-space position column, c < 2nv: velocity column, else
@@ -216,7 +220,7 @@ struct NominalWithSensors : NominalInMemory<T> {
 // control columns (either may be null).
 template <typename T, class D, class M, class S>
 B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
-                      T eps, T inv_eps, int centered, int N, int e, T* A, T* B, bool& pos_valid, bool& vel_valid) {
+                      T eps, T inv_eps, int centered, int N, int e, T* A, T* B, int& last) {
   constexpr int NQ = D::NQ, NV = D::NV;
   const int nq = M::nq(), nv = M::nv(), nu = M::nu(), ndx = 2 * nv;
   T s1[NQ + NV], s2[NQ + NV], col[2 * NV];  // the two end points of the difference quotient
@@ -226,13 +230,10 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
   T dacc[2 * NV];
   B2_UNROLL
   for (int k = 0; k < 2 * nv; k++) dacc[k] = 0;
-  int kind, i;
-  bool fwd = true, back = centered != 0;
-  if (nominal) { kind = 0; i = 0; fwd = back = false; }
-  else if (c < nv) { kind = 1; i = c; }
-  else if (c < ndx) { kind = 2; i = c - nv; }
-  else {
-    kind = 3; i = c - ndx;
+  // The column, decided once: which sides of the quotient exist (ctrlrange one-sidedness as mjd_transitionFD) ...
+  bool fwd = !nominal, back = !nominal && centered != 0;
+  if (!nominal && c >= ndx) {
+    const int i = c - ndx;
     int lim = 0;
     T lo = 0, hi = 0, u = 0;
     B2_UNROLL
@@ -241,70 +242,81 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
     fwd = !lim || (u >= lo && u <= hi && u + eps >= lo && u + eps <= hi);
     back = (centered || !fwd) && (!lim || (u - eps >= lo && u - eps <= hi && u >= lo && u <= hi));
   }
-  const int need = nominal ? 4 : ((fwd ? 1 : 0) | (back ? 2 : 0) | ((fwd != back) ? 4 : 0));  // plus, minus, nominal rollouts
+  // ... and so its rollouts: the first is the plus side (minus when only that exists), the second the opposite side
+  // (centred) or the nominal step (one-sided); the env advance is one nominal rollout.  slot: the perturbed entry of
+  // [dq; v; u] (the column index itself), -1 for none.  to2 / sg: the rollout's end and sign in the quotient (plus -> s2,
+  // minus -> s1, the nominal step -> whichever end the one-sided quotient is missing).
+  const bool both = fwd && back;
+  const int nroll = nominal ? 1 : (fwd || back ? 2 : 0);
+  int slot = nominal ? -1 : c;
+  T delta = fwd ? eps : -eps;
+  // Stage skips under Euler: a rollout at the nominal qpos (velocity / control columns, the advance) reuses the position
+  // stage of the thread's previous rollout when that one also ran at the nominal qpos (last: the thread's last column
+  // with rollouts, -1 before the first), and at the nominal qvel too (control columns, the advance) its velocity stage.
+  // bit 0: skip the position stage, bit 1: the velocity stage; for this column's first rollout, then for the rest.
+  const bool euler = M::integrator() == 0;
+  const bool reuse_pos = euler && (nominal || c >= nv), reuse_vel = euler && (nominal || c >= ndx);
+  int skip = (reuse_pos && last >= nv ? 1 : 0) | (reuse_vel && last >= ndx ? 2 : 0);
+  const int skip_rest = (reuse_pos ? 1 : 0) | (reuse_vel ? 2 : 0);
+  if (nroll > 0) last = c;
   // SENS: the column's sensor entries live in the output array itself, not in registers (the group thread of the drone is
   // at the 255-register limit already).  Each (r, c, e) entry has one owning thread: its first rollout stores the reading
   // with its sign, its second adds its own and scales, so the entry is (s2 - s1) * ih -- the plain difference quotient,
   // with no tangent-space handling (framequat components included), as upstream mjd_stepFD differences sensordata.
+  const T ih = both ? T(0.5) * inv_eps : inv_eps;
   if constexpr (S::kSens) {
     nom.col = nullptr;
     if (!nominal) {
       nom.col = c < ndx ? nom.dsdx : nom.dsdu;
       nom.ncol = c < ndx ? ndx : nu;
       if (nom.col) nom.col += (size_t)(c < ndx ? c : c - ndx) * N + e;
-      nom.first = true;
     }
   }
-  // rolled phase loop: the physics is instantiated once; all array indices stay static.  pos_valid (owned by the
-  // caller) says that env already holds the position stage of the nominal qpos from an earlier rollout of this thread
+  // rolled rollout loop: the physics is instantiated once; all array indices stay static
   B2_NOUNROLL
-  for (int phase = 0; phase < 3; phase++) {
-    if (!((need >> phase) & 1)) continue;
-    const T delta = phase == 0 ? eps : (phase == 1 ? -eps : T(0));
-    B2_UNROLL
-    for (int k = 0; k < nq; k++) env.qpos[k] = nom.q(k);
-    B2_UNROLL
-    for (int k = 0; k < nv; k++) { env.qvel[k] = nom.v(k) + ((kind == 2 && k == i) ? delta : T(0)); env.warm[k] = nom.w(k); }
-    B2_UNROLL
-    for (int k = 0; k < nu; k++) env.ctrl[k] = nom.u(k) + ((kind == 3 && k == i) ? delta : T(0));
-    if (kind == 1 && phase < 2) {
-      T dp[NV];
+  for (int ro = 0; ro < nroll; ro++) {
+    // the nominal state, then the perturbation as one update of entry `slot`
+    if (scalar_only) {
       B2_UNROLL
-      for (int k = 0; k < nv; k++) dp[k] = (k == i) ? T(1) : T(0);
-      env.integrate_pos(env.qpos, dp, delta);
+      for (int k = 0; k < nq; k++) { T x = nom.q(k); if (k == slot) x += delta; env.qpos[k] = x; }
+    } else {
+      B2_UNROLL
+      for (int k = 0; k < nq; k++) env.qpos[k] = nom.q(k);
+      if ((unsigned)slot < (unsigned)nv) {
+        T dp[NV];
+        B2_UNROLL
+        for (int k = 0; k < nv; k++) dp[k] = (k == slot) ? T(1) : T(0);
+        env.integrate_pos(env.qpos, dp, delta);
+      }
     }
-    // one mj_step; the position stage is skipped when an earlier rollout of this thread already ran
-    // it at the same qpos (velocity / control columns under Euler)
-    // ... and so is the velocity stage when that rollout also ran at the nominal qvel (control columns, the advance)
-    if (!pos_valid) env.forward_position();
-    if (!(pos_valid && vel_valid && kind != 1 && kind != 2)) env.forward_velocity();
+    B2_UNROLL
+    for (int k = 0; k < nv; k++) { T x = nom.v(k); if (nv + k == slot) x += delta; env.qvel[k] = x; env.warm[k] = nom.w(k); }
+    B2_UNROLL
+    for (int k = 0; k < nu; k++) { T x = nom.u(k); if (ndx + k == slot) x += delta; env.ctrl[k] = x; }
+    // one mj_step
+    if (!(skip & 1)) env.forward_position();
+    if (!(skip & 2)) env.forward_velocity();
     env.forward_acc();
     B2_UNROLL
     for (int k = 0; k < nv; k++) if (!(fabs(env.qacc[k]) <= T(1e10))) env.flags |= 4;
+    const bool to2 = (ro == 0) == fwd;
+    const T sg = to2 ? T(1) : T(-1);
     if constexpr (S::kSens) {
       // this rollout's sensordata: its forward pass at the perturbed input state, before integration (RK4: the first stage,
-      // as mj_step leaves it).  sensors() uses spat as scratch; nothing kept across rollouts (pos_valid / vel_valid) lives
-      // there -- the velocity stage's only use of it is as bias_forces' scratch.
+      // as mj_step leaves it).  sensors() uses spat as scratch; nothing the skipped stages reuse lives there -- the
+      // velocity stage's only use of it is as bias_forces' scratch.
       if (nom.col) {
         T sd[D::NSD];
         env.sensors(sd);
-        const bool to2 = phase == 0 || (phase == 2 && !fwd);
-        const T sg = to2 ? T(1) : T(-1), ih = (fwd && back) ? T(0.5) * inv_eps : inv_eps;
         B2_UNROLL
         for (int r = 0; r < M::nsensordata(); r++) {
           T* p = nom.col + (size_t)r * nom.ncol * N;
-          *p = nom.first ? sg * sd[r] : fma(sg, sd[r], *p) * ih;
+          *p = ro == 0 ? sg * sd[r] : fma(sg, sd[r], *p) * ih;
         }
-        nom.first = false;
       }
     }
     if (M::integrator() == 1) env.rk4(); else env.euler();
-    vel_valid = kind != 1 && kind != 2 && M::integrator() == 0;  // this rollout's velocity stage was the nominal one
-    pos_valid = kind != 1 && M::integrator() == 0;
-    // plus -> s2, minus -> s1, nominal -> whichever end the one-sided quotient is missing
-    const bool to2 = phase == 0 || (phase == 2 && !fwd);
     if (scalar_only) {
-      const T sg = to2 ? T(1) : T(-1);
       B2_UNROLL
       for (int k = 0; k < 2 * nv; k++) dacc[k] = fma(sg, k < nv ? env.qpos[k < nv ? k : 0] : env.qvel[k >= nv ? k - nv : 0], dacc[k]);
     } else {
@@ -314,11 +326,14 @@ B2_DEV void fd_column(LaneEnv<T, D, M>& env, const S& nom, int c, bool nominal,
         if (to2) s2[k] = val; else s1[k] = val;
       }
     }
+    // the second rollout
+    skip = skip_rest;
+    delta = -delta;
+    if (!both) slot = -1;
   }
   if (nominal) return;
-  if (fwd || back) {
+  if (nroll > 0) {
     // difference quotient with the reciprocal step (1 / (2 eps) = 0.5 / eps exactly): no division per entry
-    const T ih = (fwd && back) ? T(0.5) * inv_eps : inv_eps;
     if (scalar_only) {
       B2_UNROLL
       for (int k = 0; k < 2 * nv; k++) col[k] = dacc[k] * ih;
@@ -380,7 +395,8 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
   }
   typedef typename std::conditional<SENS, NominalWithSensors<T>, NominalInMemory<T>>::type Nominal;
   Nominal nom;
-  nom.st = st; nom.N = N; nom.e = e; nom.u0 = u0;
+  nom.set(st.qpos, st.qvel, st.warm, N, e);
+  nom.u0 = u0;
   if constexpr (SENS) { nom.dsdx = dsdx; nom.dsdu = dsdu; }
   const bool grouped = M::integrator() == 0;  // not a constant expression for the runtime provider
   const int groups = fd_group_count(nv, nu);
@@ -393,7 +409,7 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
   // position stage is the step's -- and leaves the new state in the shadow arrays (the other threads of the env still
   // read the nominal state); k_commit_state swaps the two afterwards
   const bool advance = grouped && task == 0 && shadow.qpos != nullptr;
-  bool pos_valid = false, vel_valid = false;
+  int last = -1;
   const T inv_eps = T(1) / eps;
   // mj_checkPos / mj_checkVel once on the nominal state (an eps perturbation of a finite state is finite)
   B2_UNROLL
@@ -406,7 +422,7 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
   B2_NOUNROLL
   for (int c = c0; c < c1 + (advance ? 1 : 0) && !frozen; c++) {
     const bool nominal = c == c1;  // the advance comes after the group's columns, on the same position stage
-    fd_column(env, nom, nominal ? ndx + nu : c, nominal, eps, inv_eps, centered, N, e, A, B, pos_valid, vel_valid);
+    fd_column(env, nom, nominal ? ndx + nu : c, nominal, eps, inv_eps, centered, N, e, A, B, last);
   }
   if (advance) {
     B2_UNROLL
@@ -781,12 +797,8 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
   for (int k = 0; k < nu; k++) u0[k] = ctrl_seq ? ctrl_seq[((size_t)t * nu + k) * N + e] : st.ctrl[(size_t)k * N + e];
   typedef typename std::conditional<SENS, NominalWithSensors<T>, NominalInMemory<T>>::type Nominal;
   Nominal nom;
-  nom.st.qpos = qpos_traj + (size_t)t * nq * N;
-  nom.st.qvel = qvel_traj + (size_t)t * nv * N;
-  nom.st.warm = warm_traj ? warm_traj + (size_t)t * nv * N : nullptr;
-  nom.st.ctrl = nullptr;
-  nom.st.flags = nullptr;
-  nom.N = N; nom.e = e; nom.u0 = u0;
+  nom.set(qpos_traj + (size_t)t * nq * N, qvel_traj + (size_t)t * nv * N, warm_traj ? warm_traj + (size_t)t * nv * N : nullptr, N, e);
+  nom.u0 = u0;
   if constexpr (SENS) {
     const size_t nsd = M::nsensordata();
     nom.dsdx = dsdx ? dsdx + (size_t)t * nsd * ndx * N : nullptr;
@@ -801,7 +813,7 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
     if (task < groups) { c0 = nv + task * B2_FD_GROUP; c1 = c0 + B2_FD_GROUP < ndx + nu ? c0 + B2_FD_GROUP : ndx + nu; }
     else { c0 = task - groups; c1 = c0 + 1; }
   }
-  bool pos_valid = false, vel_valid = false;
+  int last = -1;
   const T inv_eps = T(1) / eps;
   // mj_checkPos / mj_checkVel once on the nominal state, as k_linearize does
   B2_UNROLL
@@ -810,7 +822,7 @@ __global__ void __launch_bounds__(B2_LIN_THREADS, B2_LIN_MIN_BLOCKS) k_linearize
   for (int k = 0; k < nv; k++) env.qvel[k] = nom.v(k);
   env.check_state();
   B2_NOUNROLL
-  for (int c = c0; c < c1; c++) fd_column(env, nom, c, false, eps, inv_eps, centered, N, e, At, Bt, pos_valid, vel_valid);
+  for (int c = c0; c < c1; c++) fd_column(env, nom, c, false, eps, inv_eps, centered, N, e, At, Bt, last);
   if (st.flags && env.flags) atomicOr(st.flags + e, env.flags);
 }
 // Both launches of b2_linearize_rollout.  ntask: FD tasks per env (fd_task_count of the model).  The FD launch is skipped

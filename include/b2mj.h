@@ -303,6 +303,34 @@ int b2_tvlqr(int device, int precision, int nsteps, int nx, int nu, int nenv, co
              const double* R, const double* Qf, const void* q, const void* r, double reg, void* K, void* k, void* P0, void* dV,
              int* status, void* stream);
 
+/* Trajectory tracking cost and its exact tangent-space gradients, batched: the cost step of iLQR between
+ * b2_linearize_rollout and b2_tvlqr, and the cost of every line-search trial.  For every env, with T = nsteps:
+ *     e_t = [ q_t (-) qref_t ; v_t - vref_t ]   (t = 0..T)      w_t = u_t - uref_t   (t = 0..T-1)
+ *     J   = sum_{t<T} ( 1/2 e_t'Q e_t + 1/2 w_t'R w_t ) + 1/2 e_T'Qf e_T
+ * (-) is b2_differentiate_pos(dt = 1, qref_t -> q_t), the operator of b2_lqr_control and b2_rollout_feedback: for a free
+ * joint the world-frame position difference and log(conj(qref) (x) q) in the local frame, on the shortest path.
+ * The gradients are taken with respect to the tangent deviation of b2_linearize_rollout's A and b2_rollout_feedback:
+ * with x_t = xbar_t (+) dx_t, where (+) is b2_integrate_pos (qbar (x) Exp(dw) for a free joint's rotation),
+ *     q_t = dJ/ddx_t = G_t' M e_t   (M = Q for t < T, Qf for t = T)        r_t = dJ/du_t = R w_t
+ * G_t is the identity except on each free joint's rotation block, where it is Jr^-1(phi) with phi that joint's rotation
+ * part of e_t:  Jr^-1(phi) = I + 1/2 [phi]x + (1/th^2 - (1 + cos th) / (2 th sin th)) [phi]x^2,  th = |phi|  (below
+ * th = 0.1 the series of the coefficient, which tends to 1/12).  At th = pi (a rotation error of half a turn) the cost is
+ * not differentiable and the coefficient is unbounded.  Q, R and Qf remain the Gauss-Newton Hessian (G ~ I), so
+ * b2_tvlqr(A, B, Q, R, Qf, q, r, reg) on these outputs is the iLQR step, and (J(alpha) - J)/alpha -> dV[0] as alpha -> 0.
+ * DEVICE arrays in the batch's precision, env fastest, in the layout b2_linearize_rollout writes:
+ *     qpos_traj, qpos_ref (nsteps+1, nq, nenv), qvel_traj (nsteps+1, nv, nenv), ctrl_traj (nsteps, nu, nenv) -- required
+ *     qvel_ref (nsteps+1, nv, nenv), ctrl_ref (nsteps, nu, nenv)                                  -- may be NULL (zeros)
+ *     J (nenv), q (nsteps+1, 2nv, nenv), r (nsteps, nu, nenv)  -- b2_tvlqr's q / r; any may be NULL, not all three
+ * Q, Qf (2nv x 2nv) and R (nu x nu): HOST arrays, row-major, exactly symmetric, shared by all envs; kept on the device in
+ * b2_tvlqr's block, so that after the first call with given weights the call neither allocates nor copies and can be
+ * captured in a CUDA graph.  Reads nothing from the batch's state and writes nothing to it.  A NaN row reaches its own
+ * env's J, q and r only (a frozen env of b2_rollout_feedback has NaN control rows, so its J is NaN).  One launch on
+ * both engines; J is the same from run to run (no atomics); offsets are 64-bit.  nsteps < 1, a NULL required pointer,
+ * all outputs NULL, a model without actuators or a weight that is not exactly symmetric: B2_ERR_ARG. */
+int b2_traj_cost(b2_batch* batch, int nsteps, const void* qpos_traj, const void* qvel_traj, const void* ctrl_traj,
+                 const void* qpos_ref, const void* qvel_ref, const void* ctrl_ref, const double* Q, const double* R,
+                 const double* Qf, void* J, void* q, void* r, void* stream);
+
 /* Batched recorder sink: one CSV row per selected env and step, in the reference's column layout
  * (reference logging.py:81-247: time_s, qpos.., qvel.., ctrl.., probe columns).  A recorder is a column table
  * { array base (device pointer into a (dim, nenv) state / derived array of the batch), row } plus a selection of env

@@ -859,6 +859,40 @@ int b2_tvlqr(int device, int precision, int nsteps, int nx, int nu, int nenv, co
   return rc ? cuda_fail((cudaError_t)rc, "b2_tvlqr launch") : B2_OK;
 }
 
+// Trajectory tracking cost and its tangent-space gradients (see include/b2mj.h).  The weights go through b2_tvlqr's
+// resident block, so that the two calls of an iLQR iteration share one device copy.
+int b2_traj_cost(b2_batch* b, int nsteps, const void* qpos_traj, const void* qvel_traj, const void* ctrl_traj, const void* qpos_ref,
+                 const void* qvel_ref, const void* ctrl_ref, const double* Q, const double* R, const double* Qf, void* J, void* q, void* r,
+                 void* stream) {
+  if (nsteps < 1) return fail(B2_ERR_ARG, "b2_traj_cost: nsteps must be >= 1");
+  if (!qpos_traj || !qvel_traj || !ctrl_traj || !qpos_ref || !Q || !R || !Qf)
+    return fail(B2_ERR_ARG, "b2_traj_cost: qpos_traj, qvel_traj, ctrl_traj, qpos_ref, Q, R and Qf are required");
+  if (!J && !q && !r) return fail(B2_ERR_ARG, "b2_traj_cost: J, q and r are all NULL");
+  if (!b) return fail(B2_ERR_ARG, "b2_traj_cost: null batch");
+  const b2_model* m = b->model;
+  const int nx = 2 * m->v.nv, nu = m->v.nu;
+  if (nu == 0) return fail(B2_ERR_ARG, "b2_traj_cost: the model has no actuators");
+  // the gradient G'M dx is that of 1/2 dx'M dx only for a symmetric M
+  const double* mats[3] = {Q, R, Qf};
+  const char* names[3] = {"Q", "R", "Qf"};
+  for (int k = 0; k < 3; k++) {
+    const int n = k == 1 ? nu : nx;
+    for (int i = 0; i < n; i++)
+      for (int j = 0; j < i; j++)
+        if (!(mats[k][i * n + j] == mats[k][j * n + i])) return fail(B2_ERR_ARG, std::string("b2_traj_cost: ") + names[k] + " is not symmetric");
+  }
+  const void* lane = nullptr;
+  if (int rc = batch_images(b, &lane)) return rc;
+  std::vector<double> w(Q, Q + (size_t)nx * nx);
+  w.insert(w.end(), R, R + (size_t)nu * nu);
+  w.insert(w.end(), Qf, Qf + (size_t)nx * nx);
+  void* dw = nullptr;
+  if (int rc = resident_weights(b->device, b->precision, nx, nu, w, "b2_traj_cost", &dw)) return rc;
+  return launched(b->k->traj_cost(lane, m->cls, b->nenv, nsteps, qpos_traj, qvel_traj, ctrl_traj, qpos_ref, qvel_ref, ctrl_ref, dw, J, q, r,
+                                  stream),
+                  "b2_traj_cost launch");
+}
+
 struct b2_recorder {
   b2_batch* batch;
   void* d_cols;

@@ -971,4 +971,93 @@ __global__ void __launch_bounds__(128) k_tvlqr_law(StateDev<T> st, int N, const 
   }
 }
 
+// y <- Jr^-1(phi)' y for one free joint's rotation block: the chain rule of phi = Log(qref^-1 q) under q <- q Exp(d).
+// Jr^-1(phi) = I + 1/2 [phi]x + c [phi]x^2 with c = 1/th^2 - (1 + cos th) / (2 th sin th), th = |phi|; its transpose flips
+// the sign of the [phi]x term.  Below th = 0.1 the series of c (to th^6) replaces the cancelling difference.
+template <typename T>
+B2_DEV void jr_inv_transpose(T* y, const T* phi) {
+  const T th2 = phi[0] * phi[0] + phi[1] * phi[1] + phi[2] * phi[2];
+  T c;
+  if (th2 < T(1e-2)) c = T(1) / 12 + th2 * (T(1) / 720 + th2 * (T(1) / 30240 + th2 * (T(1) / 1209600)));
+  else {
+    const T th = sqrt(th2);
+    c = T(1) / th2 - (T(1) + cos(th)) / (T(2) * th * sin(th));
+  }
+  const T a[3] = {phi[1] * y[2] - phi[2] * y[1], phi[2] * y[0] - phi[0] * y[2], phi[0] * y[1] - phi[1] * y[0]};  // phi x y
+  const T b[3] = {phi[1] * a[2] - phi[2] * a[1], phi[2] * a[0] - phi[0] * a[2], phi[0] * a[1] - phi[1] * a[0]};  // phi x (phi x y)
+  for (int k = 0; k < 3; k++) y[k] += -T(0.5) * a[k] + c * b[k];
+}
+
+// Trajectory tracking cost and its tangent-space gradients (b2_traj_cost).  For env e, with dx_t = [q_t (-) qref_t ; v_t -
+// vref_t] (t = 0 .. nsteps) and du_t = u_t - uref_t (t < nsteps):
+//     J = sum_{t<T} (1/2 dx'Q dx + 1/2 du'R du) + 1/2 dx_T'Qf dx_T,   q_t = G_t' M dx_t,   r_t = R du_t
+// where G_t is the identity but for Jr^-1 on each free joint's rotation block.  A block serves 32 envs (one per lane) with
+// blockDim.x / 32 warps; warp w takes the steps t = w, w + warps, ... and the warps' partial costs are summed in warp order,
+// so J does not change from run to run.  W = [Q, R, Qf] (row-major, the b2_tvlqr block) is read with uniform loads.
+// vref, uref null: zeros; J, gq (nsteps+1, 2nv, N), gr (nsteps, nu, N) may be null.
+template <typename T, class D, class M>
+__global__ void __launch_bounds__(1024) k_traj_cost(int N, int nsteps, const T* __restrict__ qpos, const T* __restrict__ qvel,
+                                                    const T* __restrict__ ctrl, const T* __restrict__ qref, const T* __restrict__ vref,
+                                                    const T* __restrict__ uref, const T* __restrict__ W, T* J, T* gq, T* gr,
+                                                    const void* image = nullptr) {
+  model_load<M>(image, 0);
+  __shared__ T part[32][32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int e = blockIdx.x * 32 + lane;
+  const int nq = M::nq(), nv = M::nv(), nu = M::nu(), nx = 2 * nv;
+  const T* R = W + (size_t)nx * nx;
+  T acc = 0;
+  if (e < N) {
+    RowStore<T, D> rows;
+    LaneEnv<T, D, M> env(rows);
+    B2_NOUNROLL
+    for (int t = w; t <= nsteps; t += nw) {
+      const T* Mw = t < nsteps ? W : R + (size_t)nu * nu;
+      T a[D::NQ], b[D::NQ], x[2 * D::NV], y[2 * D::NV];
+      B2_UNROLL
+      for (int i = 0; i < nq; i++) { a[i] = qref[((size_t)t * nq + i) * N + e]; b[i] = qpos[((size_t)t * nq + i) * N + e]; }
+      env.differentiate_pos(x, T(1), a, b);
+      B2_UNROLL
+      for (int i = 0; i < nv; i++) x[nv + i] = qvel[((size_t)t * nv + i) * N + e] - (vref ? vref[((size_t)t * nv + i) * N + e] : T(0));
+      T c = 0;
+      B2_UNROLL
+      for (int i = 0; i < nx; i++) {
+        T s = 0;
+        B2_UNROLL
+        for (int j = 0; j < nx; j++) s += Mw[i * nx + j] * x[j];
+        y[i] = s;
+        c += x[i] * s;
+      }
+      if (gq) {
+        B2_UNROLL
+        for (int j = 0; j < M::njnt(); j++)
+          if (M::jnt_type(j) == JNT_FREE) jr_inv_transpose(y + M::jnt_dofadr(j) + 3, x + M::jnt_dofadr(j) + 3);
+        B2_UNROLL
+        for (int i = 0; i < nx; i++) gq[((size_t)t * nx + i) * N + e] = y[i];
+      }
+      if (t < nsteps) {
+        T du[D::NU];
+        B2_UNROLL
+        for (int i = 0; i < nu; i++) du[i] = ctrl[((size_t)t * nu + i) * N + e] - (uref ? uref[((size_t)t * nu + i) * N + e] : T(0));
+        B2_UNROLL
+        for (int i = 0; i < nu; i++) {
+          T s = 0;
+          B2_UNROLL
+          for (int j = 0; j < nu; j++) s += R[i * nu + j] * du[j];
+          c += du[i] * s;
+          if (gr) gr[((size_t)t * nu + i) * N + e] = s;
+        }
+      }
+      acc += T(0.5) * c;
+    }
+  }
+  part[w][lane] = acc;
+  __syncthreads();
+  if (w == 0 && e < N && J) {
+    T s = part[0][lane];
+    for (int k = 1; k < nw; k++) s += part[k][lane];
+    J[e] = s;
+  }
+}
+
 }  // namespace b2

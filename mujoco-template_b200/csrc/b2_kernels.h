@@ -78,6 +78,9 @@ struct Kernels {
   // one step's law of b2_rollout_feedback on the lane engine's model image (the warp engine's loop): pointers at step t's rows
   int (*tvlqr_law)(const void* image, int cls, const b2_state* st, int N, const void* ubar, const void* qbar, const void* vbar,
                    const void* K, const void* k, const void* alpha, void* ctrl_row, void* stream);
+  // b2_traj_cost on the lane engine's model image: W = Q, R, Qf on the device (the b2_tvlqr block); one launch
+  int (*traj_cost)(const void* image, int cls, int N, int nsteps, const void* qpos, const void* qvel, const void* ctrl, const void* qref,
+                   const void* vref, const void* uref, const void* W, void* J, void* q, void* r, void* stream);
 };
 extern const Kernels kernels_f64, kernels_f32;
 

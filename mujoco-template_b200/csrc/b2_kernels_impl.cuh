@@ -348,6 +348,18 @@ static int b2k_tvlqr_law(const void* image, int cls, const b2_state* st, int N, 
                        (const real*)alpha, (real*)ctrl_row, image)));
   return (int)cudaGetLastError();
 }
+static int b2k_traj_cost(const void* image, int cls, int N, int nsteps, const void* qpos, const void* qvel, const void* ctrl, const void* qref,
+                         const void* vref, const void* uref, const void* W, void* J, void* q, void* r, void* stream) {
+  // a block per 32 envs; 8 warps share its steps, more when there are too few blocks to give every SM 32 warps (a small
+  // batch of a large model), at most one warp per step
+  const int blocks = (N + 31) / 32;
+  int warps = 8;
+  while (warps < 32 && 2 * warps <= nsteps + 1 && (long long)blocks * warps < 148 * 32) warps *= 2;
+  B2_DISPATCH(cls, (k_traj_cost<real, DD, RuntimeModel<DD>><<<blocks, 32 * warps, 0, (cudaStream_t)stream>>>(
+                       N, nsteps, (const real*)qpos, (const real*)qvel, (const real*)ctrl, (const real*)qref, (const real*)vref,
+                       (const real*)uref, (const real*)W, (real*)J, (real*)q, (real*)r, image)));
+  return (int)cudaGetLastError();
+}
 // b2_tvlqr: a thread per env (compile-time sizes, registers) for the sizes k_dare_small covers, otherwise a warp per env
 // with its matrices in shared memory, as many warps (consecutive envs) per block as fit, at most four
 static int b2k_tvlqr(const void* A, const void* B, const void* W, const void* q, const void* r, int nsteps, int nx, int nu, int N, double reg,
@@ -383,7 +395,7 @@ const Kernels B2_FN(kernels) = {
     b2k_commit_state, b2k_random_controls, b2k_record_rows, b2k_dare, b2k_fma_peak,
     b2k_image_bytes, b2k_image_fill,
     b2k_warp_plan, b2k_warp_scratch_bytes, b2k_warp_image_bytes, b2k_warp_image_fill, b2k_warp_sort_bytes, b2k_warp_step, b2k_warp_linearize,
-    b2k_tvlqr, b2k_tvlqr_law,
+    b2k_tvlqr, b2k_tvlqr_law, b2k_traj_cost,
 };
 
 }  // namespace b2

@@ -27,7 +27,7 @@ EXPORTED_SYMBOLS = (
     "b2_differentiate_pos", "b2_inverse", "b2_lqr_set_gain", "b2_lqr_control", "b2_control_tick", "b2_refresh_derived", "b2_step_lazy", "b2_step_host", "b2_step_host_wait", "b2_stream_synchronize", "b2_launch_count",
     "b2_batch_size_class", "b2_last_error", "b2_version", "b2_fp_peak", "b2_batch_kernel_variant",
     "b2_recorder_create", "b2_recorder_record", "b2_recorder_destroy", "b2_dlqr", "b2_random_controls", "b2_warp_queue_histogram", "b2_lqr_control_env",
-    "b2_tvlqr", "b2_rollout_feedback",
+    "b2_tvlqr", "b2_rollout_feedback", "b2_traj_cost",
 )
 
 
@@ -101,6 +101,7 @@ def lib() -> C.CDLL:
                           C.c_double, vp, vp, vp, vp]
     L.b2_tvlqr.argtypes = [i, i, i, i, i, i, vp, vp, C.POINTER(d), C.POINTER(d), C.POINTER(d), vp, vp, d, vp, vp, vp, vp, vp, vp]
     L.b2_rollout_feedback.argtypes = [vp, C.POINTER(State), i, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(Derived), vp]
+    L.b2_traj_cost.argtypes = [vp, i, vp, vp, vp, vp, vp, vp, C.POINTER(d), C.POINTER(d), C.POINTER(d), vp, vp, vp, vp]
     L.b2_recorder_create.argtypes = [vp, C.POINTER(RecordCol), C.c_int, C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]
     L.b2_recorder_record.argtypes = [vp, C.c_double, vp, vp]
     L.b2_recorder_destroy.argtypes = [vp]
@@ -184,6 +185,17 @@ class NativeBatch:
         v - qvel_nom[t]])``, recording the applied controls and the state (and sensordata) after every step."""
         check(self._L.b2_rollout_feedback(self.handle, C.byref(state), int(nsteps), ctrl_nom, qpos_nom, qvel_nom, K, k, alpha, ctrl_traj,
                                           qpos_traj, qvel_traj, sensor_traj, C.byref(derived) if derived is not None else None, stream))
+
+    def traj_cost(self, nsteps: int, qpos: int, qvel: int, ctrl: int, qpos_ref: int, qvel_ref: int | None, ctrl_ref: int | None, Q, R, Qf,
+                  J: int | None, q: int | None, r: int | None, stream: int = 0) -> None:
+        """``b2_traj_cost``: the tracking cost ``J`` of every env's trajectory and its tangent-space gradients ``q`` / ``r``
+        (device pointers in the env-fastest layout; Q, R, Qf host arrays)."""
+        import numpy as np
+
+        # flattened row-major float64 arrays, handed over without a per-element conversion (the humanoid's Q has 2,916)
+        W = [np.ascontiguousarray(M, dtype=np.float64).reshape(-1) for M in (Q, R, Qf)]
+        check(self._L.b2_traj_cost(self.handle, int(nsteps), qpos, qvel, ctrl, qpos_ref, qvel_ref, ctrl_ref,
+                                   *[M.ctypes.data_as(C.POINTER(C.c_double)) for M in W], J, q, r, stream))
 
     def forward(self, state: State, derived: Derived | None, stream: int = 0) -> None:
         check(self._L.b2_forward(self.handle, C.byref(state), C.byref(derived) if derived is not None else None, stream))

@@ -426,6 +426,24 @@ class NativeBackend:
                      eps, centered, ptr(A), ptr(B), ptr(C_), ptr(D_), ptr(q), ptr(v), ptr(w), ptr(s))
         return tuple(out)
 
+    def traj_cost(self, qpos, qvel, ctrl, qpos_ref, qvel_ref, ctrl_ref, Q, R, Qf, nsteps: int, grad: bool, out=None):
+        """Tracking cost of every env's trajectory and, with ``grad``, its tangent-space gradients (``b2_traj_cost``).
+        Tensors in the library's layouts: ``qpos`` / ``qpos_ref`` (T+1, nq, nenv), ``qvel`` / ``qvel_ref`` (T+1, nv, nenv),
+        ``ctrl`` / ``ctrl_ref`` (T, nu, nenv); ``qvel_ref`` and ``ctrl_ref`` may be None (zeros).  ``Q``, ``R``, ``Qf``:
+        row-major host arrays.  Returns (J, q, r) of shapes (nenv,), (T+1, 2nv, nenv) and (T, nu, nenv), ``q`` / ``r``
+        None without ``grad``; fresh buffers unless ``out`` gives all three (an entry may be None: not written).  The
+        state is neither read nor written."""
+        torch, m = self.torch, self.model
+        T, n = int(nsteps), self.nenv
+        if out is None:
+            mk = ((lambda *shape: torch.zeros(shape, dtype=self.dtype).pin_memory()) if self.host_mapped else
+                  (lambda *shape: torch.empty(shape, device=f"cuda:{self.device}", dtype=self.dtype)))
+            out = (mk(n), mk(T + 1, 2 * m.nv, n) if grad else None, mk(T, m.nu, n) if grad else None)
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
+        self._launch("traj_cost", self.batch.traj_cost, T, ptr(qpos), ptr(qvel), ptr(ctrl), ptr(qpos_ref), ptr(qvel_ref), ptr(ctrl_ref),
+                     Q, R, Qf, *map(ptr, out))
+        return tuple(out)
+
     def jacobian(self, kind: int, objid: int, want_rot: bool):
         torch, m = self.torch, self.model
         mk = (lambda: torch.zeros((3, m.nv, self.nenv), dtype=self.dtype).pin_memory()) if self.host_mapped else (

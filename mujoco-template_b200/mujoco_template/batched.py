@@ -412,6 +412,75 @@ class BatchedEnv:
             traj["sensordata"] = out[3].permute(2, 0, 1)
         return traj
 
+    def traj_cost(self, qpos, qvel, ctrl, Q, R, Qf=None, *, qpos_ref, qvel_ref=None, ctrl_ref=None, grad: bool = False):
+        """Tracking cost of every env's trajectory, in one kernel launch (``b2_traj_cost``):
+
+            e_t = [q_t (-) qref_t ; v_t - vref_t]  (t = 0..T),   w_t = u_t - uref_t  (t < T)
+            J   = sum_{t<T} (1/2 e_t'Q e_t + 1/2 w_t'R w_t) + 1/2 e_T'Qf e_T
+
+        where (-) is ``mj_differentiatePos`` (the tangent space of ``linearize_rollout``'s ``A``: a quaternion log for a free
+        joint).  ``qpos`` ``(nenv, T+1, nq)`` and ``qvel`` ``(nenv, T+1, nv)`` are ``linearize_rollout``'s ``"qpos"`` /
+        ``"qvel"`` as they are, ``ctrl`` a ``(nenv, T, nu)`` control tensor; ``qpos_ref`` (required), ``qvel_ref`` and
+        ``ctrl_ref`` (None: zero) are ``(nenv, rows, dim)``, ``(rows, dim)`` or ``(dim,)`` tensors -- the last two are
+        broadcast over envs (and steps) once per call.  All on the batch's device, in its dtype.  ``Q``, ``R`` and ``Qf``
+        (default ``Q``) are exactly symmetric host matrices.
+
+        Returns ``J`` ``(nenv,)``; with ``grad=True`` ``(J, q, r)``, where ``q`` ``(nenv, T+1, 2nv)`` is the gradient with
+        respect to the tangent deviation of ``A`` and ``rollout_feedback`` (``x = xbar (+) dx``; it differs from ``Q e`` on
+        free joints' rotations by ``Jr^-1``) and ``r`` ``(nenv, T, nu)`` is ``R w``: ``batched_tvlqr``'s ``q`` / ``r``, read
+        without a copy.  A NaN row makes its own env's results NaN only.  Neither the state, ``data.time`` nor the step
+        counter moves."""
+        import torch
+
+        m, n = self.model, self.nenv
+        if m.nu == 0:
+            raise ConfigError("traj_cost: the model has no actuators (nu=0)")
+        ref = self.data.qpos
+        nx = 2 * m.nv
+
+        def check(name, t, shapes):
+            if not isinstance(t, torch.Tensor) or tuple(t.shape) not in shapes:
+                got = tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__
+                raise ConfigError(f"traj_cost: {name} must have shape {' or '.join(map(str, shapes))}, got {got}")
+            if t.device != ref.device or t.dtype != ref.dtype:
+                raise ConfigError(f"traj_cost: {name}: expected {ref.dtype} on {ref.device}, got {t.dtype} on {t.device}")
+
+        if not isinstance(ctrl, torch.Tensor) or ctrl.dim() != 3 or ctrl.shape[1] < 1:
+            raise ConfigError(f"traj_cost: ctrl must be a (nenv={n}, T, nu={m.nu}) tensor with T >= 1")
+        T = int(ctrl.shape[1])
+        rows = {"qpos": T + 1, "qvel": T + 1, "ctrl": T}
+        dims = {"qpos": m.nq, "qvel": m.nv, "ctrl": m.nu}
+
+        def traj(name, t):  # (nenv, rows, dim) -> (rows, dim, nenv) env fastest; no copy for a view of such storage
+            check(name, t, [(n, rows[name], dims[name])])
+            return t.permute(1, 2, 0).contiguous()
+
+        def reference(name, t):
+            if t is None:
+                return None
+            r, d = rows[name], dims[name]
+            check(f"{name}_ref", t, [(n, r, d), (r, d), (d,)])
+            if t.dim() == 3:
+                return t.permute(1, 2, 0).contiguous()
+            return (t[:, :, None] if t.dim() == 2 else t[None, :, None]).expand(r, d, n).contiguous()
+
+        def host(name, M, k):
+            M = np.asarray(M.cpu() if hasattr(M, "cpu") else M, dtype=float)
+            if M.shape != (k, k):
+                raise ConfigError(f"traj_cost: {name} must be ({k}, {k}), got {M.shape}")
+            return np.ascontiguousarray(M).reshape(-1)
+
+        qs, vs, us = traj("qpos", qpos), traj("qvel", qvel), traj("ctrl", ctrl)
+        if qpos_ref is None:
+            raise ConfigError("traj_cost: qpos_ref is required")
+        qr, vr, ur = reference("qpos", qpos_ref), reference("qvel", qvel_ref), reference("ctrl", ctrl_ref)
+        Qh, Rh = host("Q", Q, nx), host("R", R, m.nu)
+        Qfh = Qh if Qf is None else host("Qf", Qf, nx)
+        J, q, r = self.data.backend.traj_cost(qs, vs, us, qr, vr, ur, Qh, Rh, Qfh, T, bool(grad))
+        if not grad:
+            return J
+        return J, q.permute(2, 0, 1), r.permute(2, 0, 1)
+
     def _control_sequence(self, what: str, controls, nsteps):
         """Validates a ``(nenv, T, nu)`` control tensor and ``nsteps``; returns the controls as a ``(T, nu, nenv)`` layout
         (None without controls) and T."""

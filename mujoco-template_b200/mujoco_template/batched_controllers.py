@@ -145,6 +145,89 @@ def batched_tvlqr(A, B, Q, R, Qf=None, q=None, r=None, reg: float = 0.0):
     return Ks.permute(3, 0, 1, 2), ks.permute(2, 0, 1), Ps.permute(2, 0, 1), dVs.permute(1, 0), status
 
 
+def batched_ilqr(env, controls, Q, R, Qf=None, *, qpos_ref, qvel_ref=None, ctrl_ref=None, iters: int = 20,
+                 alphas=tuple(0.5 ** i for i in range(10)), reg: float = 1e-6, eps: float | None = None):
+    """iLQR for every env of a ``BatchedEnv`` from its current state, on the device: minimises ``BatchedEnv.traj_cost``
+    over the control sequence.  Each iteration runs
+
+        1. ``linearize_rollout(ubar)``: the nominal trajectory and its ``(A_t, B_t)``;
+        2. ``traj_cost(grad=True)``: its cost ``J`` and the gradients ``q_t`` / ``r_t``;
+        3. ``batched_tvlqr(A, B, Q, R, Qf, q, r, reg)``: the gains ``K_t``, ``k_t``;
+        4. a backtracking line search over ``alphas``: per trial one ``rollout_feedback`` with the step size of each env and
+           one ``traj_cost``.  An env accepts the first step size whose cost is finite and below its current ``J`` and then
+           keeps that result; an env whose backward pass failed (``status != 0``) rejects every trial.  The trials stop once
+           every env with a valid backward pass has accepted.
+
+    ``controls`` ``(nenv, T, nu)`` is the initial control sequence; ``Q``, ``R``, ``Qf`` and the references are those of
+    ``traj_cost``; ``eps`` is the FD step of ``linearize_rollout`` (None: the env's ``lin_eps``).  The iterations stop early
+    when one leaves every env where it was (the next would repeat it).  The env's state, warm start, controls, flags,
+    ``data.time`` and step counter are left as they were.
+
+    Returns a dict: ``"ctrl"`` ``(nenv, T, nu)``, ``"qpos"`` ``(nenv, T+1, nq)`` and ``"qvel"`` ``(nenv, T+1, nv)`` (the
+    final nominal trajectory, row 0 the current state), ``"J"`` ``(nenv,)``, ``"J_history"`` ``(iterations + 1, nenv)``
+    (the cost before the first iteration and after each) and ``"status"`` ``(nenv,)``, the last backward pass's status."""
+    import torch
+
+    data, b, m, n = env.data, env.data.backend, env.model, env.nenv
+    if not isinstance(controls, torch.Tensor) or controls.dim() != 3 or tuple(controls.shape[::2]) != (n, m.nu) or controls.shape[1] < 1:
+        raise ConfigError(f"batched_ilqr: controls must be a (nenv={n}, T, nu={m.nu}) tensor")
+    alphas = [float(a) for a in alphas]
+    if not alphas or not all(a > 0 for a in alphas) or int(iters) < 1:
+        raise ConfigError("batched_ilqr: iters must be >= 1 and alphas a non-empty sequence of positive step sizes")
+    T = int(controls.shape[1])
+    cost = dict(qpos_ref=qpos_ref, qvel_ref=qvel_ref, ctrl_ref=ctrl_ref)
+    saved = {k: b.buffers[k].clone() for k in ("qpos", "qvel", "ctrl", "qacc_warmstart", "flags") if b.buffers[k].numel()}
+    stale = b.derived_stale
+    x0 = saved["qpos"], saved["qvel"]
+    # trial trajectories: rollout_feedback records rows 1..T of (T+1)-row buffers whose row 0 is x0
+    mk = lambda *shape: torch.empty(shape, dtype=data.qpos.dtype, device=data.qpos.device)  # noqa: E731
+    tq, tv, tu = mk(T + 1, m.nq, n), mk(T + 1, m.nv, n), mk(T, m.nu, n)
+    tq[0], tv[0] = x0
+    trial = tq.permute(2, 0, 1), tv.permute(2, 0, 1), tu.permute(2, 0, 1)
+
+    def restore(keys):
+        for k in keys:
+            if k in saved:
+                b.buffers[k].copy_(saved[k])
+
+    try:
+        ubar = controls.detach().clone()
+        lin = env.linearize_rollout(ubar, eps=eps)
+        J, q, r = env.traj_cost(lin["qpos"], lin["qvel"], ubar, Q, R, Qf, grad=True, **cost)
+        xq, xv = lin["qpos"].clone(), lin["qvel"].clone()
+        history = [J.clone()]
+        status = torch.zeros(n, dtype=torch.int32, device=J.device)
+        for it in range(int(iters)):
+            K, k, _, _, status = batched_tvlqr(lin["A"], lin["B"], Q, R, Qf, q, r, reg)
+            Ks, ks = K.permute(1, 2, 3, 0), k.permute(1, 2, 0)
+            seq, qn, vn = ubar.permute(1, 2, 0).contiguous(), lin["qpos"].permute(1, 2, 0), lin["qvel"].permute(1, 2, 0)
+            accepted = torch.zeros(n, dtype=torch.bool, device=J.device)
+            done = status != 0  # NaN gains: never accepted, whatever the clip makes of them
+            for a in alphas:
+                restore(("qpos", "qvel", "qacc_warmstart", "flags"))
+                alpha = torch.full((n,), a, dtype=J.dtype, device=J.device)
+                b.rollout_feedback(seq, qn, vn, Ks, ks, alpha, T, False, out=(tu, tq[1:], tv[1:], None), derived=False)
+                Jn = env.traj_cost(*trial, Q, R, Qf, **cost)
+                take = ~done & torch.isfinite(Jn) & (Jn < J)
+                J = torch.where(take, Jn, J)
+                ubar = torch.where(take[:, None, None], trial[2], ubar)
+                xq, xv = torch.where(take[:, None, None], trial[0], xq), torch.where(take[:, None, None], trial[1], xv)
+                accepted |= take
+                done |= take
+                if bool(done.all()):
+                    break
+            history.append(J.clone())
+            if not bool(accepted.any()) or it == int(iters) - 1:
+                break
+            restore(("qpos", "qvel", "qacc_warmstart", "flags"))
+            lin = env.linearize_rollout(ubar, eps=eps)
+            _, q, r = env.traj_cost(lin["qpos"], lin["qvel"], ubar, Q, R, Qf, grad=True, **cost)
+    finally:
+        restore(saved)
+        b.derived_stale = stale
+    return {"ctrl": ubar, "qpos": xq, "qvel": xv, "J": J, "J_history": torch.stack(history), "status": status}
+
+
 class BatchedLQRController:
     def __init__(self, qpos_ref: np.ndarray | None = None, ctrl_ref: np.ndarray | None = None,
                  Q: np.ndarray | None = None, R: np.ndarray | None = None, eps: float = 1e-6,
@@ -328,4 +411,5 @@ class BatchedRandomController:
         b._launch("random_controls", b.batch.random_controls, b.state_struct(), self.lo, self.hi, self.seed, row, thr, rq, rv)
 
 
-__all__ = ["BatchedLQRController", "BatchedTVLQRController", "BatchedRandomController", "batched_dlqr_gain", "batched_tvlqr", "dlqr_gain"]
+__all__ = ["BatchedLQRController", "BatchedTVLQRController", "BatchedRandomController", "batched_dlqr_gain", "batched_ilqr", "batched_tvlqr",
+           "dlqr_gain"]
